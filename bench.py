@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: IQ Msamples/s from uint8 IQ to Signal records (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c4] [--dump-outputs DIR]
 
 Workloads (one *step* = one engine launch for every stream of the batch; weak scaling: every GPU owns its own 64 streams,
 no collective on the data path -- streams are independent analyzers, SURVEY.md section 8e):
@@ -22,6 +22,10 @@ no collective on the data path -- streams are independent analyzers, SURVEY.md s
 `parity`       the oracle on two streams of the very batch that was timed (BASELINE.md section 4: the gate reported with the number).
 `cpu_baseline` the oracle port of the reference's scipy path on ONE host core, one full step of the workload (N = 1 only);
                `--impl reference` runs the same port with one analyzer process per host core.
+
+`--dump-outputs DIR` writes the candidate records (include/rt_engine.h `rt_record`) of the last timed launch, one float64
+array per field: stream, fi, start, end, max_lin, row_mean, mean_lin, std_db (with `rank<r>_` in front when N > 1).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -57,7 +61,12 @@ def parse():
     ap.add_argument("--bpl", type=int, default=0, help="c4: callback blocks per launch (rt_config.blocks_per_launch; 0 = the workload's default, 10)")
     ap.add_argument("--fft-impl", default="auto", choices=["auto", "reg256", "tc256", "generic"],
                     help="spectrogram kernel: auto = reg256 (registers, packed fp32x2); tc256 = tensor-core stage 1 (tcgen05)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the candidate records of the last timed launch to DIR/<field>.npy (float64, one array per rt_record field)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the records of the GPU path (--impl b200)")
+    return args
 
 
 class Work:
@@ -317,18 +326,33 @@ def cpu_port_single(wk):
 # ----------------------------------------------------------------------------------------------------
 def drain(eng):
     """Fetch (and drop) every launch that has not been fetched yet, so that the next submit / collect pair talks about the same
-    launch.  The device-resident loops launch K times and fetch once: up to one result stays in the engine's ring behind them."""
+    launch.  The device-resident loops launch K times and fetch once: up to one result stays in the engine's ring behind them.
+    Returns the records of the newest launch fetched here (None if none was left)."""
     from pyradiotracking_b200.engine import RT_ERR_STATE, EngineError
 
-    n = 0
+    last = None
     while True:
         try:
-            eng.fetch()
-            n += 1
+            last = eng.fetch()
         except EngineError as e:
             if e.code != RT_ERR_STATE:
                 raise
-            return n
+            return last
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_records(recs, out_dir, prefix=""):
+    """One float64 array per rt_record field (integers and float32 values are exact in float64).  Above DUMP_LIMIT_BYTES a
+    fixed, seeded sample of the records is written, in record order."""
+    per_record = 8 * len(recs.dtype.names)
+    if len(recs) * per_record > DUMP_LIMIT_BYTES:
+        keep = np.random.default_rng(0).choice(len(recs), DUMP_LIMIT_BYTES // per_record, replace=False)
+        recs = recs[np.sort(keep)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name in recs.dtype.names:
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), recs[name].astype(np.float64))
 
 
 def parity_gate(wk, ba, hnp, streams):
@@ -459,9 +483,12 @@ def run_b200(args):
     ms = max(ms_ranks)
     tim = eng.timing(reset=True)
     eng.enable_timing(0)
-    n_rec = len(eng.fetch())
+    recs = eng.fetch()
+    n_rec = len(recs)
     work_items = eng.last_counts()[0]
-    drain(eng)          # K launches, one fetch: the newest result is still in the ring
+    newest = drain(eng)          # K launches, one fetch: the newest result is still in the ring
+    if args.dump_outputs:
+        dump_records(recs if newest is None else newest, args.dump_outputs, f"rank{rank}_" if world > 1 else "")
 
     # ---- end to end through the public API with host buffers -----------------------------------------
     import datetime

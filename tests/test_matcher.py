@@ -118,20 +118,3 @@ def test_non_signal_messages_are_ignored_and_naive_timestamps_work():
     assert len(q.items) == 1 and q.items[0]._avgs == [-55.0, -57.0] and q.items[0].ts == t
     assert q.items[0].duration == datetime.timedelta(milliseconds=10)
     m.close()
-
-
-def test_live_reference_when_present():
-    """In the build container the unmodified reference is importable: drive it and the native matcher side by side."""
-    from oracle import ref_harness
-
-    if not ref_harness.available():
-        pytest.skip("reference checkout not present")
-    from oracle.make_matcher_golden import run_reference
-
-    for name in ("with_margins", "boundaries"):
-        sigs, emitted, still_open, _ = run_reference(name)
-        q = _Q()
-        m = SignalMatcher(signal_queue=q, **M.matcher_kwargs(name))
-        m.add_batch(_as_signals(sigs))
-        assert M.groups_as_ids(q.items) == emitted and M.groups_as_ids(m._matched) == still_open
-        m.close()

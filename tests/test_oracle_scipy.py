@@ -1,11 +1,11 @@
 """Spectrogram restatement vs the installed scipy (the de-facto pin of the unvendored
-dependency, SURVEY.md §8c) and vs the reference itself when it is present."""
+dependency, SURVEY.md §8c).  The comparison with the reference itself runs on its stored
+outputs (tests/test_oracle_golden.py)."""
 import datetime
 
 import numpy as np
 import pytest
 
-from oracle import ref_harness
 from oracle import restatement as R
 from pyradiotracking_b200 import synth
 
@@ -36,19 +36,3 @@ def test_empty_and_single_column():
     f, t, S = R.spectrogram(R.bytes_to_iq(synth.make_stream(synth.C1, 0, 1)[0][:512]), 300000, "hamming", 256)
     with pytest.raises(IndexError):       # analyze.py:354 indexes times[1]
         R.extract_sequential(P, f, t, S, None, datetime.datetime(2026, 1, 1))
-
-
-@pytest.mark.skipif(not ref_harness.available(), reason="reference tree not present (GPU box)")
-def test_restatement_matches_live_reference():
-    w = synth.C1
-    cap = synth.make_stream(w, 17, 3)
-    t0 = datetime.datetime(2026, 5, 5, 5, 5, 5)
-    ref = ref_harness.ReferenceRunner(t0, sample_rate=w.sample_rate)
-    ora = R.OracleAnalyzer(R.Params.make(sample_rate=w.sample_rate))
-    bl = datetime.timedelta(seconds=1)
-    for b in range(3):
-        queued = ref.feed(cap[b])
-        _, _, S, found, kept = ora.process_block(cap[b], t0 + (b - 1) * bl)
-        np.testing.assert_allclose(S, ref.spectrogram_last, rtol=1e-9)
-        assert [(s.ts, s.frequency, s.duration) for s in ref.pre_shadow[-1]] == [(d.ts, d.frequency, d.duration) for d in found]
-        assert [(s.ts, s.frequency) for s in queued] == [(d.ts, d.frequency) for d in kept]
