@@ -85,7 +85,10 @@ typedef struct rt_config {
     int32_t blocks_per_launch;  /* offline replay: this many CONSECUTIVE callback blocks of every stream per launch (>= 1).
                                    Block b of stream s is the analyzer unit s * blocks_per_launch + b: it has its own row
                                    means and records, and its carry (analyze.py:383-398) is block b-1 of the same launch,
-                                   or the last block of the previous launch for b = 0 */
+                                   or the last block of the previous launch for b = 0.
+                                   With nperseg 256 and blocks_per_launch > 1, the register kernel needs block_samples to be
+                                   a multiple of 8 (16-byte aligned blocks): otherwise RT_FFT_AUTO runs the generic kernel and
+                                   RT_FFT_REG256 is rejected by rt_engine_create */
     int32_t reserved[3];        /* zero */
 } rt_config;
 

@@ -23,6 +23,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -867,6 +868,11 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     if (cfg->launch_streams == 2 && cfg->scan_schedule == RT_SCAN_SERIAL) return fail(RT_ERR_INVALID, "two launch streams need an overlapped scan schedule");
     if (cfg->chunk_segs < 0 || cfg->chunk_segs % (PERM_TG > 2 ? 4 * PERM_TG : 8) != 0) return fail(RT_ERR_INVALID, "chunk_segs must be 0 (auto) or a multiple of 8");
     if (cfg->fft_impl == RT_FFT_TC256 && bpl != 1) return fail(RT_ERR_INVALID, "RT_FFT_TC256 does not take blocks_per_launch > 1");
+    // the register kernel reads every unit's segments with 16-byte bulk copies: with blocks_per_launch > 1 the units of a stream
+    // lie block_bytes apart, so the block must be a multiple of 16 bytes.  The PERM layout is fixed here, so this is decided here.
+    const bool reg256_unaligned = n == 256 && bpl > 1 && (2 * cfg->block_samples) % 16 != 0;
+    if (cfg->fft_impl == RT_FFT_REG256 && reg256_unaligned)
+        return fail(RT_ERR_INVALID, "RT_FFT_REG256 with blocks_per_launch > 1 needs block_samples to be a multiple of 8");
     for (int r : cfg->reserved) if (r != 0) return fail(RT_ERR_INVALID, "rt_config.reserved must be zero");
 
     int ndev = 0;
@@ -888,7 +894,7 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     e->n_units = cfg->n_streams * bpl;
     e->block_bytes = 2 * (size_t)cfg->block_samples;
     e->n_probes = (e->T + cfg->probe_stride - 1) / cfg->probe_stride;
-    e->reg256 = (n == 256) && (cfg->fft_impl != RT_FFT_GENERIC);
+    e->reg256 = (n == 256) && (cfg->fft_impl != RT_FFT_GENERIC) && !reg256_unaligned;     // RT_FFT_AUTO: generic kernel then
     e->tc256 = cfg->fft_impl == RT_FFT_TC256;
     e->r16 = (n == 1024 || n == 4096) && cfg->fft_impl == RT_FFT_AUTO;
 #ifdef RT_LAB
@@ -1059,8 +1065,15 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     }
 #endif
     if (!e->reg256) {
-        const size_t smem = (size_t)n * (2 * sizeof(float2) + sizeof(float)) + 16;
-        CUE(cudaFuncSetAttribute(spectro_generic<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        // the limit belongs to the kernel, not to this engine: only ever raise it, or an engine created later with a smaller
+        // nperseg would make every launch of a larger one in the same process fail
+        const int smem = (int)((size_t)n * (2 * sizeof(float2) + sizeof(float)) + 16);
+        static std::mutex attr_mu;                  // engines may be created from several threads
+        std::lock_guard<std::mutex> lock(attr_mu);
+        cudaFuncAttributes ga;
+        CUE(cudaFuncGetAttributes(&ga, spectro_generic<256>));
+        if (ga.maxDynamicSharedSizeBytes < smem)
+            CUE(cudaFuncSetAttribute(spectro_generic<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     } else {
         CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256, cudaFuncAttributeMaxDynamicSharedMemorySize, R256Prod::SMEM)));
         CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));

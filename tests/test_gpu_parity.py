@@ -185,6 +185,9 @@ def test_engine_rejects_bad_configuration():
     with pytest.raises(E.EngineError):
         E.Engine(n_streams=1, block_samples=300, nperseg=256, window=np.ones(256), sample_rate=1e5,
                  signal_threshold=1e-9, snr_threshold=3.0, probe_stride=1, min_cols=0, max_cols=10)
+    with pytest.raises(E.EngineError):       # register kernel, several blocks per launch, blocks not a multiple of 16 bytes
+        E.Engine(n_streams=1, block_samples=250_123, nperseg=256, window=np.hamming(256), sample_rate=3e5, signal_threshold=1e-9,
+                 snr_threshold=3.0, probe_stride=1, min_cols=0, max_cols=10, fft_impl=E.FFT_REG256, blocks_per_launch=2)
     with pytest.raises(IndexError):          # one-column block: analyze.py:354
         BatchAnalyzer(**parity.batch_kwargs(dict(BY_NAME["c1_default_300k"].analyzer_kwargs(), sdr_callback_length=300)))
 
@@ -395,7 +398,7 @@ def _extreme_blocks(n_samples, rng):
     return dict(full_scale=full, all_high=hi, split_iq=split, dc_offset_tone=off)
 
 
-@pytest.mark.parametrize("nperseg", [256, 1024, 4096])
+@pytest.mark.parametrize("nperseg", [8, 32, 128, 256, 1024, 2048, 4096])
 def test_extreme_byte_patterns_match_the_float64_spectrogram(nperseg):
     fs, n_samples = 2_400_000, 64 * 4096 + 77                                     # ragged tail: the last partial segment is dropped
     rng = np.random.default_rng(20261018)
