@@ -38,7 +38,8 @@ enum {
 
 /* fft_impl selector: which spectrogram kernel runs (tests compare them). */
 enum {
-    RT_FFT_AUTO = 0,      /* nperseg 256: RT_FFT_REG256; 1024 / 4096: radix-16 Stockham kernel (spectro_r16.cuh); otherwise RT_FFT_GENERIC */
+    RT_FFT_AUTO = 0,      /* nperseg 256: RT_FFT_REG256; 1024 / 4096: radix-16 Stockham kernel (spectro_r16.cuh); otherwise RT_FFT_GENERIC.
+                           * RT_SAMPLE_CI16 / RT_SAMPLE_CF32: always RT_FFT_GENERIC */
     RT_FFT_GENERIC = 1,   /* shared-memory Stockham FFT, any power-of-two nperseg */
     RT_FFT_REG256 = 2,    /* nperseg 256: 16x16 FFT in registers (packed fp32x2), TMA-fed */
     RT_FFT_TC256 = 3      /* nperseg 256, boxcar/hann/hamming: first FFT stage on the tensor cores (tcgen05, fp16 x split-fp16 -> fp32).
@@ -46,6 +47,26 @@ enum {
                            * rest of the segment mean is removed from the bins 0 and +-1 afterwards, so captures whose DC offset is far
                            * from 128 (tens of LSB) lose precision in exactly those three bins (tests/test_gpu_parity.py, extreme byte
                            * patterns); the default kernels subtract the exact mean per sample and have no such limit. */
+};
+
+/* sample_format: the element type of the interleaved I,Q input, named after the SigMF datatypes.  The spectrogram is that of the
+ * normalised complex samples below; the thresholds apply to them (calibration_db absorbs the receiver's gain).
+ *   format           element         normalised sample   bytes per complex sample   kernels
+ *   RT_SAMPLE_CU8    uint8 I, Q      b / 127.5 - 1       2                          every RT_FFT_* (pyrtlsdr, RTL-SDR)
+ *   RT_SAMPLE_CI8    int8 I, Q       v / 128             2                          every RT_FFT_* (v ^ 0x80 is a cu8 byte)
+ *   RT_SAMPLE_CI16   int16 LE I, Q   v / 32768           4                          RT_FFT_GENERIC (RT_FFT_AUTO picks it)
+ *   RT_SAMPLE_CF32   float32 LE I, Q x as stored         8                          RT_FFT_GENERIC (RT_FFT_AUTO picks it)
+ * RT_FFT_REG256 and RT_FFT_TC256 with RT_SAMPLE_CI16 / RT_SAMPLE_CF32 are rejected by rt_engine_create.
+ * Accuracy limit of RT_SAMPLE_CF32: the segment mean is an fp32 sum (fixed order: per thread, then a shuffle tree, then the
+ * warps in order) whose error is at most about (nperseg / 256 + 13) * 2^-24 * max|x|.  Where the DC offset dominates, the
+ * centred samples x - mean are exact (Sterbenz), so that error is one constant per segment, which the window carries into the
+ * bins where its DFT lives (bin 0, and +-1 for hann / hamming).  A capture with a DC offset D far above its signals loses
+ * precision in those bins only: an absolute error of up to about 1.7e-6 * D (nperseg 4096; 8.3e-7 * D at 256) per sample */
+enum {
+    RT_SAMPLE_CU8 = 0,
+    RT_SAMPLE_CI8 = 1,
+    RT_SAMPLE_CI16 = 2,
+    RT_SAMPLE_CF32 = 3
 };
 
 /* scan_schedule: where the scan kernels (row mean, probe, extraction) of a launch run. */
@@ -89,7 +110,8 @@ typedef struct rt_config {
                                    With nperseg 256 and blocks_per_launch > 1, the register kernel needs block_samples to be
                                    a multiple of 8 (16-byte aligned blocks): otherwise RT_FFT_AUTO runs the generic kernel and
                                    RT_FFT_REG256 is rejected by rt_engine_create */
-    int32_t reserved[3];        /* zero */
+    int32_t sample_format;      /* RT_SAMPLE_* (0 = RT_SAMPLE_CU8: uint8 bytes, as before this field existed) */
+    int32_t reserved[2];        /* zero */
 } rt_config;
 
 /*
@@ -140,9 +162,10 @@ int rt_engine_reset_stream(rt_engine *e, int32_t stream);
 
 /*
  * One callback for every stream of the batch (analyze.py:234-248 without the shadow
- * filter): `iq` holds, for every stream, blocks_per_launch consecutive blocks of 2*block_samples
- * interleaved uint8 I,Q bytes, stream s starting at iq + s*stream_stride_bytes.  iq_on_device != 0:
- * `iq` is a device pointer (no copy); otherwise a host pointer (pinned or pageable) that is copied in.
+ * filter): `iq` holds, for every stream, blocks_per_launch consecutive blocks of block_samples
+ * interleaved I,Q samples in rt_config.sample_format (bytes_per_sample * block_samples bytes each, RT_SAMPLE_*),
+ * stream s starting at iq + s*stream_stride_bytes.  iq_on_device != 0: `iq` is a device pointer (no copy), aligned, like
+ * stream_stride_bytes, to one complex sample (2, 4 or 8 bytes); otherwise a host pointer (pinned or pageable) that is copied in.
  * Blocks until done.  Records come back sorted by (stream, fi, start).
  * On RT_ERR_OVERFLOW *n_out is the number that would have been needed and `out` holds the first
  * min(max_out, max_records) of them.

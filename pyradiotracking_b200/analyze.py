@@ -179,7 +179,12 @@ class BatchAnalyzer:
                  signal_threshold_dbw: float, snr_threshold_db: float, sdr_callback_length: Optional[int] = None,
                  cuda_device: int = 0, max_records: int = 0, fft_impl: int = _engine.FFT_AUTO,
                  scan_schedule: int = _engine.SCAN_AUTO, launch_streams: int = 0, chunk_segs: int = 0,
-                 blocks_per_launch: int = 1):
+                 blocks_per_launch: int = 1, sample_format: str = "cu8"):
+        """`sample_format`: the SigMF datatype of the input blocks, one of `engine.SAMPLE_FORMATS` (cu8: RTL-SDR bytes, ci8, ci16_le,
+        cf32_le); the thresholds apply to the normalised samples (INTEGRATION.md)."""
+        if sample_format not in _engine.SAMPLE_FORMATS:
+            raise ValueError(f"sample_format = {sample_format!r}: the B200 engine reads {', '.join(_engine.SAMPLE_FORMATS)} (see INTEGRATION.md)")
+        self.sample_format = sample_format
         self.devices = [str(d) for d in devices]
         self.n_streams = len(self.devices)
         self.calibration_db = [float(c) for c in calibration_db]
@@ -227,7 +232,7 @@ class BatchAnalyzer:
                 probe_stride=self.plan.stride, min_cols=self.plan.min_cols, max_cols=self.plan.max_cols,
                 max_records=self.max_records, cuda_device=self.cuda_device, fft_impl=self.fft_impl,
                 scan_schedule=self.scan_schedule, launch_streams=self.launch_streams, chunk_segs=self.chunk_segs,
-                blocks_per_launch=self.blocks_per_launch)
+                blocks_per_launch=self.blocks_per_launch, sample_format=self.sample_format)
         return self._engine
 
     def close(self):
@@ -368,8 +373,9 @@ class BatchAnalyzer:
         return out
 
     def process_blocks(self, iq, ts_start: Sequence[datetime.datetime]):
-        """`iq`: uint8 `[n_streams, 2*block_samples]` (`[n_streams, blocks_per_launch, 2*block_samples]`) on the host, or a
-        CUDA tensor of that shape.  -> per analyzer unit `(filtered_signals, all_signals, keys)`."""
+        """`iq`: `[n_streams, 2*block_samples]` (`[n_streams, blocks_per_launch, 2*block_samples]`) interleaved I,Q elements of
+        the analyzer's `sample_format` (uint8, int8, int16 or float32; cf32_le also complex64 with `block_samples` per block) on
+        the host, or a CUDA tensor of that shape.  -> per analyzer unit `(filtered_signals, all_signals, keys)`."""
         self.submit(iq)
         return self.collect(ts_start, with_all=True)
 

@@ -16,7 +16,7 @@ LIB = os.path.join(CSRC, "librtb200.so")
 PYFINAL_SRC = os.path.join(CSRC, "rt_pyfinal.c")
 PYFINAL = os.path.join(HERE, "_rtfinal.so")
 SOURCES = ["rt_engine.cu", "rt_matcher.cpp"]
-HEADERS = ["predicate.h", "fft_cpk.cuh", "spectro256.cuh", "spectro_tc256.cuh", "spectro_r16.cuh", os.path.join("..", "..", "include", "rt_engine.h"),
+HEADERS = ["predicate.h", "sample_format.cuh", "fft_cpk.cuh", "spectro256.cuh", "spectro_tc256.cuh", "spectro_r16.cuh", os.path.join("..", "..", "include", "rt_engine.h"),
            os.path.join("..", "..", "include", "rt_matcher.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

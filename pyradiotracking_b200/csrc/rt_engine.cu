@@ -6,7 +6,7 @@
 // extract_signals' probe / backward / forward scans and per-signal statistics.
 //
 // Kernels (one launch each per engine call, all streams of the batch at once):
-//   spectro_*      uint8 IQ -> power cells S (fp32, layout per kernel) + row sums / row means
+//   spectro_*      IQ samples (rt_config.sample_format) -> power cells S (fp32, layout per kernel) + row sums / row means
 //   probe          prologue: deterministic reduction of the chunk sums -> freq_avg[stream][bin] (the tensor-core
 //                  kernel does this itself in the last warp-group run of each stream); then one thread per
 //                  (stream, bin, 8 probe columns k*stride): predicate test, cheap pruning of short noise runs,
@@ -29,6 +29,7 @@
 
 #include "../../include/rt_engine.h"
 #include "predicate.h"
+#include "sample_format.cuh"
 #include "spectro256.cuh"
 #include "spectro_tc256.cuh"
 #include "spectro_r16.cuh"
@@ -87,6 +88,7 @@ using R256Prod = rt::R256v7T<4, 4, PERM_LMAP>;
 // time groupings (tools/build_lab_lib.sh, RT_PERM_TG = 1 | 4 | 8) keep v7n, which knows all of them
 #if RT_PERM_TG == 2
 #define RT_SPECTRO_REG256 rt::spectro_reg256_v8<true, 2>
+#define RT_SPECTRO_REG256_CI8 rt::spectro_reg256_v8<true, 2, true>
 #else
 #define RT_SPECTRO_REG256 rt::spectro_reg256_v7n<true, PERM_TG, PERM_LMAP>
 #endif
@@ -131,7 +133,7 @@ struct CellRef {
 // ---------------------------------------------------------------------------------------------
 using rt::SpectroArgs;
 
-template <int NT>
+template <int NT, int FMT>
 __global__ void __launch_bounds__(NT) spectro_generic(SpectroArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int n = a.n;
@@ -147,33 +149,10 @@ __global__ void __launch_bounds__(NT) spectro_generic(SpectroArgs a) {
     for (int i = tid; i < n; i += NT) rowacc[i] = 0.f;
 
     for (int seg = seg0; seg < seg1; ++seg) {
-        const uchar2* src = reinterpret_cast<const uchar2*>(a.unit_base(s) + (size_t)seg * 2 * n);
-        if (tid == 0) sums[0] = sums[1] = 0;
-        __syncthreads();
-        // scipy detrend='constant': the segment's complex mean; byte sums are exact integers
-        int sI = 0, sQ = 0;
-        for (int i = tid; i < n; i += NT) {
-            uchar2 v = src[i];
-            sI += v.x;
-            sQ += v.y;
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            sI += __shfl_xor_sync(0xffffffffu, sI, o);
-            sQ += __shfl_xor_sync(0xffffffffu, sQ, o);
-        }
-        if ((tid & 31) == 0) {
-            atomicAdd(&sums[0], sI);
-            atomicAdd(&sums[1], sQ);
-        }
-        __syncthreads();
-        const float mI = (float)sums[0] / (float)n;   // exact: sum < 2^24, n a power of two
-        const float mQ = (float)sums[1] / (float)n;
-        for (int i = tid; i < n; i += NT) {
-            uchar2 v = src[i];
-            float w = a.win[i];
-            buf0[i] = make_float2(((float)v.x - mI) * w, ((float)v.y - mQ) * w);
-        }
+        // scipy detrend='constant' (the segment's complex mean) and the window, per sample format (sample_format.cuh); buf1 is
+        // free until the first FFT pass
+        using In = rt::SegmentIn<FMT>;
+        In::template centre<NT>(a.unit_base(s) + (size_t)seg * In::BYTES * n, n, tid, a.win, buf0, sums, buf1);
         __syncthreads();
         float2* X = buf0;
         float2* Y = buf1;
@@ -225,6 +204,17 @@ __global__ void __launch_bounds__(NT) spectro_generic(SpectroArgs a) {
     }
     float* pd = a.part + ((size_t)s * a.n_chunks + blockIdx.x) * n;
     for (int i = tid; i < n; i += NT) pd[i] = rowacc[i];
+}
+
+// the generic kernel's instantiation for a sample format (RT_SAMPLE_*, validated by rt_engine_create)
+using SpectroKernel = void (*)(SpectroArgs);
+SpectroKernel generic_kernel(int fmt) {
+    switch (fmt) {
+        case RT_SAMPLE_CI8: return spectro_generic<256, RT_SAMPLE_CI8>;
+        case RT_SAMPLE_CI16: return spectro_generic<256, RT_SAMPLE_CI16>;
+        case RT_SAMPLE_CF32: return spectro_generic<256, RT_SAMPLE_CF32>;
+        default: return spectro_generic<256, RT_SAMPLE_CU8>;
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -700,7 +690,9 @@ struct rt_engine {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     int n = 0, T = 0, n_streams = 0, bpl = 1, n_units = 0, n_chunks = 0, chunk_segs = 0, n_probes = 0;
-    size_t block_bytes = 0;
+    size_t block_bytes = 0;                  // bytes per block of one stream: bytes per complex sample * block_samples
+    int sample_bytes = 2;                    // bytes per complex sample (rt_config.sample_format)
+    bool ci8 = false;                        // RT_SAMPLE_CI8: the byte kernels' int8 instantiations
     int max_work = 0;                        // capacity of d_work
     int max_records = 0;                     // effective capacity of one launch's record list
     bool reg256 = false;                     // nperseg 256: register kernel (v7n) or tensor-core kernel
@@ -868,9 +860,17 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     if (cfg->launch_streams == 2 && cfg->scan_schedule == RT_SCAN_SERIAL) return fail(RT_ERR_INVALID, "two launch streams need an overlapped scan schedule");
     if (cfg->chunk_segs < 0 || cfg->chunk_segs % (PERM_TG > 2 ? 4 * PERM_TG : 8) != 0) return fail(RT_ERR_INVALID, "chunk_segs must be 0 (auto) or a multiple of 8");
     if (cfg->fft_impl == RT_FFT_TC256 && bpl != 1) return fail(RT_ERR_INVALID, "RT_FFT_TC256 does not take blocks_per_launch > 1");
+    rt::SampleFormatInfo fmt;
+    if (!rt::sample_format_info(cfg->sample_format, &fmt)) return fail(RT_ERR_INVALID, "unknown sample_format");
+    const bool byte_fmt = rt::sample_format_is_byte(cfg->sample_format);
+    if (!byte_fmt && (cfg->fft_impl == RT_FFT_REG256 || cfg->fft_impl == RT_FFT_TC256))
+        return fail(RT_ERR_INVALID, "RT_FFT_REG256 / RT_FFT_TC256 read bytes: RT_SAMPLE_CI16 / RT_SAMPLE_CF32 run on RT_FFT_GENERIC");
+#if RT_PERM_TG != 2
+    if (cfg->sample_format == RT_SAMPLE_CI8 && n == 256 && cfg->fft_impl != RT_FFT_GENERIC) return fail(RT_ERR_INVALID, "lab builds: ci8 at nperseg 256 needs RT_FFT_GENERIC");
+#endif
     // the register kernel reads every unit's segments with 16-byte bulk copies: with blocks_per_launch > 1 the units of a stream
     // lie block_bytes apart, so the block must be a multiple of 16 bytes.  The PERM layout is fixed here, so this is decided here.
-    const bool reg256_unaligned = n == 256 && bpl > 1 && (2 * cfg->block_samples) % 16 != 0;
+    const bool reg256_unaligned = n == 256 && bpl > 1 && (fmt.bytes * cfg->block_samples) % 16 != 0;
     if (cfg->fft_impl == RT_FFT_REG256 && reg256_unaligned)
         return fail(RT_ERR_INVALID, "RT_FFT_REG256 with blocks_per_launch > 1 needs block_samples to be a multiple of 8");
     for (int r : cfg->reserved) if (r != 0) return fail(RT_ERR_INVALID, "rt_config.reserved must be zero");
@@ -892,11 +892,13 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     e->n_streams = cfg->n_streams;
     e->bpl = bpl;
     e->n_units = cfg->n_streams * bpl;
-    e->block_bytes = 2 * (size_t)cfg->block_samples;
+    e->sample_bytes = fmt.bytes;
+    e->ci8 = cfg->sample_format == RT_SAMPLE_CI8;
+    e->block_bytes = (size_t)fmt.bytes * (size_t)cfg->block_samples;
     e->n_probes = (e->T + cfg->probe_stride - 1) / cfg->probe_stride;
-    e->reg256 = (n == 256) && (cfg->fft_impl != RT_FFT_GENERIC) && !reg256_unaligned;     // RT_FFT_AUTO: generic kernel then
+    e->reg256 = (n == 256) && (cfg->fft_impl != RT_FFT_GENERIC) && !reg256_unaligned && byte_fmt;     // RT_FFT_AUTO: generic kernel then
     e->tc256 = cfg->fft_impl == RT_FFT_TC256;
-    e->r16 = (n == 1024 || n == 4096) && cfg->fft_impl == RT_FFT_AUTO;
+    e->r16 = (n == 1024 || n == 4096) && cfg->fft_impl == RT_FFT_AUTO && byte_fmt;
 #ifdef RT_LAB
     if (e->r16 && rt_lab_s256) { e->r16 = false; e->s256 = true; }
 #endif
@@ -946,12 +948,12 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     CUE(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     e->own_stream = true;
 
-    // window with the density scaling and the 1/127.5 byte scale folded in:
-    // S = |FFT(w (x - mean))|^2 / (fs sum w^2),  x = b/127.5 - 1  =>  S = |FFT(w' (b - mean_b))|^2
+    // window with the density scaling and the full scale of the sample format folded in (sample_format.cuh):
+    // S = |FFT(w (x - mean))|^2 / (fs sum w^2),  x = b / scale (- 1 for cu8)  =>  S = |FFT(w' (b - mean_b))|^2
     double sw2 = 0.0;
     for (int i = 0; i < n; ++i) sw2 += cfg->window[i] * cfg->window[i];
     if (!(sw2 > 0)) { free_engine(e); return fail(RT_ERR_INVALID, "window has no energy"); }
-    const double amp = std::sqrt(1.0 / (cfg->sample_rate * sw2)) / 127.5;
+    const double amp = std::sqrt(1.0 / (cfg->sample_rate * sw2)) / fmt.full_scale;
     std::vector<float> hwin(n);
     for (int i = 0; i < n; ++i) hwin[i] = (float)(cfg->window[i] * amp);
     int sms = 0;
@@ -994,7 +996,8 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     if (e->tc256) {
         CUE(cudaMalloc(&e->d_bmat, e->tc_tab.bmat.size() * sizeof(uint16_t)));
         CUE(cudaMemcpy(e->d_bmat, e->tc_tab.bmat.data(), e->tc_tab.bmat.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
-        CUE(cudaFuncSetAttribute(rt::spectro_tc256_k<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::Tc256<2>::SMEM));
+        if (e->ci8) CUE((cudaFuncSetAttribute(rt::spectro_tc256_k<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::Tc256<2>::SMEM)));
+        else CUE(cudaFuncSetAttribute(rt::spectro_tc256_k<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::Tc256<2>::SMEM));
     }
     CUE(cudaMalloc(&e->d_thr, e->n_units * sizeof(float)));
     CUE(cudaMalloc(&e->d_hasprev, e->n_units * sizeof(int)));
@@ -1057,6 +1060,8 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
         CUE(cudaMemcpy(e->d_tw1, htw1.data(), htw1.size() * sizeof(float2), cudaMemcpyHostToDevice));
         if (n == 4096) CUE(cudaFuncSetAttribute(rt::spectro_r16_k<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<4096>::SMEM));
         else CUE(cudaFuncSetAttribute(rt::spectro_r16_k<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<1024>::SMEM));
+        if (e->ci8 && n == 4096) CUE((cudaFuncSetAttribute(rt::spectro_r16_k<4096, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<4096>::SMEM)));
+        if (e->ci8 && n == 1024) CUE((cudaFuncSetAttribute(rt::spectro_r16_k<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<1024>::SMEM)));
     }
 #ifdef RT_LAB
     if (e->s256) {
@@ -1070,10 +1075,16 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
         const int smem = (int)((size_t)n * (2 * sizeof(float2) + sizeof(float)) + 16);
         static std::mutex attr_mu;                  // engines may be created from several threads
         std::lock_guard<std::mutex> lock(attr_mu);
+        const SpectroKernel gk = generic_kernel(cfg->sample_format);
         cudaFuncAttributes ga;
-        CUE(cudaFuncGetAttributes(&ga, spectro_generic<256>));
+        CUE(cudaFuncGetAttributes(&ga, gk));
         if (ga.maxDynamicSharedSizeBytes < smem)
-            CUE(cudaFuncSetAttribute(spectro_generic<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            CUE(cudaFuncSetAttribute(gk, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    } else if (e->ci8) {
+#ifdef RT_SPECTRO_REG256_CI8
+        CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256_CI8, cudaFuncAttributeMaxDynamicSharedMemorySize, R256Prod::SMEM)));
+        CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256_CI8, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
+#endif
     } else {
         CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256, cudaFuncAttributeMaxDynamicSharedMemorySize, R256Prod::SMEM)));
         CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
@@ -1151,6 +1162,8 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         d_iq = e->d_stage[sb];
         stride = e->stage_stride;
     }
+    if (((uintptr_t)d_iq | (e->n_streams > 1 ? stride : 0)) % (uintptr_t)e->sample_bytes != 0)
+        return fail(RT_ERR_INVALID, "IQ pointer / stream stride not aligned to one complex sample");
     const bool aligned = (((uintptr_t)d_iq | stride | (e->bpl > 1 ? e->block_bytes : 0)) & 15) == 0;
     if (e->reg256 && !aligned) return fail(RT_ERR_INVALID, "register FFT path needs 16-byte aligned IQ, stream stride and (blocks_per_launch > 1) block size");
     const int slot = (int)(e->launch_seq % RT_SLOTS);
@@ -1199,8 +1212,13 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         ta.S = e->d_S[next]; ta.S_stream_stride = e->s_stride;
         ta.part = e->d_part[slot]; ta.part_slots = e->tc_slots; ta.avg = e->d_avg[slot]; ta.ctr = e->d_ctr[slot];
         ta.store = 1; ta.dbg = 0; ta.prof = nullptr;
-        rt::spectro_tc256_k<2><<<e->tc_grid, 512, rt::Tc256<2>::SMEM, st>>>(ta);
+        if (e->ci8) rt::spectro_tc256_k<2, true><<<e->tc_grid, 512, rt::Tc256<2>::SMEM, st>>>(ta);
+        else rt::spectro_tc256_k<2><<<e->tc_grid, 512, rt::Tc256<2>::SMEM, st>>>(ta);
     } else if (use_reg) {
+#ifdef RT_SPECTRO_REG256_CI8
+        if (e->ci8) RT_SPECTRO_REG256_CI8<<<grid, R256Prod::THREADS, R256Prod::SMEM, st>>>(sa);
+        else
+#endif
         RT_SPECTRO_REG256<<<grid, R256Prod::THREADS, R256Prod::SMEM, st>>>(sa);
 #ifdef RT_LAB
     } else if (e->s256 && aligned) {
@@ -1208,11 +1226,16 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         else rt::spectro_s256_k<1024><<<grid, 256, rt::S256Cfg<1024>::SMEM, st>>>(sa);
 #endif
     } else if (e->r16 && aligned) {
-        if (e->n == 4096) rt::spectro_r16_k<4096><<<grid, 256, rt::R16Cfg<4096>::SMEM, st>>>(sa);
-        else rt::spectro_r16_k<1024><<<grid, 256, rt::R16Cfg<1024>::SMEM, st>>>(sa);
+        if (e->n == 4096) {
+            if (e->ci8) rt::spectro_r16_k<4096, true><<<grid, 256, rt::R16Cfg<4096>::SMEM, st>>>(sa);
+            else rt::spectro_r16_k<4096><<<grid, 256, rt::R16Cfg<4096>::SMEM, st>>>(sa);
+        } else {
+            if (e->ci8) rt::spectro_r16_k<1024, true><<<grid, 256, rt::R16Cfg<1024>::SMEM, st>>>(sa);
+            else rt::spectro_r16_k<1024><<<grid, 256, rt::R16Cfg<1024>::SMEM, st>>>(sa);
+        }
     } else {
         const size_t smem = (size_t)e->n * (2 * sizeof(float2) + sizeof(float)) + 16;
-        spectro_generic<256><<<grid, 256, smem, st>>>(sa);
+        generic_kernel(e->cfg.sample_format)<<<grid, 256, smem, st>>>(sa);
     }
     CU(cudaGetLastError());
     if (evs) CU(cudaEventRecord(evs->ev[1], st));

@@ -20,7 +20,7 @@ struct SpectroArgs {
     const uint8_t* iq;
     size_t stream_stride;
     int n, T, chunk_segs, n_chunks;
-    const float* win;      // window * sqrt(1/(fs*sum(w^2))) / 127.5
+    const float* win;      // window * sqrt(1/(fs*sum(w^2))) / full scale of the sample format (127.5 for cu8, sample_format.cuh)
     const float2* tw;      // exp(-2 pi i k / n)
     const float2* tw1 = nullptr;   // spectro_r16: pass-1 twiddles exp(-2 pi i (b i) / n) as [i - 1][b], i = 1..15, b < n / 16
     float* S;              // generic kernel: [stream][T][n]; register kernel: [stream][T][pos(bin)] (see rt_engine.cu)
@@ -440,7 +440,7 @@ __global__ void __launch_bounds__(R256v7::THREADS, 4) spectro_reg256_v7n(Spectro
 // TMA loads and / or the S stores -- all within +-0.5 us; integer detrend + I2F (a non-FMA pipe) instead of FHADD: 32 FMA-pipe cycles
 // less but 56 instructions more per round, 168 us -- issue slots and the FMA pipe bind together.
 // ---------------------------------------------------------------------------------------------
-template <bool STORE, int TG, class C = R256v7T<4, 4, true>>
+template <bool STORE, int TG, bool CI8 = false, class C = R256v7T<4, 4, true>>
 __device__ __forceinline__ void spectro_reg256_v8_body(const SpectroArgs& a) {
     static_assert(TG == 1 || TG == 2, "time group");
     static_assert(C::LMAP, "v8 uses the LMAP lane mapping");
@@ -509,9 +509,10 @@ __device__ __forceinline__ void spectro_reg256_v8_body(const SpectroArgs& a) {
 
     for (int it = 0; it < n_it; ++it) {
         // this thread's 16 samples as fp16 pairs (1024 + I) | (1024 + Q) << 16, and the segment's byte sums from the same words
+        // (ci8: one LOP3 per sample turns the int8 pair into the cu8 pair v + 128, sample_format.cuh)
         unsigned hv[16];
 #pragma unroll
-        for (int n1 = 0; n1 < 16; ++n1) hv[n1] = __byte_perm(lds_u16(my_u16 + st_off + 32 * n1), 0x64646464u, 0x5140);
+        for (int n1 = 0; n1 < 16; ++n1) hv[n1] = __byte_perm(lds_u16(my_u16 + st_off + 32 * n1) ^ (CI8 ? 0x8080u : 0u), 0x64646464u, 0x5140);
         unsigned t = 0;
 #pragma unroll
         for (int n1 = 0; n1 < 16; ++n1) t += hv[n1];
@@ -590,9 +591,9 @@ __device__ __forceinline__ void spectro_reg256_v8_body(const SpectroArgs& a) {
     }
 }
 
-template <bool STORE, int TG = 2>
+template <bool STORE, int TG = 2, bool CI8 = false>
 __global__ void __launch_bounds__(R256v7::THREADS, 4) spectro_reg256_v8(SpectroArgs a) {
-    spectro_reg256_v8_body<STORE, TG>(a);
+    spectro_reg256_v8_body<STORE, TG, CI8>(a);
 }
 
 }  // namespace rt

@@ -67,7 +67,8 @@ __device__ __forceinline__ void r16_lds_tw(uint32_t addr, float& wr, float& wi) 
     asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(wr), "=f"(wi) : "r"(addr));
 }
 
-template <int N>
+// CI8: int8 input, taken as cu8 with the top bit of every byte flipped (sample_format.cuh)
+template <int N, bool CI8 = false>
 __global__ void __maxnreg__(R16Cfg<N>::MAXR) spectro_r16_k(SpectroArgs a) {
     using C = R16Cfg<N>;
     constexpr int BT = C::BT, M1 = N / 16, M2 = N / 256;
@@ -148,7 +149,7 @@ __global__ void __maxnreg__(R16Cfg<N>::MAXR) spectro_r16_k(SpectroArgs a) {
         unsigned packed = 0;
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
-            u[i] = __byte_perm(lds_u16(rb + i * (2 * M1)), 0x64646464u, 0x5140);
+            u[i] = __byte_perm(lds_u16(rb + i * (2 * M1)) ^ (CI8 ? 0x8080u : 0u), 0x64646464u, 0x5140);
             packed += u[i];
         }
         packed -= 0x40064000u;                                 // I in the low half, Q in the high half (each <= 16 * 255)

@@ -105,7 +105,7 @@ inline float tc_half_val(uint16_t u) {
     return __half2float(h);
 }
 
-// window[n] as scipy returns it; amp = sqrt(1 / (fs * sum w^2)) / 127.5
+// window[n] as scipy returns it; amp = sqrt(1 / (fs * sum w^2)) / 127.5 (cu8) or / 128 (ci8)
 inline TcTables tc_make_tables(const double* window, double amp) {
     TcTables t;
     double wmax = 0;
@@ -208,7 +208,8 @@ __device__ __forceinline__ void octet_transpose_reduce32(float (&v)[32], int lan
 #undef RT_TR_STEP
 }
 
-template <int NG>
+// CI8: int8 input, taken as cu8 with the top bit of every byte flipped (sample_format.cuh)
+template <int NG, bool CI8 = false>
 __global__ void __launch_bounds__(512, 1) spectro_tc256_k(TcArgs a) {
     using C = Tc256<NG>;
     extern __shared__ __align__(128) unsigned char tc_smem[];
@@ -330,7 +331,7 @@ __global__ void __launch_bounds__(512, 1) spectro_tc256_k(TcArgs a) {
                 const int row = wg + C::GROUP_WARPS * i;
                 const uint32_t* src = reinterpret_cast<const uint32_t*>(base + (size_t)row * 512 + 128 * cc + 4 * pp);
 #pragma unroll
-                for (int u = 0; u < 4; ++u) w[i][u] = (row < nseg) ? __ldg(src + 8 * u) : 0x80808080u;
+                for (int u = 0; u < 4; ++u) w[i][u] = (row < nseg) ? (__ldg(src + 8 * u) ^ (CI8 ? 0x80808080u : 0u)) : 0x80808080u;   // ci8: + 128 per byte
             }
 #pragma unroll
             for (int i = 0; i < 8; ++i) {

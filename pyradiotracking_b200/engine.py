@@ -5,6 +5,7 @@ CPU fallback: if the shared library is missing or no CUDA device is present, cre
 an `Engine` raises.
 """
 import ctypes
+import functools
 import logging
 import os
 from typing import Optional, Sequence, Tuple, Union
@@ -17,6 +18,27 @@ RT_OK, RT_ERR_INVALID, RT_ERR_CUDA, RT_ERR_OVERFLOW, RT_ERR_STATE = 0, -1, -2, -
 RT_ABI_VERSION = 2
 FFT_AUTO, FFT_GENERIC, FFT_REG256, FFT_TC256 = 0, 1, 2, 3
 SCAN_AUTO, SCAN_SERIAL, SCAN_OVERLAP, SCAN_LEAN = 0, 1, 2, 3
+SAMPLE_CU8, SAMPLE_CI8, SAMPLE_CI16, SAMPLE_CF32 = 0, 1, 2, 3
+
+# rt_config.sample_format by SigMF datatype: (code, element dtype, bytes per complex sample).  The engine analyses the normalised
+# samples (cu8: b / 127.5 - 1 as pyrtlsdr delivers them, ci8: v / 128, ci16_le: v / 32768, cf32_le: x); include/rt_engine.h
+# has the table and its limits.
+SAMPLE_FORMATS = {
+    "cu8": (SAMPLE_CU8, np.dtype(np.uint8), 2),
+    "ci8": (SAMPLE_CI8, np.dtype(np.int8), 2),
+    "ci16_le": (SAMPLE_CI16, np.dtype("<i2"), 4),
+    "cf32_le": (SAMPLE_CF32, np.dtype("<f4"), 8),
+}
+_FORMAT_BY_CODE = {v[0]: k for k, v in SAMPLE_FORMATS.items()}
+
+
+def sample_format_name(fmt: Union[str, int]) -> str:
+    """The SigMF name of a sample format given by name or by rt_config.sample_format code; ValueError if unknown."""
+    name = _FORMAT_BY_CODE.get(fmt) if isinstance(fmt, (int, np.integer)) and not isinstance(fmt, bool) else fmt
+    if name not in SAMPLE_FORMATS:
+        raise ValueError(f"unknown sample format {fmt!r}: expected one of {', '.join(SAMPLE_FORMATS)}")
+    return name
+
 
 logger = logging.getLogger(__name__)
 
@@ -40,7 +62,7 @@ class RtConfig(ctypes.Structure):
         ("snr_threshold", ctypes.c_double), ("probe_stride", ctypes.c_int32), ("min_cols", ctypes.c_int32),
         ("max_cols", ctypes.c_int32), ("max_records", ctypes.c_int32), ("fft_impl", ctypes.c_int32),
         ("scan_schedule", ctypes.c_int32), ("launch_streams", ctypes.c_int32), ("chunk_segs", ctypes.c_int32),
-        ("blocks_per_launch", ctypes.c_int32), ("reserved", ctypes.c_int32 * 3),
+        ("blocks_per_launch", ctypes.c_int32), ("sample_format", ctypes.c_int32), ("reserved", ctypes.c_int32 * 2),
     ]
 
 
@@ -117,24 +139,34 @@ def device_count() -> int:
     return n
 
 
-def _device_pointer(obj, n_rows: int, row_bytes: int) -> Optional[Tuple[int, int]]:
-    """(pointer, row stride in bytes) if `obj` lives in device memory, else None.  `obj` must be uint8 and hold
-    `n_rows` rows of `row_bytes` contiguous bytes (a 1-D object: one row); a wrong size would be read out of bounds."""
+@functools.lru_cache(maxsize=None)
+def _cai_type(typestr: str) -> Tuple[str, int]:
+    """(numpy name, itemsize) of a __cuda_array_interface__ typestr; the name is empty for a non-native byte order."""
+    dt = np.dtype(typestr)
+    return (dt.name if dt.isnative else ""), dt.itemsize
+
+
+def _device_pointer(obj, n_rows: int, row_bytes: int, dtypes: Tuple[str, ...] = ("uint8",)) -> Optional[Tuple[int, int]]:
+    """(pointer, row stride in bytes) if `obj` lives in device memory, else None.  `obj` must have one of the native-endian
+    element types named in `dtypes` (numpy names; default uint8) and hold `n_rows` rows of `row_bytes` contiguous bytes (a 1-D
+    object: one row); a wrong size would be read out of bounds."""
     if hasattr(obj, "data_ptr") and getattr(obj, "is_cuda", False):      # torch.Tensor, without importing torch
-        if "uint8" not in str(obj.dtype):
-            raise TypeError("IQ blocks must be uint8 interleaved I,Q bytes")
-        shape, strides = tuple(obj.shape), tuple(int(x) for x in obj.stride())
+        if str(obj.dtype)[6:] not in dtypes:                            # "torch.uint8"
+            raise TypeError(f"IQ blocks must be {' / '.join(dtypes)}, got {obj.dtype}")
+        item = obj.element_size()
+        shape, strides = tuple(obj.shape), tuple(int(x) * item for x in obj.stride())
         ptr = int(obj.data_ptr())
     else:
         cai = getattr(obj, "__cuda_array_interface__", None)
         if cai is None:
             return None
-        if cai["typestr"] not in ("|u1", "<u1", ">u1"):
-            raise TypeError("IQ blocks must be uint8 interleaved I,Q bytes")
+        name, item = _cai_type(cai["typestr"])
+        if name not in dtypes:
+            raise TypeError(f"IQ blocks must be {' / '.join(dtypes)}, got {cai['typestr']}")
         shape = tuple(cai["shape"])
         st = cai.get("strides")
-        if st is None:                                                   # C-contiguous: strides in BYTES (itemsize 1)
-            st, acc = [], 1
+        if st is None:                                                   # C-contiguous: strides in BYTES
+            st, acc = [], item
             for d in reversed(shape):
                 st.insert(0, acc)
                 acc *= d
@@ -143,12 +175,12 @@ def _device_pointer(obj, n_rows: int, row_bytes: int) -> Optional[Tuple[int, int
     # the trailing axes of a row must be dense; the leading axis is the stream
     if len(shape) == 1:
         shape, strides = (1,) + shape, (shape[0] * strides[0],) + strides
-    inner, dense = 1, True
+    inner, dense = item, True
     for d, st in zip(reversed(shape[1:]), reversed(strides[1:])):
         dense = dense and (d == 1 or st == inner)
         inner *= d
     if shape[0] != n_rows or inner != row_bytes or not dense:
-        raise ValueError(f"expected uint8 [{n_rows}, {row_bytes}] on the device, got shape {shape} strides {strides}")
+        raise ValueError(f"expected {' / '.join(dtypes)} [{n_rows}, {row_bytes // item}] on the device, got shape {shape} strides {strides}")
     return ptr, (strides[0] if n_rows > 1 else row_bytes)
 
 
@@ -158,7 +190,9 @@ class Engine:
     def __init__(self, *, n_streams: int, block_samples: int, nperseg: int, window: np.ndarray, sample_rate: float,
                  signal_threshold: Union[float, Sequence[float]], snr_threshold: float, probe_stride: int,
                  min_cols: int, max_cols: int, max_records: int = 0, cuda_device: int = 0, fft_impl: int = FFT_AUTO,
-                 scan_schedule: int = SCAN_AUTO, launch_streams: int = 0, chunk_segs: int = 0, blocks_per_launch: int = 1):
+                 scan_schedule: int = SCAN_AUTO, launch_streams: int = 0, chunk_segs: int = 0, blocks_per_launch: int = 1,
+                 sample_format: Union[str, int] = "cu8"):
+        """`sample_format`: the SigMF datatype of the input (`SAMPLE_FORMATS`) or an rt_config.sample_format code."""
         self._lib = load_library()
         self._h = ctypes.c_void_p()
         win = np.ascontiguousarray(window, dtype=np.float64)
@@ -174,8 +208,14 @@ class Engine:
             max_cols=int(max_cols), max_records=int(max_records), fft_impl=int(fft_impl),
             scan_schedule=int(scan_schedule), launch_streams=int(launch_streams), chunk_segs=int(chunk_segs),
             blocks_per_launch=int(blocks_per_launch),
+            sample_format=int(sample_format) if isinstance(sample_format, (int, np.integer)) else SAMPLE_FORMATS[sample_format_name(sample_format)][0],
         )
         _check(self._lib.rt_engine_create(ctypes.byref(cfg), ctypes.byref(self._h)))
+        self.sample_format = sample_format_name(cfg.sample_format)       # the engine accepted it: a known format
+        _, dtype, self.sample_bytes = SAMPLE_FORMATS[self.sample_format]
+        # element types a launch accepts: the format's, and complex64 (an I,Q pair of float32) for cf32
+        self._dtypes = (dtype, np.dtype(np.complex64)) if self.sample_format == "cf32_le" else (dtype,)
+        self._dtype_names = tuple(d.name for d in self._dtypes)
         self.n_streams, self.nperseg, self.block_samples = n_streams, nperseg, block_samples
         self.blocks_per_launch = int(blocks_per_launch)
         self.n_units = n_streams * self.blocks_per_launch      # analyzer units per launch: rt_record.stream counts these
@@ -204,20 +244,24 @@ class Engine:
 
     # -- data path ----------------------------------------------------------------------------
     def _resolve(self, iq) -> Tuple[int, int, int]:
-        row = 2 * self.block_samples * self.blocks_per_launch       # the consecutive blocks of one stream
-        dev = _device_pointer(iq, self.n_streams, row)
+        """(pointer, on device, row stride in bytes) of one launch's input: [n_streams, 2 * block_samples * blocks_per_launch]
+        elements of the engine's sample format (or [n_streams, blocks_per_launch, 2 * block_samples]); cf32 also as complex64 with
+        half as many elements per row."""
+        row = self.sample_bytes * self.block_samples * self.blocks_per_launch       # bytes: the consecutive blocks of one stream
+        dev = _device_pointer(iq, self.n_streams, row, self._dtype_names)
         if dev is not None:
             return dev[0], 1, dev[1]
         arr = np.asarray(iq)
-        if arr.dtype != np.uint8:
-            raise TypeError("IQ blocks must be uint8 interleaved I,Q bytes")
-        if arr.ndim == 3 and arr.shape[1:] == (self.blocks_per_launch, 2 * self.block_samples) and arr[0].flags.c_contiguous:
+        if arr.dtype not in self._dtypes:
+            raise TypeError(f"IQ blocks must be {' / '.join(self._dtype_names)} for sample format {self.sample_format}, got {arr.dtype}")
+        item = arr.itemsize
+        if arr.ndim == 3 and arr.shape[1:] == (self.blocks_per_launch, row // self.blocks_per_launch // item) and arr[0].flags.c_contiguous:
             arr = arr.reshape(arr.shape[0], -1) if arr.flags.c_contiguous else np.lib.stride_tricks.as_strided(
-                arr, (arr.shape[0], row), (arr.strides[0], 1))
+                arr, (arr.shape[0], row // item), (arr.strides[0], item))
         if arr.ndim == 1:
             arr = arr.reshape(1, -1)
-        if arr.shape != (self.n_streams, row) or arr.strides[1] != 1:
-            raise ValueError(f"expected uint8 [{self.n_streams}, {row}], got {arr.shape}")
+        if arr.shape != (self.n_streams, row // item) or arr.strides[1] != item:
+            raise ValueError(f"expected {arr.dtype.name} [{self.n_streams}, {row // item}], got {arr.shape}")
         self._keepalive = (self._keepalive + [arr])[-2:]
         return int(arr.ctypes.data), 0, int(arr.strides[0])
 

@@ -1,10 +1,12 @@
 """Recorded-capture ingest for the batched engine (SURVEY.md section 8f rank 2, BASELINE configs[3]).
 
 The reference ingests only live (`sdr.read_samples_async`, radiotracking/analyze.py:143-157) and has no file reader;
-its wire format is what librtlsdr delivers and `rtl_sdr -f ... file.bin` records: interleaved uint8 I,Q bytes.  This
-module feeds such recordings -- one file per station channel -- to a `BatchAnalyzer`:
+its wire format is what librtlsdr delivers and `rtl_sdr -f ... file.bin` records: interleaved uint8 I,Q bytes ("cu8").
+Archives of other receivers hold ci8 (HackRF), ci16_le (Airspy, SDRplay, USRP sc16) or cf32_le (GNU Radio file sinks,
+`.cfile`); the reader takes the element type from `sample_format` or from a SigMF `.sigmf-meta` file beside the data
+(`core:datatype`).  This module feeds such recordings -- one file per station channel -- to a `BatchAnalyzer`:
 
-    CaptureReader     blocks `[n_streams, 2*block_samples]` uint8 (or groups of `blocks_per_read` consecutive blocks per
+    CaptureReader     blocks `[n_streams, 2*block_samples]` elements (or groups of `blocks_per_read` consecutive blocks per
                       stream) out of a ring of (pinned) host buffers, filled by a reader thread so that disk reads overlap
                       the GPU
     replay()          submit / collect with two launches in flight; an analyzer built with `blocks_per_launch = B` gets B
@@ -23,7 +25,11 @@ import queue
 import threading
 from typing import Callable, Iterator, List, Optional, Sequence
 
+import json
+
 import numpy as np
+
+from .engine import SAMPLE_FORMATS
 
 
 def _alloc(shape, pinned: bool) -> np.ndarray:
@@ -46,23 +52,53 @@ def _alloc(shape, pinned: bool) -> np.ndarray:
 _alloc.keep = []
 
 
+def sigmf_meta_path(path: str) -> str:
+    """The SigMF metadata file that belongs to a data file: `x.sigmf-data` -> `x.sigmf-meta`, any other name -> name + `.sigmf-meta`."""
+    stem = path[: -len(".sigmf-data")] if path.endswith(".sigmf-data") else path
+    return stem + ".sigmf-meta"
+
+
+def sigmf_sample_format(path: str) -> Optional[str]:
+    """`core:datatype` of the SigMF metadata beside the data file `path`, or None without one.  ValueError for a datatype the
+    engine does not read (big-endian, real-valued, or not in `engine.SAMPLE_FORMATS`)."""
+    meta = sigmf_meta_path(path)
+    if not os.path.exists(meta):
+        return None
+    with open(meta, "r", encoding="utf-8") as f:
+        dt = json.load(f).get("global", {}).get("core:datatype")
+    if dt not in SAMPLE_FORMATS:
+        raise ValueError(f"{meta}: core:datatype {dt!r} is not one of {', '.join(SAMPLE_FORMATS)}")
+    return dt
+
+
 class CaptureReader:
-    """Iterate over the blocks of `paths` (one raw uint8 IQ file per stream).
+    """Iterate over the blocks of `paths` (one raw IQ file per stream).
+
+    `sample_format`: the element type of the files (`engine.SAMPLE_FORMATS`); None takes it from the SigMF metadata beside the
+    files (all must agree) and reads cu8 without one.  An explicit format that a metadata file contradicts is a ValueError.
+    Items are arrays of that element type (views of byte buffers).
 
     Yields `(block_index, array)`; `array` is a view of one of `n_buffers` ring buffers and stays valid until
     `n_buffers - 1` further blocks have been taken (with the default 4: two blocks in flight in the engine plus the one
-    being filled).  With `blocks_per_read = B > 1` an item is a group of B consecutive blocks, `[n_streams, B * block_bytes]`
-    (`block_index` = index of its first block); a last, incomplete group is padded with the byte 0 (its blocks beyond
+    being filled).  With `blocks_per_read = B > 1` an item is a group of B consecutive blocks, `[n_streams, B * 2 * block_samples]`
+    (`block_index` = index of its first block); a last, incomplete group is padded with zero bytes (its blocks beyond
     `n_blocks` must be ignored by the consumer)."""
 
     def __init__(self, paths: Sequence[str], block_samples: int, n_buffers: int = 4, pinned: bool = True,
-                 max_blocks: Optional[int] = None, blocks_per_read: int = 1):
+                 max_blocks: Optional[int] = None, blocks_per_read: int = 1, sample_format: Optional[str] = None):
         if not paths:
             raise ValueError("no capture files")
         if n_buffers < 2:
             raise ValueError("need at least two ring buffers")
         self.paths = list(paths)
-        self.block_bytes = 2 * int(block_samples)
+        if sample_format is not None and sample_format not in SAMPLE_FORMATS:
+            raise ValueError(f"sample_format {sample_format!r} is not one of {', '.join(SAMPLE_FORMATS)}")
+        metas = {m for m in (sigmf_sample_format(p) for p in self.paths) if m is not None}
+        if len(metas) > 1 or (sample_format is not None and metas and metas != {sample_format}):
+            raise ValueError(f"SigMF metadata says {', '.join(sorted(metas))}, expected {sample_format or 'one format for every file'}")
+        self.sample_format = sample_format or (metas.pop() if metas else "cu8")
+        _, self.dtype, sample_bytes = SAMPLE_FORMATS[self.sample_format]
+        self.block_bytes = sample_bytes * int(block_samples)
         sizes = [os.path.getsize(p) for p in self.paths]
         self.n_blocks = min(sizes) // self.block_bytes              # tail dropped
         if max_blocks is not None:
@@ -121,7 +157,7 @@ class CaptureReader:
             held.append(i)
             if len(held) == len(self._bufs):                     # the oldest view is no longer needed by contract
                 self._free.put(held.pop(0))
-            yield b, self._bufs[i]
+            yield b, self._bufs[i].view(self.dtype)
         self._thread.join()
 
     def close(self):
@@ -131,7 +167,8 @@ class CaptureReader:
 
 def replay(paths: Sequence[str], analyzer, t0: datetime.datetime, on_block: Optional[Callable] = None,
            max_blocks: Optional[int] = None, pinned: bool = True) -> int:
-    """Run every full block of the recordings through `analyzer` (a `BatchAnalyzer` with one stream per file).
+    """Run every full block of the recordings through `analyzer` (a `BatchAnalyzer` with one stream per file), read in the
+    analyzer's `sample_format` (a SigMF metadata file beside a recording must agree with it).
 
     `on_block(block_index, per_stream)` receives what `BatchAnalyzer.collect` returns for that block
     (`per_stream[s] = (shadow-filtered Signals, candidates before the filter)`), in block order -- also when the
@@ -139,7 +176,8 @@ def replay(paths: Sequence[str], analyzer, t0: datetime.datetime, on_block: Opti
     if analyzer.n_streams != len(paths):
         raise ValueError("one capture file per analyzer stream")
     B = getattr(analyzer, "blocks_per_launch", 1)
-    reader = CaptureReader(paths, analyzer.block_samples, pinned=pinned, max_blocks=max_blocks, blocks_per_read=B)
+    reader = CaptureReader(paths, analyzer.block_samples, pinned=pinned, max_blocks=max_blocks, blocks_per_read=B,
+                           sample_format=getattr(analyzer, "sample_format", "cu8"))
     dt = datetime.timedelta(seconds=analyzer.block_samples / analyzer.sample_rate)
     pending: List[int] = []
     done = 0

@@ -81,6 +81,33 @@ def make_stream(w: Workload, stream: int = 0, n_blocks: Optional[int] = None, se
     Bursts are laid on the continuous timeline so some cross block boundaries
     (the reference re-finds those from the next block, analyze.py:383-398).
     """
+    iq = _signal_lsb(w, stream, n_blocks, seed)
+    iq += np.float32(127.5)
+    np.rint(iq, out=iq)
+    np.clip(iq, 0, 255, out=iq)
+    return iq.astype(np.uint8).reshape(iq.shape[0] // w.block_samples, 2 * w.block_samples)
+
+
+def make_stream_format(w: Workload, fmt: str, stream: int = 0, n_blocks: Optional[int] = None, seed: Optional[int] = None) -> np.ndarray:
+    """The signal of `make_stream` (noise and bursts in units of 1/127.5) quantised to the sample format `fmt` (a SigMF datatype):
+    `[n_blocks, 2*block_samples]` elements whose normalised samples (cu8 b / 127.5 - 1, ci8 v / 128, ci16_le v / 32768,
+    cf32_le x) approximate the same complex signal.  cu8 is `make_stream` itself."""
+    if fmt == "cu8":
+        return make_stream(w, stream, n_blocks, seed)
+    x = _signal_lsb(w, stream, n_blocks, seed).astype(np.float64) / 127.5
+    if fmt == "ci8":
+        q = np.clip(np.rint(x * 128.0), -128, 127).astype(np.int8)
+    elif fmt == "ci16_le":
+        q = np.clip(np.rint(x * 32768.0), -32768, 32767).astype("<i2")
+    elif fmt == "cf32_le":
+        q = x.astype("<f4")
+    else:
+        raise ValueError(f"unknown sample format {fmt!r}")
+    return q.reshape(q.shape[0] // w.block_samples, 2 * w.block_samples)
+
+
+def _signal_lsb(w: Workload, stream: int, n_blocks: Optional[int], seed: Optional[int]) -> np.ndarray:
+    """float32 `[n_blocks * block_samples, 2]`: receiver noise plus bursts in 8-bit LSB, before the offset and rounding."""
     nb = w.n_blocks if n_blocks is None else n_blocks
     N = w.block_samples
     M = nb * N
@@ -121,11 +148,7 @@ def make_stream(w: Workload, stream: int = 0, n_blocks: Optional[int] = None, se
         arg = 2 * np.pi * f * n + ph
         iq[s0:e0, 0] += (a * np.cos(arg)).astype(np.float32)
         iq[s0:e0, 1] += (a * np.sin(arg)).astype(np.float32)
-
-    iq += np.float32(127.5)
-    np.rint(iq, out=iq)
-    np.clip(iq, 0, 255, out=iq)
-    return iq.astype(np.uint8).reshape(nb, 2 * N)
+    return iq
 
 
 def make_batch(w: Workload, streams: Sequence[int], n_blocks: Optional[int] = None) -> np.ndarray:
