@@ -154,7 +154,8 @@ int rt_device_count(void);
 int rt_engine_create(const rt_config *cfg, rt_engine **out);
 void rt_engine_destroy(rt_engine *e);
 
-/* Launch on this CUDA stream (cudaStream_t) instead of the engine's own. */
+/* Launch on this CUDA stream (cudaStream_t) instead of the engine's own.  Work queued on it before a launch orders that
+ * launch; work on any other stream does not (rt_engine_wait_stream). */
 int rt_engine_set_stream(rt_engine *e, void *cuda_stream);
 
 /* Forget the carry of one stream (= a restarted analyzer: _spectrogram_last = None, analyze.py:128). */
@@ -192,6 +193,15 @@ int rt_engine_peek(rt_engine *e, int32_t *n_records);
  * event on it or reuses a device-resident `iq` buffer from another stream.  rt_engine_fetch does not need it.
  */
 int rt_engine_join(rt_engine *e);
+
+/*
+ * The other direction: the next launch is ordered after all work queued on `cuda_stream` (a cudaStream_t; also
+ * cudaStreamLegacy / cudaStreamPerThread) so far, e.g. the kernel or copy that produces a device-resident `iq`.  The
+ * engine's streams are non-blocking: without this (or the producer being the stream given to rt_engine_set_stream) a
+ * launch may read `iq` before it is written.  An event is recorded on `cuda_stream` and the launch stream waits for it;
+ * the engine-internal streams fork from the launch stream and inherit the wait.
+ */
+int rt_engine_wait_stream(rt_engine *e, void *cuda_stream);
 
 /* Counters of the last fetched launch: probe hits handed to the extraction kernel, and records emitted. */
 int rt_engine_last_counts(rt_engine *e, int32_t *work_items, int32_t *records);

@@ -337,7 +337,8 @@ class BatchAnalyzer:
     # -- one callback for every stream --------------------------------------------------------------
     def submit(self, iq) -> None:
         """Enqueue one block of every stream (H2D copy if `iq` is a host array, then the kernels); returns at once.
-        Up to two submissions may be in flight; results come back in order from `collect`."""
+        Up to two submissions may be in flight; results come back in order from `collect`.  A CUDA tensor is read after the work
+        queued so far on its device's current stream; `iq` is held until `collect` has returned this submission or a later one."""
         self.engine.launch(iq)
 
     def collect(self, ts_start: Sequence[datetime.datetime], with_all: bool = False):

@@ -724,6 +724,7 @@ struct rt_engine {
     // that launch i+1 fills the SMs while the last CTAs of launch i drain: step 227.7 -> 213.9 us at config 2
     cudaStream_t lstream[2] = {nullptr, nullptr};
     cudaEvent_t fork_ev = nullptr;
+    cudaEvent_t wait_ev = nullptr;           // rt_engine_wait_stream: the caller's stream, recorded (created on first use)
     int n_lstreams = 1;
     cudaEvent_t spec_done[RT_SLOTS] = {nullptr, nullptr};
     float* d_thr = nullptr;                  // [unit]
@@ -806,6 +807,7 @@ void free_engine(rt_engine* e) {
     if (e->scan_stream) cudaStreamDestroy(e->scan_stream);
     for (auto& ls : e->lstream) if (ls) cudaStreamDestroy(ls);
     if (e->fork_ev) cudaEventDestroy(e->fork_ev);
+    if (e->wait_ev) cudaEventDestroy(e->wait_ev);
     if (e->h_rec) cudaFreeHost(e->h_rec);
     if (e->h_counters) cudaFreeHost(e->h_counters);
     if (e->own_stream && e->stream) cudaStreamDestroy(e->stream);
@@ -1107,6 +1109,16 @@ int rt_engine_set_stream(rt_engine* e, void* cuda_stream) {
         e->own_stream = false;
     }
     e->stream = (cudaStream_t)cuda_stream;
+    return RT_OK;
+}
+
+int rt_engine_wait_stream(rt_engine* e, void* cuda_stream) {
+    if (!e) return fail(RT_ERR_INVALID, "null engine");
+    CU(cudaSetDevice(e->dev));
+    if (!e->wait_ev) CU(cudaEventCreateWithFlags(&e->wait_ev, cudaEventDisableTiming));
+    // the internal launch streams fork from e->stream at the next launch, so they inherit this wait
+    CU(cudaEventRecord(e->wait_ev, (cudaStream_t)cuda_stream));
+    CU(cudaStreamWaitEvent(e->stream, e->wait_ev, 0));
     return RT_OK;
 }
 

@@ -8,6 +8,7 @@ import ctypes
 import functools
 import logging
 import os
+import sys
 from typing import Optional, Sequence, Tuple, Union
 
 import numpy as np
@@ -19,6 +20,7 @@ RT_ABI_VERSION = 2
 FFT_AUTO, FFT_GENERIC, FFT_REG256, FFT_TC256 = 0, 1, 2, 3
 SCAN_AUTO, SCAN_SERIAL, SCAN_OVERLAP, SCAN_LEAN = 0, 1, 2, 3
 SAMPLE_CU8, SAMPLE_CI8, SAMPLE_CI16, SAMPLE_CF32 = 0, 1, 2, 3
+RT_SLOTS = 2        # results the engine holds: a third launch without a fetch drops the oldest (include/rt_engine.h)
 
 # rt_config.sample_format by SigMF datatype: (code, element dtype, bytes per complex sample).  The engine analyses the normalised
 # samples (cu8: b / 127.5 - 1 as pyrtlsdr delivers them, ci8: v / 128, ci16_le: v / 32768, cf32_le: x); include/rt_engine.h
@@ -47,7 +49,7 @@ EXPORTS = (
     "rt_last_error", "rt_abi_version", "rt_device_count", "rt_engine_create", "rt_engine_destroy",
     "rt_engine_set_stream", "rt_engine_reset_stream", "rt_engine_process", "rt_engine_launch", "rt_engine_fetch", "rt_engine_peek",
     "rt_engine_shape", "rt_engine_read_spectrogram", "rt_engine_read_row_means", "rt_engine_enable_timing",
-    "rt_engine_get_timing", "rt_engine_join", "rt_engine_last_counts", "rt_tc256_tables",
+    "rt_engine_get_timing", "rt_engine_join", "rt_engine_wait_stream", "rt_engine_last_counts", "rt_tc256_tables",
     # include/rt_matcher.h
     "rt_matcher_create", "rt_matcher_destroy", "rt_matcher_add", "rt_matcher_pending", "rt_matcher_drain",
     "rt_matcher_open", "rt_matcher_read_open",
@@ -114,6 +116,7 @@ def load_library() -> ctypes.CDLL:
     lib.rt_engine_fetch.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]
     lib.rt_engine_peek.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32)]
     lib.rt_engine_join.argtypes = [ctypes.c_void_p]
+    lib.rt_engine_wait_stream.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
     lib.rt_tc256_tables.argtypes = [ctypes.c_void_p, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
     lib.rt_engine_last_counts.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]
     lib.rt_engine_shape.argtypes = [ctypes.c_void_p] + [ctypes.POINTER(ctypes.c_int32)] * 3
@@ -144,6 +147,20 @@ def _cai_type(typestr: str) -> Tuple[str, int]:
     """(numpy name, itemsize) of a __cuda_array_interface__ typestr; the name is empty for a non-native byte order."""
     dt = np.dtype(typestr)
     return (dt.name if dt.isnative else ""), dt.itemsize
+
+
+def _producer_stream(obj) -> Optional[int]:
+    """The cudaStream_t handle whose queued work a reader of the device object `obj` must wait for: for a torch tensor the
+    current stream of its device (0: the legacy default stream), for a __cuda_array_interface__ object its `stream` entry
+    (None when absent or None: the producer has synchronised; 1 and 2 are the legacy and per-thread default streams)."""
+    if hasattr(obj, "data_ptr") and getattr(obj, "is_cuda", False):      # torch.Tensor: torch is loaded, the binding does not import it
+        return sys.modules["torch"].cuda.current_stream(obj.device).cuda_stream
+    s = obj.__cuda_array_interface__.get("stream")
+    if s is None:
+        return None
+    if int(s) == 0:         # the CUDA Array Interface (v3) forbids 0: it would not say which default stream is meant
+        raise ValueError("__cuda_array_interface__ stream 0 is ambiguous: use 1 (legacy default) or 2 (per-thread default)")
+    return int(s)
 
 
 def _device_pointer(obj, n_rows: int, row_bytes: int, dtypes: Tuple[str, ...] = ("uint8",)) -> Optional[Tuple[int, int]]:
@@ -222,13 +239,19 @@ class Engine:
         self.T = block_samples // nperseg
         self.cuda_device = cuda_device
         self.truncated = 0           # records the last fetch could not return (rt_config.max_records exceeded)
-        self._keepalive = []         # host buffers of launches not fetched yet (the H2D copy is asynchronous)
+        # The inputs (host or device) of the launches no fetch has returned yet, oldest first: the kernels of a launch may still
+        # read its input, also after a third launch dropped its result from the engine's ring.  A fetch has waited for its
+        # launch's kernels and for every earlier launch's (the scan kernels run in launch order), so it releases them.
+        self._held = []
+        self._launches = self._fetches = 0    # mirror of the engine's ring: launches made, results fetched or dropped
+        self._stream = None                   # the cudaStream_t handle last given to set_stream
 
     # -- lifetime ---------------------------------------------------------------------------
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
-            self._lib.rt_engine_destroy(self._h)
+            self._lib.rt_engine_destroy(self._h)          # waits for the engine's streams
             self._h = ctypes.c_void_p()
+        self._held = []
 
     def __del__(self):
         try:
@@ -243,14 +266,15 @@ class Engine:
         self.close()
 
     # -- data path ----------------------------------------------------------------------------
-    def _resolve(self, iq) -> Tuple[int, int, int]:
-        """(pointer, on device, row stride in bytes) of one launch's input: [n_streams, 2 * block_samples * blocks_per_launch]
-        elements of the engine's sample format (or [n_streams, blocks_per_launch, 2 * block_samples]); cf32 also as complex64 with
-        half as many elements per row."""
+    def _resolve(self, iq) -> Tuple[int, int, int, Optional[int], object]:
+        """(pointer, on device, row stride in bytes, producer stream, object that owns the memory) of one launch's input:
+        [n_streams, 2 * block_samples * blocks_per_launch] elements of the engine's sample format (or [n_streams,
+        blocks_per_launch, 2 * block_samples]); cf32 also as complex64 with half as many elements per row.  The producer stream
+        (`_producer_stream`) is None for host memory."""
         row = self.sample_bytes * self.block_samples * self.blocks_per_launch       # bytes: the consecutive blocks of one stream
         dev = _device_pointer(iq, self.n_streams, row, self._dtype_names)
         if dev is not None:
-            return dev[0], 1, dev[1]
+            return dev[0], 1, dev[1], _producer_stream(iq), iq
         arr = np.asarray(iq)
         if arr.dtype not in self._dtypes:
             raise TypeError(f"IQ blocks must be {' / '.join(self._dtype_names)} for sample format {self.sample_format}, got {arr.dtype}")
@@ -262,13 +286,20 @@ class Engine:
             arr = arr.reshape(1, -1)
         if arr.shape != (self.n_streams, row // item) or arr.strides[1] != item:
             raise ValueError(f"expected {arr.dtype.name} [{self.n_streams}, {row // item}], got {arr.shape}")
-        self._keepalive = (self._keepalive + [arr])[-2:]
-        return int(arr.ctypes.data), 0, int(arr.strides[0])
+        return int(arr.ctypes.data), 0, int(arr.strides[0]), None, arr
 
     def launch(self, iq) -> None:
-        """Enqueue one block (`blocks_per_launch` consecutive blocks) for every stream (asynchronous)."""
-        ptr, on_dev, stride = self._resolve(iq)
+        """Enqueue one block (`blocks_per_launch` consecutive blocks) for every stream (asynchronous).  A CUDA tensor is read
+        after the work queued so far on its device's current stream, a __cuda_array_interface__ object after its `stream`;
+        `iq` is held until a fetch has returned this launch or a later one."""
+        ptr, on_dev, stride, producer, owner = self._resolve(iq)
+        if producer is not None and producer != self._stream:
+            _check(self._lib.rt_engine_wait_stream(self._h, ctypes.c_void_p(producer)))
         _check(self._lib.rt_engine_launch(self._h, ctypes.c_void_p(ptr), on_dev, stride))
+        self._held.append(owner)
+        self._launches += 1
+        if self._launches - self._fetches > RT_SLOTS:
+            self._fetches += 1            # the engine dropped the oldest unfetched result; its input stays held
 
     def fetch(self) -> np.ndarray:
         """Wait for the oldest unfetched launch; candidate records sorted by (unit, fi, start).  If the launch produced more
@@ -280,6 +311,9 @@ class Engine:
         need = ctypes.c_int32(0)
         rc = self._lib.rt_engine_fetch(self._h, out.ctypes.data_as(ctypes.c_void_p), n.value, ctypes.byref(need))
         self.truncated = 0
+        if rc in (RT_OK, RT_ERR_OVERFLOW):              # the launch was consumed: release its input and every older one
+            self._fetches += 1
+            del self._held[:len(self._held) - (self._launches - self._fetches)]
         if rc == RT_ERR_OVERFLOW:
             self.truncated = need.value - n.value
             logger.error("rt_engine: %d candidate records exceed max_records, %d dropped", need.value, self.truncated)
@@ -295,7 +329,9 @@ class Engine:
         _check(self._lib.rt_engine_reset_stream(self._h, stream))
 
     def set_stream(self, cuda_stream: int) -> None:
+        """Launch on this cudaStream_t handle.  Inputs produced on it need no extra wait (`launch`)."""
         _check(self._lib.rt_engine_set_stream(self._h, ctypes.c_void_p(cuda_stream)))
+        self._stream = int(cuda_stream)
 
     def last_counts(self) -> tuple:
         """(probe hits handed to the extraction kernel, records emitted) of the last fetched launch."""

@@ -40,6 +40,117 @@ def test_no_cpu_fallback_without_device():
                  signal_threshold=1e-9, snr_threshold=3.0, probe_stride=9, min_cols=8, max_cols=49)
 
 
+class _StreamCai:
+    """A CuPy / Numba style device array (CUDA Array Interface v3) with an optional `stream` entry."""
+
+    def __init__(self, n=64, ptr=0x10000, **stream):
+        self.__cuda_array_interface__ = dict(shape=(1, n), typestr="|u1", data=(ptr, False), version=3, strides=None, **stream)
+
+
+class _RecordingLib:
+    """Stands in for librtb200.so: records the engine calls of the binding."""
+
+    def __init__(self):
+        self.calls = []
+
+    def rt_engine_create(self, cfg, h):
+        h._obj.value = 0x1000
+        return E.RT_OK
+
+    def rt_engine_destroy(self, h):
+        self.calls.append(("destroy",))
+
+    def rt_engine_set_stream(self, h, s):
+        self.calls.append(("set_stream", s.value or 0))
+        return E.RT_OK
+
+    def rt_engine_wait_stream(self, h, s):
+        self.calls.append(("wait", s.value or 0))
+        return E.RT_OK
+
+    def rt_engine_launch(self, h, iq, on_dev, stride):
+        self.calls.append(("launch", on_dev))
+        return E.RT_OK
+
+    def rt_engine_peek(self, h, n):
+        n._obj.value = 0
+        return E.RT_OK
+
+    def rt_engine_fetch(self, h, out, max_out, need):
+        need._obj.value = 0
+        return E.RT_OK
+
+
+def test_producer_stream_of_device_inputs(monkeypatch):
+    """_producer_stream: a CAI `stream` as given (absent / None: no wait; 1 legacy and 2 per-thread default streams and
+    pointers pass through; 0 is forbidden by the interface), and for a torch tensor the current stream of its device."""
+    assert E._producer_stream(_StreamCai()) is None
+    assert E._producer_stream(_StreamCai(stream=None)) is None
+    for s in (1, 2, 0x7F00DEADBEE0):
+        assert E._producer_stream(_StreamCai(stream=s)) == s
+    with pytest.raises(ValueError, match="stream 0"):
+        E._producer_stream(_StreamCai(stream=0))
+    assert E._device_pointer(_StreamCai(stream=7), 1, 64) == (0x10000, 64)     # the pointer and stride do not change
+    torch = pytest.importorskip("torch")
+    asked = []
+
+    class _Stream:
+        cuda_stream = 0x5150
+
+    def current_stream(device=None):
+        asked.append(device)
+        return _Stream()
+
+    class _Tensor:                           # what the binding reads of a CUDA torch.Tensor
+        is_cuda, dtype, shape, device = True, "torch.uint8", (1, 64), "cuda:3"
+
+        def data_ptr(self):
+            return 0x20000
+
+        def element_size(self):
+            return 1
+
+        def stride(self):
+            return (64, 1)
+
+    monkeypatch.setattr(torch.cuda, "current_stream", current_stream)
+    assert E._device_pointer(_Tensor(), 1, 64) == (0x20000, 64)
+    assert E._producer_stream(_Tensor()) == 0x5150
+    assert asked == ["cuda:3"]
+
+
+def test_launch_waits_for_the_producer_and_holds_inputs_until_fetched(monkeypatch):
+    """The binding's side of the stream contract, on a stand-in library: a launch waits for its input's producer stream unless
+    that is the stream given to set_stream, and every input stays referenced until a fetch returned its launch or a later one
+    (also after a third launch dropped the oldest result), and until close()."""
+    lib = _RecordingLib()
+    monkeypatch.setattr(E, "load_library", lambda: lib)
+    eng = E.Engine(n_streams=1, block_samples=32, nperseg=8, window=np.ones(8), sample_rate=3e5, signal_threshold=1e-9,
+                   snr_threshold=3.0, probe_stride=1, min_cols=1, max_cols=4)
+    xs = [_StreamCai(stream=7), _StreamCai(stream=1), _StreamCai(), _StreamCai(stream=2)]
+    for x in xs:
+        eng.launch(x)
+    assert [c for c in lib.calls if c[0] != "launch"] == [("wait", 7), ("wait", 1), ("wait", 2)]
+    assert [id(x) for x in eng._held] == [id(x) for x in xs]       # 4 launches, none fetched: the engine dropped 2 results
+    eng.fetch()                                                      # launch 2
+    assert [id(x) for x in eng._held] == [id(xs[3])]
+    eng.fetch()
+    assert eng._held == []
+    lib.calls.clear()
+    eng.set_stream(7)
+    eng.launch(xs[0])                                                # produced on the launch stream: no extra call
+    with pytest.raises(ValueError):
+        eng.launch(_StreamCai(stream=0))
+    host = np.zeros((1, 64), np.uint8)
+    eng.launch(host)
+    assert lib.calls == [("set_stream", 7), ("launch", 1), ("launch", 0)]
+    assert [id(x) for x in eng._held] == [id(xs[0]), id(host)]
+    eng.fetch()                                                      # launch 4: launch 5 is still in flight
+    assert len(eng._held) == 1
+    eng.close()
+    assert eng._held == [] and lib.calls[-1] == ("destroy",)
+
+
 @pytest.mark.parametrize("fs,n,N", [(300000, 256, 300000), (2400000, 256, 2400000), (256000, 256, 256000),
                                     (20000000, 1024, 20000000), (20000000, 4096, 2000000), (300000, 256, 250123)])
 def test_plan_matches_scipy_axes_and_reference_stride(fs, n, N):
