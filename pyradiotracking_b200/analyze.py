@@ -174,14 +174,15 @@ class BatchAnalyzer:
     """`n` independent analyzers (same sample rate / FFT / duration keys, own device name and
     calibration) evaluated together on one GPU."""
 
-    def __init__(self, devices: Sequence[str], calibration_db: Sequence[float], sample_rate: int, center_freq: int,
+    def __init__(self, devices: Sequence[str], calibration_db: Sequence[float], sample_rate: int, center_freq,
                  fft_nperseg: int, fft_window, signal_min_duration_ms: float, signal_max_duration_ms: float,
                  signal_threshold_dbw: float, snr_threshold_db: float, sdr_callback_length: Optional[int] = None,
                  cuda_device: int = 0, max_records: int = 0, fft_impl: int = _engine.FFT_AUTO,
                  scan_schedule: int = _engine.SCAN_AUTO, launch_streams: int = 0, chunk_segs: int = 0,
                  blocks_per_launch: int = 1, sample_format: str = "cu8"):
         """`sample_format`: the SigMF datatype of the input blocks, one of `engine.SAMPLE_FORMATS` (cu8: RTL-SDR bytes, ci8, ci16_le,
-        cf32_le); the thresholds apply to the normalised samples (INTEGRATION.md)."""
+        cf32_le); the thresholds apply to the normalised samples (INTEGRATION.md).  `center_freq`: one value for every device, or
+        one per device (the channels of a wideband recording, wideband.py); a Signal's frequency is `freqs[fi] + center_freq`."""
         if sample_format not in _engine.SAMPLE_FORMATS:
             raise ValueError(f"sample_format = {sample_format!r}: the B200 engine reads {', '.join(_engine.SAMPLE_FORMATS)} (see INTEGRATION.md)")
         self.sample_format = sample_format
@@ -197,6 +198,11 @@ class BatchAnalyzer:
             raise ValueError("blocks_per_launch must be >= 1")
         self.sample_rate = sample_rate
         self.center_freq = center_freq
+        self._center_freqs = None           # per device, or None: one scalar for all
+        if np.ndim(center_freq) != 0:
+            self._center_freqs = np.asarray(center_freq)
+            if self._center_freqs.shape != (self.n_streams,):
+                raise ValueError("center_freq: one value, or one per device")
         self.fft_nperseg = int(fft_nperseg)
         self.fft_window = fft_window
         self.blocks_per_launch = int(blocks_per_launch)
@@ -267,7 +273,7 @@ class BatchAnalyzer:
             fin = Finalized(
                 stream=stream, fi=r["fi"].astype(np.int64), start=r["start"].astype(np.int64), end=r["end"].astype(np.int64),
                 ts_off_us=timedelta_us(start_dt), dur_us=timedelta_us(duration_s),
-                frequency=plan.freqs[r["fi"]] + self.center_freq,
+                frequency=plan.freqs[r["fi"]] + (self.center_freq if self._center_freqs is None else self._center_freqs[stream // self.blocks_per_launch]),
                 max=10 * np.log10(r["max_lin"].astype(np.float64)) - cal, avg=10 * np.log10(mean) - cal,
                 std=r["std_db"].astype(np.float64), noise=10 * np.log10(row), snr=10 * np.log10(mean / row),
                 shadow=np.zeros(len(r), dtype=bool))
@@ -422,6 +428,11 @@ class SignalAnalyzer(multiprocessing.Process):
                 sys.exit(1)
         self.sample_rate = sample_rate
         self.center_freq = center_freq
+        self._center_freqs = None           # per device, or None: one scalar for all
+        if np.ndim(center_freq) != 0:
+            self._center_freqs = np.asarray(center_freq)
+            if self._center_freqs.shape != (self.n_streams,):
+                raise ValueError("center_freq: one value, or one per device")
         try:
             self.gain = float(gain)
         except ValueError:

@@ -13,18 +13,19 @@
 
 namespace rt {
 
-// host-side table: bytes per complex sample and the divisor that maps an element to the normalised sample
-// (cu8: b / 127.5 - 1, whose offset is removed by the detrend)
+// host-side table: bytes per complex sample, and the divisor and offset that map an element to the normalised sample
+// element / full_scale + offset (cu8: b / 127.5 - 1; the spectrogram kernels drop the offset, the detrend removes it)
 struct SampleFormatInfo {
     int bytes;
     double full_scale;
+    double offset;
 };
 inline bool sample_format_info(int fmt, SampleFormatInfo* out) {
     switch (fmt) {
-        case RT_SAMPLE_CU8: *out = {2, 127.5}; return true;
-        case RT_SAMPLE_CI8: *out = {2, 128.0}; return true;
-        case RT_SAMPLE_CI16: *out = {4, 32768.0}; return true;
-        case RT_SAMPLE_CF32: *out = {8, 1.0}; return true;
+        case RT_SAMPLE_CU8: *out = {2, 127.5, -1.0}; return true;
+        case RT_SAMPLE_CI8: *out = {2, 128.0, 0.0}; return true;
+        case RT_SAMPLE_CI16: *out = {4, 32768.0, 0.0}; return true;
+        case RT_SAMPLE_CF32: *out = {8, 1.0, 0.0}; return true;
         default: return false;
     }
 }
@@ -152,5 +153,25 @@ struct SegmentIn<RT_SAMPLE_CF32> {
         }
     }
 };
+
+// The normalised complex sample i of an interleaved I,Q row: fma(element, scale, offset) with scale = (float)(1 / full_scale) and
+// offset from sample_format_info (cf32: scale 1, offset 0, the value as stored).
+template <int FMT>
+__device__ __forceinline__ float2 load_normalised(const unsigned char* row, long long i, float scale, float offset) {
+    float re, im;
+    if (FMT == RT_SAMPLE_CU8) {
+        const uchar2 v = reinterpret_cast<const uchar2*>(row)[i];
+        re = v.x; im = v.y;
+    } else if (FMT == RT_SAMPLE_CI8) {
+        const char2 v = reinterpret_cast<const char2*>(row)[i];
+        re = v.x; im = v.y;
+    } else if (FMT == RT_SAMPLE_CI16) {
+        const short2 v = reinterpret_cast<const short2*>(row)[i];
+        re = v.x; im = v.y;
+    } else {
+        return reinterpret_cast<const float2*>(row)[i];
+    }
+    return make_float2(__fmaf_rn(re, scale, offset), __fmaf_rn(im, scale, offset));
+}
 
 }  // namespace rt
