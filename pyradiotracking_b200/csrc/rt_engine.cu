@@ -33,9 +33,6 @@
 #include "spectro256.cuh"
 #include "spectro_tc256.cuh"
 #include "spectro_r16.cuh"
-#ifdef RT_LAB
-#include "../../tools/spectro_s256_lab.cuh"      // 256-point-core kernel for nperseg 1024 / 4096: measured, not adopted (profiles/r02_s256_kernel.txt)
-#endif
 
 namespace {
 
@@ -71,58 +68,41 @@ __device__ __forceinline__ bool above(float p, float thr, float avg, float snr) 
 //                                  cells per 32-byte sector
 //   TILE   (tensor-core kernel)    S[stream][t / 32][quad][t % 32][4], quad = 4 k1 + (k2 >> 2) (rt::tile_cell_off): a thread owns a
 //                                  segment, a warp stores 512 contiguous bytes, 32 time steps of a bin lie within 512 bytes
-//   PERMR  (spectro_s256, n = 256 R) S[stream][t][256 k2 + pos(k1)] for bin = R k1 + k2, pos() as in PERM: half-warp k2 of a team stores the
-//                                  bins of its 256-point sub-transform, 256 contiguous bytes per store instruction
 // (time-blocked variants of PERM were measured and rejected: DESIGN.md 5.7)
-enum { LAYOUT_LINEAR = 0, LAYOUT_PERM = 1, LAYOUT_TILE = 2, LAYOUT_PERMR = 3 };
-// PERM time group (spectro256.cuh, TG): S[stream][t / TG][pos / 4][t % TG][pos % 4]
-#ifndef RT_PERM_TG
-#define RT_PERM_TG 2
-#endif
-constexpr int PERM_TG = RT_PERM_TG;
+enum { LAYOUT_LINEAR = 0, LAYOUT_PERM = 1, LAYOUT_TILE = 2 };
+// PERM time group (spectro256.cuh, TG): S[stream][t / TG][pos / 4][t % TG][pos % 4]; pairs of time steps (DESIGN.md 11.6)
+constexpr int PERM_TG = 2;
 // with time pairs the register kernel maps a segment's 16 threads onto the lanes {0-3, 8-11, ...} (spectro256.cuh, LMAP): every quarter-warp
 // phase of its 128-bit stores then covers one whole 128-byte line; back to back 173.9 -> 169.7 us (one time step per row: 170.8 us)
-constexpr bool PERM_LMAP = PERM_TG == 2;
-using R256Prod = rt::R256v7T<4, 4, PERM_LMAP>;
-// the nperseg-256 register kernel of the product: v8 (spectro256.cuh) under the time-pair layout; lab builds with other
-// time groupings (tools/build_lab_lib.sh, RT_PERM_TG = 1 | 4 | 8) keep v7n, which knows all of them
-#if RT_PERM_TG == 2
-#define RT_SPECTRO_REG256 rt::spectro_reg256_v8<true, 2>
-#define RT_SPECTRO_REG256_CI8 rt::spectro_reg256_v8<true, 2, true>
-#else
-#define RT_SPECTRO_REG256 rt::spectro_reg256_v7n<true, PERM_TG, PERM_LMAP>
-#endif
-__host__ __device__ constexpr int perm256(int k) { return ((k >> 6) << 6) | ((k & 15) << 2) | ((k >> 4) & 3); }                // bin -> position
+using R256Prod = rt::R256v7T<4, 4, true>;
+__host__ __device__ __forceinline__ constexpr int perm256(int k) { return ((k >> 6) << 6) | ((k & 15) << 2) | ((k >> 4) & 3); }                // bin -> position
 __host__ __device__ constexpr int unperm256(int p) { return ((p >> 2) & 15) + 16 * (4 * (p >> 6) + (p & 3)); }                 // position -> bin
-// row position -> FFT bin for the layouts whose rows are not in bin order (n = bins per row)
+// row position -> FFT bin for the layouts whose rows are not in bin order
 template <int L>
-__device__ __forceinline__ int pos_to_bin(int idx, int n) {
-    if (L == LAYOUT_PERM) return unperm256(idx);
-    if (L == LAYOUT_PERMR) return (n >> 8) * unperm256(idx & 255) + (idx >> 8);
-    return idx;
+__device__ __forceinline__ int pos_to_bin(int idx) {
+    return L == LAYOUT_PERM ? unperm256(idx) : idx;
 }
 
 struct CellRef {
     const float* base;     // stream base + the bin's constant part
-    int step;              // LINEAR / PERM: floats per time step
+    int step;              // LINEAR: floats per time step
     template <int L>
     __device__ __forceinline__ static CellRef make(const float* S, size_t stream_stride, int s, int fi, int n) {
         CellRef c;
         if (L == LAYOUT_TILE) { c.base = S + (size_t)s * stream_stride + (size_t)((fi & 15) * 4 + (fi >> 6)) * 128 + ((fi >> 4) & 3); c.step = 0; }
         else if (L == LAYOUT_PERM) {
-            const int pos = ((fi >> 6) << 6) | ((fi & 15) << 2) | ((fi >> 4) & 3);
+            const int pos = perm256(fi);
             c.base = S + (size_t)s * stream_stride + (pos >> 2) * (4 * PERM_TG) + (pos & 3);
             c.step = 256;
         }
-        else if (L == LAYOUT_PERMR) { const int R = n >> 8; c.base = S + (size_t)s * stream_stride + 256 * (fi & (R - 1)) + perm256(fi / R); c.step = n; }
         else { c.base = S + (size_t)s * stream_stride + fi; c.step = n; }
         return c;
     }
     template <int L>
     __device__ __forceinline__ const float* ptr(int t) const {
         return L == LAYOUT_TILE ? base + ((size_t)(t >> 5) * 8192 + (size_t)(t & 31) * 4)
-             : (L == LAYOUT_PERM && PERM_TG > 1) ? base + ((size_t)(t / PERM_TG) * (256 * PERM_TG) + (size_t)(t % PERM_TG) * 4)
-                                                 : base + (size_t)t * step;
+             : L == LAYOUT_PERM ? base + ((size_t)(t / PERM_TG) * (256 * PERM_TG) + (size_t)(t % PERM_TG) * 4)
+                                : base + (size_t)t * step;
     }
     template <int L>
     __device__ __forceinline__ float at(int t) const { return *ptr<L>(t); }
@@ -251,7 +231,7 @@ __global__ void __launch_bounds__(128, 16) row_mean_kernel(const float* part, fl
     const int fi = g >> 2, k = g & 3;
     const bool active = fi < n;
     // part_perm: the register kernel writes its chunk sums in PERM position order (n == 256)
-    const int src = part_perm ? (((fi >> 6) << 6) | ((fi & 15) << 2) | ((fi >> 4) & 3)) : fi;
+    const int src = part_perm ? perm256(fi) : fi;
     const float* p = part + (size_t)blockIdx.y * n_chunks * n + (active ? src : 0);
     double t = 0.0;
     for (int c0 = k; c0 < n_chunks; c0 += 32) {          // 8 of this thread's chunk sums per memory round trip
@@ -289,9 +269,6 @@ struct ScanArgs {
                            // the two floats save the extraction warp two dependent round trips in front of its first cells
     int max_work;          // capacity of the work list (worst case: every probe column of every bin)
     int widen;             // extraction: widen the forward walk after three round trips (small launches)
-#ifdef RT_LAB
-    int lab_mode;          // tools/ timing experiments (wrong results): bit 0 no statistics, bit 2 first block only
-#endif
     int* counters;         // [0] work items, [1] records
     rt_record* rec;
     int max_records;
@@ -325,9 +302,7 @@ __global__ void probe_kernel(ScanArgs a) {
     // PERM layout: the thread index is the position inside the S row (and inside the chunk-sum rows, which the register
     // kernel writes in the same order), so a warp reads 128 contiguous bytes per load instead of 2 floats out of each of
     // 8 sectors; position 64 a + 4 k1 + b holds bin k1 + 16 (4 a + b)
-    const int n_bins = a.n;
-    auto bin_of = [n_bins](int ix) { return pos_to_bin<TILE>(ix, n_bins); };
-    const int fi = bin_of(idx);
+    const int fi = pos_to_bin<TILE>(idx);
     const float thr = a.thr[s], snr = a.snr;
     if (tid == 0) s_n = 0;
     s_live[tid] = 0;
@@ -395,7 +370,7 @@ __global__ void probe_kernel(ScanArgs a) {
     for (int e = tid; e < n_list; e += blockDim.x) {
         const unsigned ent = s_list[e];
         const int o = (int)(ent >> 5), i = (int)(ent & 31u);
-        if (resolve(bin_of(bb * blockDim.x + o), s_avg[o], i)) atomicOr(&s_live[o], 1u << i);
+        if (resolve(pos_to_bin<TILE>(bb * blockDim.x + o), s_avg[o], i)) atomicOr(&s_live[o], 1u << i);
     }
     __syncthreads();
     live |= s_live[tid];
@@ -430,7 +405,7 @@ __global__ void __launch_bounds__(128, 16) probe_lean_kernel(ScanArgs a) {
         const int pb = tile % npb, g = (tile / npb) % ngr, s = tile / (npb * ngr);
         const int idx = pb * 32 + lane;
         if (idx >= a.n) continue;
-        const int fi = pos_to_bin<TILE>(idx, a.n);
+        const int fi = pos_to_bin<TILE>(idx);
         const CellRef col = CellRef::make<TILE>(a.S, a.stream_stride, s, fi, a.n);
         float c0[LEAN_PPT];
 #pragma unroll
@@ -461,9 +436,6 @@ __global__ void __launch_bounds__(128, 16) probe_lean_kernel(ScanArgs a) {
             bool keep = true;
             int lo = -1, hi = -1;
             bool lo_open = true, hi_open = true;
-#ifdef RT_LAB
-            if (a.lab_mode & 8) lo_open = hi_open = false;      // timing only: no neighbour loads (every hit survives)
-#endif
 #pragma unroll 1
             for (int d = 1; d <= PROBE_QUICK && (lo_open || hi_open); ++d) {
                 const int tl = ti - d, th = ti + d;
@@ -495,7 +467,7 @@ __device__ __forceinline__ float warp_max(float v) {
 }
 
 // extract2_kernel: one warp per work item (the round-1 extract_kernel at about half its memory sectors and round trips).  Measured
-// (tools/scan_skip.py, configs[1]): beside the spectrogram of the next launch the extraction alone costs the step 23 of its 30 us
+// (DESIGN.md 11.6, configs[1]): beside the spectrogram of the next launch the extraction alone costs the step 23 of its 30 us
 // of scan overhead, and that cost follows the number of scattered 32-byte sectors it reads (a first version with wide
 // speculative fetches -- 4 round trips per run instead of 11, the same ~340 sectors -- was 4 us SLOWER).
 //   * cells travel in ALIGNED blocks of 32 columns (lane = column & 31), the probe's own block first, then one block down
@@ -532,9 +504,6 @@ __global__ void __launch_bounds__(128, MINB) extract2_kernel(ScanArgs a) {
         float mx = 0.f;
         double sum = 0.0, sdb = 0.0, sdb2 = 0.0;
         auto acc = [&](float p) {
-#ifdef RT_LAB
-            if (a.lab_mode & 1) { mx = fmaxf(mx, p); return; }
-#endif
             mx = fmaxf(mx, p);
             sum += (double)p;
             // dB of one cell in float (MUFU.LG2: ~1e-6 dB absolute error, the record tolerance is 5e-4 dB); the sums stay float64
@@ -558,9 +527,6 @@ __global__ void __launch_bounds__(128, MINB) extract2_kernel(ScanArgs a) {
         bool bopen = nb < 0 && 32 * bh > lo_lim;
         bool fopen = end < 0 && 32 * kf < T;
         bool too_long = false;
-#ifdef RT_LAB
-        if (a.lab_mode & 4) { bopen = fopen = false; if (end < 0) end = ti + 1; if (nb < 0) nb = max(ti - 1, 0); }
-#endif
         // forward blocks per round trip: 1, 1, 1, then (WF = 4 and a.widen: small launches, where the chain of round trips IS the kernel
         // time and the sectors cost nothing) 2, 2, 4, 4, ... -- a 25-block pulse of a 20 MS/s stream takes 9 round trips instead of 25.
         // The lean instantiation (WF = 1) keeps one block per direction: beside the spectrogram every sector counts and 32 registers
@@ -659,7 +625,7 @@ __global__ void __launch_bounds__(128, MINB) extract2_kernel(ScanArgs a) {
     }
 }
 
-// PERM / TILE / PERMR -> [T][n] for the parity hook, with the power scale of the tensor-core path undone (a power of two: exact)
+// PERM / TILE -> [T][n] for the parity hook, with the power scale of the tensor-core path undone (a power of two: exact)
 template <int L>
 __global__ void untile_kernel(const float* S, float* out, int total, int n, float inv_scale) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -668,18 +634,18 @@ __global__ void untile_kernel(const float* S, float* out, int total, int n, floa
     out[idx] = CellRef::make<L>(S, 0, 0, fi, n).template at<L>(t) * inv_scale;
 }
 
-}  // namespace
-
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-#ifdef RT_LAB
-// tools/ only (tools/build_lab_lib.sh, never the shipped library): leave scan kernels out to time what each one costs the step
-extern "C" { int rt_lab_nowait = 0; int rt_lab_extract_mode = 0; int rt_lab_skip = 0; int rt_lab_lean_per_sm = 0; int rt_lab_extract_per_sm = 0; int rt_lab_s256 = 0; int rt_lab_probe_ppt = 0; }      // skip: bit 0 row means, bit 1 probe, bit 2 extraction; lean CTAs per SM (0 = default)
-#define RT_LAB_SKIP(b) (rt_lab_skip & (b))
-#else
-#define RT_LAB_SKIP(b) 0
-#endif
+// The spectrogram kernels of the engine (choose_kernels decides one per engine)
+enum class Spectro {
+    GENERIC,     // spectro_generic: every nperseg and sample format, LINEAR layout
+    REG256,      // nperseg 256, byte formats: register kernel spectro_reg256_v8 (spectro256.cuh), PERM layout
+    TC256,       // nperseg 256, byte formats, RT_FFT_TC256: tensor-core stage 1 (spectro_tc256.cuh), TILE layout
+    R16,         // nperseg 1024 / 4096, byte formats: radix-16 Stockham kernel (spectro_r16.cuh), LINEAR layout
+};
+
+}  // namespace
 
 // error text for the other translation units of the library (rt_matcher.cpp)
 int rt_internal_fail(int code, const char* msg) { return fail(code, msg); }
@@ -695,12 +661,14 @@ struct rt_engine {
     bool ci8 = false;                        // RT_SAMPLE_CI8: the byte kernels' int8 instantiations
     int max_work = 0;                        // capacity of d_work
     int max_records = 0;                     // effective capacity of one launch's record list
-    bool reg256 = false;                     // nperseg 256: register kernel (v7n) or tensor-core kernel
-    bool tc256 = false;                      // tensor-core stage 1 (spectro_tc256.cuh), TILE layout
-    bool r16 = false;                        // nperseg 1024 / 4096: radix-16 Stockham kernel (spectro_r16.cuh), LINEAR layout
-    bool s256 = false;                       // lab builds only: 256-point-core kernel (tools/spectro_s256_lab.cuh), PERMR layout
-    int last_layout = LAYOUT_LINEAR;         // S layout of the latest launch (rt_engine_read_spectrogram)
+    // ---- decided by choose_kernels
+    Spectro kind = Spectro::GENERIC;
+    int layout = LAYOUT_LINEAR;              // S layout
     size_t s_stride = 0;                     // floats per unit in a spectrogram buffer
+    int part_rows = 0;                       // partial row sums per unit (d_part)
+    bool part_perm = false;                  // the partial sums are in PERM position order (register kernel)
+    bool sep_mean = false;                   // the scan runs row_mean_kernel (else the probe kernel or the tensor-core kernel does)
+    int (*scan)(const rt_engine*, const ScanArgs&, cudaStream_t, cudaEvent_t) = nullptr;   // launch_scan<layout>, set by select_scan
     float pscale = 1.f;                      // power factor carried by S / row means / thresholds (tensor-core path), a power of two
     uint4* d_bmat = nullptr;                 // tensor-core operand image
     rt::TcTables tc_tab;
@@ -826,6 +794,187 @@ int peek_oldest(rt_engine* e) {
     return RT_OK;
 }
 
+// The engine's spectrogram kernel and everything that follows from it: the S layout, the chunking, the partial row sums, who takes
+// the row means, and the scan schedule that RT_SCAN_AUTO stands for (returned).  Called once, by rt_engine_create, on a validated
+// configuration; it reads n, T, bpl, n_units and block_bytes.
+int choose_kernels(rt_engine* e, const rt_config& cfg, bool byte_fmt, int sms) {
+    const int n = e->n, T = e->T;
+    // the register and tensor-core kernels read every unit's segments with 16-byte bulk copies: with blocks_per_launch > 1 the units
+    // of a stream lie block_bytes apart (RT_FFT_AUTO runs the generic kernel then, RT_FFT_REG256 was refused)
+    const bool units_aligned = e->bpl == 1 || e->block_bytes % 16 == 0;
+    if (cfg.fft_impl == RT_FFT_TC256) e->kind = Spectro::TC256;
+    else if (n == 256 && cfg.fft_impl != RT_FFT_GENERIC && byte_fmt && units_aligned) e->kind = Spectro::REG256;
+    else if ((n == 1024 || n == 4096) && cfg.fft_impl == RT_FFT_AUTO && byte_fmt) e->kind = Spectro::R16;
+    else e->kind = Spectro::GENERIC;
+
+    // chunking: it depends on T only, so a stream gives bit-identical row means whether it runs alone or inside a batch
+    e->chunk_segs = 32;
+    if (e->kind == Spectro::REG256 || e->kind == Spectro::TC256) {
+        // short blocks (300 kS/s SDRs, replay): shorter chunks = more CTAs per unit
+        e->chunk_segs = T >= 8192 ? 192 : (T >= 2048 ? 128 : 64);   // 192 at T = 9375 (49 chunks per stream): step 205.0 -> 202.8 us vs 128, 209.8 at 256
+        if (cfg.chunk_segs > 0) e->chunk_segs = cfg.chunk_segs;
+    }
+    e->n_chunks = (T + e->chunk_segs - 1) / e->chunk_segs;
+    if (e->kind == Spectro::R16) {
+        // segments are dealt round-robin over n_chunks CTAs (x teams) per unit: 148 SMs x the resident CTAs (3 at 1024, 2 at 4096)
+        const int teams = n == 4096 ? 1 : 4;
+        const int resident = 148 * (n == 4096 ? rt::R16Cfg<4096>::CTAS_PER_SM : rt::R16Cfg<1024>::CTAS_PER_SM);
+        e->n_chunks = std::min(resident, (T + teams - 1) / teams);
+        e->chunk_segs = (T + e->n_chunks - 1) / e->n_chunks;      // informational
+    }
+    e->part_rows = e->n_chunks;              // one partial row per CTA
+    e->part_perm = e->kind == Spectro::REG256;
+
+    switch (e->kind) {
+        case Spectro::TC256: {
+            e->layout = LAYOUT_TILE;
+            e->s_stride = (size_t)((T + 31) / 32) * 8192;
+            constexpr int NG = 2;
+            e->tc_bps = (T + rt::Tc256<NG>::BATCH - 1) / rt::Tc256<NG>::BATCH;
+            const long long Btot = (long long)e->n_units * e->tc_bps;
+            e->tc_grid = (int)std::max<long long>(1, std::min<long long>(sms, Btot / NG));
+            const long long G = (long long)e->tc_grid * NG;
+            for (int s = 0; s < e->n_units; ++s)
+                e->tc_slots = std::max(e->tc_slots, rt::tc_last_run(s, e->tc_bps, G, Btot) - rt::tc_first_run(s, e->tc_bps, G, Btot) + 1);
+            e->part_rows = e->tc_slots;      // one partial row per warp-group run
+            break;
+        }
+        case Spectro::REG256:
+            e->layout = LAYOUT_PERM;
+            e->s_stride = (size_t)((T + PERM_TG - 1) / PERM_TG) * PERM_TG * n;      // whole time groups
+            break;
+        default:
+            e->layout = LAYOUT_LINEAR;
+            e->s_stride = (size_t)T * n;
+    }
+
+    int sched = cfg.scan_schedule;
+    if (sched == RT_SCAN_AUTO)
+        // lean only where it was measured to win: the register kernel (the tensor-core kernel owns its SMs) with at least
+        // ~100 us of spectrogram per launch (short launches: the slower lean kernels become the critical path)
+        // (round-2 kernels, 2.4 MS/s streams: 32 streams 112.5 overlap / 113.9 lean, 48: 151.3 / 153.3, 64: 197.4 / 189.0 us;
+        //  lean probe + full-size extraction: 188.0, full-size probe + lean extraction: 196.5)
+        sched = (e->kind == Spectro::REG256 && (long long)e->n_units * T >= 500000) ? RT_SCAN_LEAN : RT_SCAN_OVERLAP;
+    e->scan_lean = sched == RT_SCAN_LEAN;
+    // the tensor-core kernel writes the row means itself; otherwise the probe kernel sums up to 48 partial rows (row_mean_of)
+    // and row_mean_kernel runs for more, and always under the lean schedule (the lean probe reads finished row means)
+    e->sep_mean = e->kind != Spectro::TC256 && (e->scan_lean || e->n_chunks > 48);
+    return sched;
+}
+
+size_t generic_smem(int n) { return (size_t)n * (2 * sizeof(float2) + sizeof(float)) + 16; }
+
+// The generic kernel's dynamic shared-memory limit.  The limit belongs to the kernel, not to this engine: only ever raise it, or an
+// engine created later with a smaller nperseg would make every launch of a larger one in the same process fail
+int raise_generic_smem(int sample_format, int n) {
+    static std::mutex attr_mu;                  // engines may be created from several threads
+    std::lock_guard<std::mutex> lock(attr_mu);
+    const SpectroKernel gk = generic_kernel(sample_format);
+    cudaFuncAttributes ga;
+    CU(cudaFuncGetAttributes(&ga, gk));
+    if (ga.maxDynamicSharedSizeBytes < (int)generic_smem(n))
+        CU(cudaFuncSetAttribute(gk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)generic_smem(n)));
+    return RT_OK;
+}
+
+// Kernel attributes of the engine's spectrogram kernel; CI8: the int8 instantiations of the byte kernels
+template <bool CI8>
+int set_spectro_attributes(const rt_engine* e) {
+    constexpr cudaFuncAttribute SMEM = cudaFuncAttributeMaxDynamicSharedMemorySize;
+    switch (e->kind) {
+        case Spectro::TC256:
+            CU((cudaFuncSetAttribute(rt::spectro_tc256_k<2, CI8>, SMEM, rt::Tc256<2>::SMEM)));
+            return RT_OK;
+        case Spectro::REG256:
+            CU((cudaFuncSetAttribute(rt::spectro_reg256_v8<true, 2, CI8>, SMEM, R256Prod::SMEM)));
+            CU((cudaFuncSetAttribute(rt::spectro_reg256_v8<true, 2, CI8>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
+            return RT_OK;
+        case Spectro::R16:
+            if (e->n == 4096) CU((cudaFuncSetAttribute(rt::spectro_r16_k<4096, CI8>, SMEM, rt::R16Cfg<4096>::SMEM)));
+            else CU((cudaFuncSetAttribute(rt::spectro_r16_k<1024, CI8>, SMEM, rt::R16Cfg<1024>::SMEM)));
+            return raise_generic_smem(e->cfg.sample_format, e->n);      // for unaligned input (launch_spectrogram)
+        case Spectro::GENERIC:
+            return raise_generic_smem(e->cfg.sample_format, e->n);
+    }
+    return RT_OK;
+}
+
+// The engine's spectrogram kernel for one launch; CI8 as above
+template <bool CI8>
+void launch_spectrogram(const rt_engine* e, const SpectroArgs& sa, int slot, bool aligned, cudaStream_t st) {
+    const dim3 grid(e->n_chunks, e->n_units);
+    switch (e->kind) {
+        case Spectro::TC256: {
+            rt::TcArgs ta;
+            ta.iq = sa.iq; ta.stream_stride = sa.stream_stride; ta.T = e->T; ta.n_streams = e->n_units;
+            ta.bps = e->tc_bps; ta.total_batches = e->n_units * e->tc_bps;
+            ta.bmat = e->d_bmat; ta.wc0 = e->tc_tab.wc0; ta.wc1 = e->tc_tab.wc1; ta.wc255 = e->tc_tab.wc255;
+            ta.S = sa.S; ta.S_stream_stride = e->s_stride;
+            ta.part = sa.part; ta.part_slots = e->tc_slots; ta.avg = e->d_avg[slot]; ta.ctr = e->d_ctr[slot];
+            ta.store = 1; ta.dbg = 0; ta.prof = nullptr;
+            rt::spectro_tc256_k<2, CI8><<<e->tc_grid, 512, rt::Tc256<2>::SMEM, st>>>(ta);
+            return;
+        }
+        case Spectro::REG256:
+            rt::spectro_reg256_v8<true, 2, CI8><<<grid, R256Prod::THREADS, R256Prod::SMEM, st>>>(sa);
+            return;
+        case Spectro::R16:
+            // the one choice made per launch: the radix-16 kernel reads 16-byte aligned input only.  Given anything else, the
+            // generic kernel runs with the same chunking (one partial row per CTA) and writes the same LINEAR layout
+            if (!aligned) break;
+            if (e->n == 4096) rt::spectro_r16_k<4096, CI8><<<grid, 256, rt::R16Cfg<4096>::SMEM, st>>>(sa);
+            else rt::spectro_r16_k<1024, CI8><<<grid, 256, rt::R16Cfg<1024>::SMEM, st>>>(sa);
+            return;
+        case Spectro::GENERIC:
+            break;
+    }
+    generic_kernel(e->cfg.sample_format)<<<grid, 256, generic_smem(e->n), st>>>(sa);
+}
+
+// The probe and extraction kernels of one launch for S layout L (rt_engine::scan); probe_done is recorded between them (timing)
+template <int L>
+int launch_scan(const rt_engine* e, const ScanArgs& sc, cudaStream_t st, cudaEvent_t probe_done) {
+    if (e->scan_lean) {
+        probe_lean_kernel<L><<<e->lean_ctas, 128, 0, st>>>(sc);
+    } else {
+        const int pbins = std::min(e->n, 256), ppt = e->probe_ppt;
+        const dim3 pgrid(((e->n + pbins - 1) / pbins) * ((e->n_probes + ppt - 1) / ppt), e->n_units);
+        if (ppt == 8) probe_kernel<L, 8><<<pgrid, pbins, 0, st>>>(sc);
+        else if (ppt == 16) probe_kernel<L, 16><<<pgrid, pbins, 0, st>>>(sc);
+        else probe_kernel<L, 32><<<pgrid, pbins, 0, st>>>(sc);
+    }
+    CU(cudaGetLastError());
+    if (probe_done) CU(cudaEventRecord(probe_done, st));
+    // full size: one wave of 128-thread CTAs, four 32-cell windows per round trip; lean: one 32-cell window, no speculative
+    // forward fetch (fewest sectors: the kernel runs beside the spectrogram of the next launch)
+    if (e->scan_lean) extract2_kernel<L, 16><<<e->lean_ctas, 128, 0, st>>>(sc);
+    else if (sc.widen) extract2_kernel<L, 8, 4><<<148 * 24, 128, 0, st>>>(sc);
+    else extract2_kernel<L, 8><<<148 * 24, 128, 0, st>>>(sc);
+    CU(cudaGetLastError());
+    return RT_OK;
+}
+
+// The scan kernels of the engine's layout: rt_engine::scan, and the lean schedule's carve-out (the same as the resident spectrogram
+// CTAs': an SM does not change its L1 / shared split while CTAs are resident, so a kernel asking for another split could not join them)
+template <int L>
+int use_scan_layout(rt_engine* e) {
+    e->scan = launch_scan<L>;
+    if (e->scan_lean) {
+        CU(cudaFuncSetAttribute(row_mean_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        CU(cudaFuncSetAttribute(probe_lean_kernel<L>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        CU((cudaFuncSetAttribute(extract2_kernel<L, 16>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
+    }
+    return RT_OK;
+}
+
+int select_scan(rt_engine* e) {
+    switch (e->layout) {
+        case LAYOUT_PERM: return use_scan_layout<LAYOUT_PERM>(e);
+        case LAYOUT_TILE: return use_scan_layout<LAYOUT_TILE>(e);
+        default: return use_scan_layout<LAYOUT_LINEAR>(e);
+    }
+}
+
 }  // namespace
 
 extern "C" {
@@ -860,20 +1009,16 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     if (cfg->scan_schedule < RT_SCAN_AUTO || cfg->scan_schedule > RT_SCAN_LEAN) return fail(RT_ERR_INVALID, "unknown scan_schedule");
     if (cfg->launch_streams < 0 || cfg->launch_streams > 2) return fail(RT_ERR_INVALID, "launch_streams must be 0 (auto), 1 or 2");
     if (cfg->launch_streams == 2 && cfg->scan_schedule == RT_SCAN_SERIAL) return fail(RT_ERR_INVALID, "two launch streams need an overlapped scan schedule");
-    if (cfg->chunk_segs < 0 || cfg->chunk_segs % (PERM_TG > 2 ? 4 * PERM_TG : 8) != 0) return fail(RT_ERR_INVALID, "chunk_segs must be 0 (auto) or a multiple of 8");
+    if (cfg->chunk_segs < 0 || cfg->chunk_segs % 8 != 0) return fail(RT_ERR_INVALID, "chunk_segs must be 0 (auto) or a multiple of 8");
     if (cfg->fft_impl == RT_FFT_TC256 && bpl != 1) return fail(RT_ERR_INVALID, "RT_FFT_TC256 does not take blocks_per_launch > 1");
     rt::SampleFormatInfo fmt;
     if (!rt::sample_format_info(cfg->sample_format, &fmt)) return fail(RT_ERR_INVALID, "unknown sample_format");
     const bool byte_fmt = rt::sample_format_is_byte(cfg->sample_format);
     if (!byte_fmt && (cfg->fft_impl == RT_FFT_REG256 || cfg->fft_impl == RT_FFT_TC256))
         return fail(RT_ERR_INVALID, "RT_FFT_REG256 / RT_FFT_TC256 read bytes: RT_SAMPLE_CI16 / RT_SAMPLE_CF32 run on RT_FFT_GENERIC");
-#if RT_PERM_TG != 2
-    if (cfg->sample_format == RT_SAMPLE_CI8 && n == 256 && cfg->fft_impl != RT_FFT_GENERIC) return fail(RT_ERR_INVALID, "lab builds: ci8 at nperseg 256 needs RT_FFT_GENERIC");
-#endif
     // the register kernel reads every unit's segments with 16-byte bulk copies: with blocks_per_launch > 1 the units of a stream
-    // lie block_bytes apart, so the block must be a multiple of 16 bytes.  The PERM layout is fixed here, so this is decided here.
-    const bool reg256_unaligned = n == 256 && bpl > 1 && (fmt.bytes * cfg->block_samples) % 16 != 0;
-    if (cfg->fft_impl == RT_FFT_REG256 && reg256_unaligned)
+    // lie block_bytes apart, so the block must be a multiple of 16 bytes (choose_kernels)
+    if (cfg->fft_impl == RT_FFT_REG256 && bpl > 1 && (fmt.bytes * cfg->block_samples) % 16 != 0)
         return fail(RT_ERR_INVALID, "RT_FFT_REG256 with blocks_per_launch > 1 needs block_samples to be a multiple of 8");
     for (int r : cfg->reserved) if (r != 0) return fail(RT_ERR_INVALID, "rt_config.reserved must be zero");
 
@@ -898,19 +1043,9 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     e->ci8 = cfg->sample_format == RT_SAMPLE_CI8;
     e->block_bytes = (size_t)fmt.bytes * (size_t)cfg->block_samples;
     e->n_probes = (e->T + cfg->probe_stride - 1) / cfg->probe_stride;
-    e->reg256 = (n == 256) && (cfg->fft_impl != RT_FFT_GENERIC) && !reg256_unaligned && byte_fmt;     // RT_FFT_AUTO: generic kernel then
-    e->tc256 = cfg->fft_impl == RT_FFT_TC256;
-    e->r16 = (n == 1024 || n == 4096) && cfg->fft_impl == RT_FFT_AUTO && byte_fmt;
-#ifdef RT_LAB
-    if (e->r16 && rt_lab_s256) { e->r16 = false; e->s256 = true; }
-#endif
-    e->chunk_segs = 32;
-    if (e->reg256) {
-        // short blocks (300 kS/s SDRs, replay): shorter chunks = more CTAs per unit.  The choice depends on T only, so a
-        // stream gives bit-identical row means whether it runs alone or inside a batch.
-        e->chunk_segs = e->T >= 8192 ? 192 : (e->T >= 2048 ? 128 : 64);   // 192 at T = 9375 (49 chunks per stream): step 205.0 -> 202.8 us vs 128, 209.8 at 256
-        if (cfg->chunk_segs > 0) e->chunk_segs = cfg->chunk_segs;
-    }
+    int sms = 0;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->dev) != cudaSuccess || sms < 1) sms = 148;
+    const int sched = choose_kernels(e, *cfg, byte_fmt, sms);
     {
         // full-size probe kernel: as many CTAs as fit in ONE wave beside the resident spectrogram CTAs of the next launch (about one
         // 256-thread CTA per SM).  Fewer probe columns per thread = more CTAs and shorter chains of round trips, but a second wave
@@ -922,18 +1057,6 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
             if (bin_blocks * ((e->n_probes + ppt - 1) / ppt) * e->n_units <= 148) break;
         }
     }
-    e->n_chunks = (e->T + e->chunk_segs - 1) / e->chunk_segs;
-    if (e->r16 || e->s256) {
-        // segments are dealt round-robin over n_chunks CTAs (x teams) per unit: 148 SMs x the resident CTAs (r16: 3 at 1024, 2 at 4096)
-        const int teams = n == 4096 ? 1 : 4;
-        const int resident = 148 * (e->s256 ? 2 : n == 4096 ? rt::R16Cfg<4096>::CTAS_PER_SM : rt::R16Cfg<1024>::CTAS_PER_SM);
-        // (depends on T only, like chunk_segs above: the same row means alone and inside a batch)
-        e->n_chunks = std::min(resident, (e->T + teams - 1) / teams);
-        e->chunk_segs = (e->T + e->n_chunks - 1) / e->n_chunks;      // informational
-    }
-    e->s_stride = e->tc256 ? (size_t)((e->T + 31) / 32) * 8192
-                : e->reg256 ? (size_t)((e->T + PERM_TG - 1) / PERM_TG) * PERM_TG * n      // PERM: whole time groups
-                            : (size_t)e->T * n;
     const size_t max_work = (size_t)e->n_units * n * e->n_probes;    // every probe cell a hit: the work list cannot overflow
     // every record belongs to a different probe hit, so max_work records is the worst case; capped at 4 Mi (160 MB per slot)
     e->max_records = cfg->max_records > 0 ? cfg->max_records : (int)std::min<size_t>(max_work, (size_t)4 << 20);
@@ -958,19 +1081,10 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     const double amp = std::sqrt(1.0 / (cfg->sample_rate * sw2)) / fmt.full_scale;
     std::vector<float> hwin(n);
     for (int i = 0; i < n; ++i) hwin[i] = (float)(cfg->window[i] * amp);
-    int sms = 0;
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->dev) != cudaSuccess || sms < 1) sms = 148;
-    if (e->tc256) {
+    if (e->kind == Spectro::TC256) {
         e->tc_tab = rt::tc_make_tables(cfg->window, amp);
         if (!e->tc_tab.eligible) { free_engine(e); return fail(RT_ERR_INVALID, "RT_FFT_TC256 needs a window whose DFT is confined to the bins 0 and +-1 (boxcar, hann, hamming)"); }
         e->pscale = e->tc_tab.pscale;
-        constexpr int NG = 2;
-        e->tc_bps = (e->T + rt::Tc256<NG>::BATCH - 1) / rt::Tc256<NG>::BATCH;
-        const long long Btot = (long long)e->n_units * e->tc_bps;
-        e->tc_grid = (int)std::max<long long>(1, std::min<long long>(sms, Btot / NG));
-        const long long G = (long long)e->tc_grid * NG;
-        for (int s = 0; s < e->n_units; ++s)
-            e->tc_slots = std::max(e->tc_slots, rt::tc_last_run(s, e->tc_bps, G, Btot) - rt::tc_first_run(s, e->tc_bps, G, Btot) + 1);
     }
     std::vector<float2> htw(n);
     for (int k = 0; k < n; ++k) {
@@ -981,13 +1095,13 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     for (int u = 0; u < e->n_units; ++u) hthr[u] = (float)cfg->signal_threshold[u / bpl] * e->pscale;   // pscale is a power of two: exact
 
     const size_t cells = (size_t)e->n_units * e->s_stride;
-    const size_t part_rows = e->tc256 ? (size_t)e->tc_slots : (size_t)e->n_chunks;
+    const size_t part_cells = (size_t)e->n_units * e->part_rows * n;
     CUE(cudaMalloc(&e->d_win, n * sizeof(float)));
     CUE(cudaMalloc(&e->d_tw, n * sizeof(float2)));
     for (int k = 0; k < RT_SBUFS; ++k) CUE(cudaMalloc(&e->d_S[k], cells * sizeof(float)));
     for (int k = 0; k < RT_SLOTS; ++k) {
-        CUE(cudaMalloc(&e->d_part[k], (size_t)e->n_units * part_rows * n * sizeof(float)));
-        CUE(cudaMemset(e->d_part[k], 0, (size_t)e->n_units * part_rows * n * sizeof(float)));
+        CUE(cudaMalloc(&e->d_part[k], part_cells * sizeof(float)));
+        CUE(cudaMemset(e->d_part[k], 0, part_cells * sizeof(float)));
         CUE(cudaMalloc(&e->d_avg[k], (size_t)e->n_units * n * sizeof(float)));
         CUE(cudaMalloc(&e->d_ctr[k], e->n_units * sizeof(unsigned)));
         CUE(cudaMemset(e->d_ctr[k], 0, e->n_units * sizeof(unsigned)));
@@ -995,11 +1109,9 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
         CUE(cudaEventCreateWithFlags(&e->done[k], cudaEventDisableTiming));
         CUE(cudaEventCreateWithFlags(&e->spec_done[k], cudaEventDisableTiming));
     }
-    if (e->tc256) {
+    if (e->kind == Spectro::TC256) {
         CUE(cudaMalloc(&e->d_bmat, e->tc_tab.bmat.size() * sizeof(uint16_t)));
         CUE(cudaMemcpy(e->d_bmat, e->tc_tab.bmat.data(), e->tc_tab.bmat.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
-        if (e->ci8) CUE((cudaFuncSetAttribute(rt::spectro_tc256_k<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::Tc256<2>::SMEM)));
-        else CUE(cudaFuncSetAttribute(rt::spectro_tc256_k<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::Tc256<2>::SMEM));
     }
     CUE(cudaMalloc(&e->d_thr, e->n_units * sizeof(float)));
     CUE(cudaMalloc(&e->d_hasprev, e->n_units * sizeof(int)));
@@ -1008,14 +1120,7 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     CUE(cudaMalloc(&e->d_counters, 2 * RT_SLOTS * sizeof(int)));
     CUE(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
 
-    // ---- schedule (rt_config.scan_schedule / launch_streams; DESIGN.md 5.7)
-    int sched = cfg->scan_schedule;
-    if (sched == RT_SCAN_AUTO)
-        // lean only where it was measured to win: the register kernel (the tensor-core kernel owns its SMs) with at least
-        // ~100 us of spectrogram per launch (short launches: the slower lean kernels become the critical path)
-        // (round-2 kernels, 2.4 MS/s streams: 32 streams 112.5 overlap / 113.9 lean, 48: 151.3 / 153.3, 64: 197.4 / 189.0 us;
-        //  lean probe + full-size extraction: 188.0, full-size probe + lean extraction: 196.5)
-        sched = (e->reg256 && !e->tc256 && (long long)e->n_units * e->T >= 500000) ? RT_SCAN_LEAN : RT_SCAN_OVERLAP;
+    // ---- schedule (rt_config.scan_schedule / launch_streams, resolved by choose_kernels; DESIGN.md 5.7)
     if (sched != RT_SCAN_SERIAL) {
         // the scan kernels are small and latency bound: give them priority over the next launch's spectrogram CTAs
         int prio_lo = 0, prio_hi = 0;
@@ -1027,25 +1132,9 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
             e->n_lstreams = 2;
         }
     }
-    e->scan_lean = sched == RT_SCAN_LEAN;
     // lean scan kernels: 128-thread CTAs capped at 32 registers (4096 per CTA -- what four resident spectrogram CTAs leave free
     // on an SM), 12 per SM (8 ... 16 time the same within 1 %)
     e->lean_ctas = sms * 12;
-    if (e->scan_lean) {
-        // same shared-memory carve-out as the resident spectrogram CTAs: an SM does not change its L1 / shared split
-        // while CTAs are resident, so a kernel asking for another split could not join them
-        CUE(cudaFuncSetAttribute(row_mean_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        CUE(cudaFuncSetAttribute(probe_lean_kernel<LAYOUT_PERM>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        CUE(cudaFuncSetAttribute(probe_lean_kernel<LAYOUT_LINEAR>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        CUE(cudaFuncSetAttribute(probe_lean_kernel<LAYOUT_TILE>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-#ifdef RT_LAB
-        CUE(cudaFuncSetAttribute(probe_lean_kernel<LAYOUT_PERMR>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        CUE((cudaFuncSetAttribute(extract2_kernel<LAYOUT_PERMR, 16>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
-#endif
-        CUE(cudaFuncSetAttribute(extract2_kernel<LAYOUT_PERM, 16>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        CUE(cudaFuncSetAttribute(extract2_kernel<LAYOUT_LINEAR, 16>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        CUE(cudaFuncSetAttribute(extract2_kernel<LAYOUT_TILE, 16>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    }
     CUE(cudaMallocHost(&e->h_counters, 2 * sizeof(int)));
     CUE(cudaMemcpy(e->d_win, hwin.data(), n * sizeof(float), cudaMemcpyHostToDevice));
     CUE(cudaMemcpy(e->d_tw, htw.data(), n * sizeof(float2), cudaMemcpyHostToDevice));
@@ -1053,45 +1142,18 @@ int rt_engine_create(const rt_config* cfg, rt_engine** out) {
     e->h_hasprev.assign(e->n_streams, 0);
     e->h_hasprev_units.assign(e->n_units, 0);
     e->hasprev_dirty = true;
-    if (e->r16) {
+    if (e->kind == Spectro::R16) {
         const int bt = n / 16;
         std::vector<float2> htw1((size_t)15 * bt);
         for (int i = 1; i < 16; ++i)
             for (int b = 0; b < bt; ++b) htw1[(size_t)(i - 1) * bt + b] = htw[(b * i) & (n - 1)];
         CUE(cudaMalloc(&e->d_tw1, htw1.size() * sizeof(float2)));
         CUE(cudaMemcpy(e->d_tw1, htw1.data(), htw1.size() * sizeof(float2), cudaMemcpyHostToDevice));
-        if (n == 4096) CUE(cudaFuncSetAttribute(rt::spectro_r16_k<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<4096>::SMEM));
-        else CUE(cudaFuncSetAttribute(rt::spectro_r16_k<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<1024>::SMEM));
-        if (e->ci8 && n == 4096) CUE((cudaFuncSetAttribute(rt::spectro_r16_k<4096, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<4096>::SMEM)));
-        if (e->ci8 && n == 1024) CUE((cudaFuncSetAttribute(rt::spectro_r16_k<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::R16Cfg<1024>::SMEM)));
-    }
-#ifdef RT_LAB
-    if (e->s256) {
-        if (n == 4096) CUE(cudaFuncSetAttribute(rt::spectro_s256_k<4096>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::S256Cfg<4096>::SMEM));
-        else CUE(cudaFuncSetAttribute(rt::spectro_s256_k<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, rt::S256Cfg<1024>::SMEM));
-    }
-#endif
-    if (!e->reg256) {
-        // the limit belongs to the kernel, not to this engine: only ever raise it, or an engine created later with a smaller
-        // nperseg would make every launch of a larger one in the same process fail
-        const int smem = (int)((size_t)n * (2 * sizeof(float2) + sizeof(float)) + 16);
-        static std::mutex attr_mu;                  // engines may be created from several threads
-        std::lock_guard<std::mutex> lock(attr_mu);
-        const SpectroKernel gk = generic_kernel(cfg->sample_format);
-        cudaFuncAttributes ga;
-        CUE(cudaFuncGetAttributes(&ga, gk));
-        if (ga.maxDynamicSharedSizeBytes < smem)
-            CUE(cudaFuncSetAttribute(gk, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    } else if (e->ci8) {
-#ifdef RT_SPECTRO_REG256_CI8
-        CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256_CI8, cudaFuncAttributeMaxDynamicSharedMemorySize, R256Prod::SMEM)));
-        CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256_CI8, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
-#endif
-    } else {
-        CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256, cudaFuncAttributeMaxDynamicSharedMemorySize, R256Prod::SMEM)));
-        CUE((cudaFuncSetAttribute(RT_SPECTRO_REG256, cudaFuncAttributePreferredSharedMemoryCarveout, 100)));
     }
 #undef CUE
+    int rc = e->ci8 ? set_spectro_attributes<true>(e) : set_spectro_attributes<false>(e);
+    if (rc == RT_OK) rc = select_scan(e);
+    if (rc != RT_OK) { free_engine(e); return rc; }
     *out = e;
     return RT_OK;
 }
@@ -1177,7 +1239,7 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
     if (((uintptr_t)d_iq | (e->n_streams > 1 ? stride : 0)) % (uintptr_t)e->sample_bytes != 0)
         return fail(RT_ERR_INVALID, "IQ pointer / stream stride not aligned to one complex sample");
     const bool aligned = (((uintptr_t)d_iq | stride | (e->bpl > 1 ? e->block_bytes : 0)) & 15) == 0;
-    if (e->reg256 && !aligned) return fail(RT_ERR_INVALID, "register FFT path needs 16-byte aligned IQ, stream stride and (blocks_per_launch > 1) block size");
+    if ((e->kind == Spectro::REG256 || e->kind == Spectro::TC256) && !aligned) return fail(RT_ERR_INVALID, "register FFT path needs 16-byte aligned IQ, stream stride and (blocks_per_launch > 1) block size");
     const int slot = (int)(e->launch_seq % RT_SLOTS);
     if (e->launch_seq - e->fetch_seq == RT_SLOTS) { e->fetch_seq++; e->peeked = false; }   // ring full: the oldest unfetched result is dropped
     int* d_cnt = e->d_counters + 2 * slot;
@@ -1185,10 +1247,6 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
     // Two streams: the spectrogram of this launch runs on the launch stream while the scan kernels of the
     // previous launch are still busy on the scan stream.  The buffers this launch writes (S[next], part[slot])
     // were last read by the scan of launch i-2, whose completion event is done[slot].
-#ifdef RT_LAB
-    if (rt_lab_nowait) {}      // timing only (racy): is the scan chain of launch i - 2 the critical path of launch i?
-    else
-#endif
     if (e->launch_seq >= RT_SLOTS && e->scan_stream) CU(cudaStreamWaitEvent(st, e->done[slot], 0));
 
     rt_engine::EvSet* evs = nullptr;
@@ -1214,41 +1272,8 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
     sa.chunk_segs = e->chunk_segs; sa.n_chunks = e->n_chunks;
     sa.win = e->d_win; sa.tw = e->d_tw; sa.tw1 = e->d_tw1; sa.S = e->d_S[next]; sa.part = e->d_part[slot];
     sa.S_stream_stride = e->s_stride;
-    const bool use_reg = e->reg256;
-    dim3 grid(e->n_chunks, e->n_units);
-    if (use_reg && e->tc256) {
-        rt::TcArgs ta;
-        ta.iq = d_iq; ta.stream_stride = stride; ta.T = e->T; ta.n_streams = e->n_units;
-        ta.bps = e->tc_bps; ta.total_batches = e->n_units * e->tc_bps;
-        ta.bmat = e->d_bmat; ta.wc0 = e->tc_tab.wc0; ta.wc1 = e->tc_tab.wc1; ta.wc255 = e->tc_tab.wc255;
-        ta.S = e->d_S[next]; ta.S_stream_stride = e->s_stride;
-        ta.part = e->d_part[slot]; ta.part_slots = e->tc_slots; ta.avg = e->d_avg[slot]; ta.ctr = e->d_ctr[slot];
-        ta.store = 1; ta.dbg = 0; ta.prof = nullptr;
-        if (e->ci8) rt::spectro_tc256_k<2, true><<<e->tc_grid, 512, rt::Tc256<2>::SMEM, st>>>(ta);
-        else rt::spectro_tc256_k<2><<<e->tc_grid, 512, rt::Tc256<2>::SMEM, st>>>(ta);
-    } else if (use_reg) {
-#ifdef RT_SPECTRO_REG256_CI8
-        if (e->ci8) RT_SPECTRO_REG256_CI8<<<grid, R256Prod::THREADS, R256Prod::SMEM, st>>>(sa);
-        else
-#endif
-        RT_SPECTRO_REG256<<<grid, R256Prod::THREADS, R256Prod::SMEM, st>>>(sa);
-#ifdef RT_LAB
-    } else if (e->s256 && aligned) {
-        if (e->n == 4096) rt::spectro_s256_k<4096><<<grid, 256, rt::S256Cfg<4096>::SMEM, st>>>(sa);
-        else rt::spectro_s256_k<1024><<<grid, 256, rt::S256Cfg<1024>::SMEM, st>>>(sa);
-#endif
-    } else if (e->r16 && aligned) {
-        if (e->n == 4096) {
-            if (e->ci8) rt::spectro_r16_k<4096, true><<<grid, 256, rt::R16Cfg<4096>::SMEM, st>>>(sa);
-            else rt::spectro_r16_k<4096><<<grid, 256, rt::R16Cfg<4096>::SMEM, st>>>(sa);
-        } else {
-            if (e->ci8) rt::spectro_r16_k<1024, true><<<grid, 256, rt::R16Cfg<1024>::SMEM, st>>>(sa);
-            else rt::spectro_r16_k<1024><<<grid, 256, rt::R16Cfg<1024>::SMEM, st>>>(sa);
-        }
-    } else {
-        const size_t smem = (size_t)e->n * (2 * sizeof(float2) + sizeof(float)) + 16;
-        generic_kernel(e->cfg.sample_format)<<<grid, 256, smem, st>>>(sa);
-    }
+    if (e->ci8) launch_spectrogram<true>(e, sa, slot, aligned, st);
+    else launch_spectrogram<false>(e, sa, slot, aligned, st);
     CU(cudaGetLastError());
     if (evs) CU(cudaEventRecord(evs->ev[1], st));
     if (e->scan_stream) CU(cudaEventRecord(e->spec_done[slot], st));
@@ -1264,82 +1289,26 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
     }
     CU(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int), sc_st));
     if (evs) CU(cudaEventRecord(evs->ev[2], sc_st));
-    const bool lean = e->scan_lean;
-#ifdef RT_LAB
-    if (rt_lab_lean_per_sm > 0) e->lean_ctas = 148 * rt_lab_lean_per_sm;
-#endif
-    // the r16 kernel leaves one partial row per CTA: its n_chunks is the number of partial rows per unit either way
-    const bool sep_mean = !(use_reg && e->tc256) && (lean || e->n_chunks > 48);
-    if (sep_mean && !RT_LAB_SKIP(1)) {
-        row_mean_kernel<<<dim3((4 * e->n + 127) / 128, e->n_units), 128, 0, sc_st>>>(e->d_part[slot], e->d_avg[slot], e->n, e->n_chunks, e->T, (use_reg && !e->tc256) ? 1 : 0);
+    if (e->sep_mean) {
+        row_mean_kernel<<<dim3((4 * e->n + 127) / 128, e->n_units), 128, 0, sc_st>>>(e->d_part[slot], e->d_avg[slot], e->n, e->n_chunks, e->T, e->part_perm ? 1 : 0);
         CU(cudaGetLastError());
     }
     if (evs) CU(cudaEventRecord(evs->ev[3], sc_st));
 
     ScanArgs sc;
     sc.S = e->d_S[next]; sc.Sprev = e->d_S[e->cur]; sc.stream_stride = e->s_stride; sc.avg = e->d_avg[slot];
-    sc.part = ((use_reg && e->tc256) || sep_mean) ? nullptr : e->d_part[slot];
-    sc.n_chunks = e->n_chunks; sc.part_perm = (use_reg && !e->tc256) ? 1 : 0; sc.thr = e->d_thr; sc.has_prev = e->d_hasprev;
+    // the probe kernel takes the row means from the partial sums unless they are already in avg
+    sc.part = (e->kind == Spectro::TC256 || e->sep_mean) ? nullptr : e->d_part[slot];
+    sc.n_chunks = e->n_chunks; sc.part_perm = e->part_perm ? 1 : 0; sc.thr = e->d_thr; sc.has_prev = e->d_hasprev;
     sc.bpl = e->bpl;
     sc.snr = (float)e->cfg.snr_threshold;
     sc.n = e->n; sc.T = e->T; sc.stride = e->cfg.probe_stride; sc.n_probes = e->n_probes;
     sc.min_cols = e->cfg.min_cols; sc.max_cols = e->cfg.max_cols;
     sc.n_streams_scan = e->n_units;
-#ifdef RT_LAB
-    sc.lab_mode = rt_lab_extract_mode;
-#endif
     sc.widen = ((long long)e->n_units * e->T < 300000) ? 1 : 0;
     sc.work = e->d_work; sc.max_work = e->max_work; sc.counters = d_cnt; sc.rec = e->d_rec[slot]; sc.max_records = e->max_records;
-    const int pbins = std::min(e->n, 256);
-    int ppt = e->probe_ppt;
-#ifdef RT_LAB
-    if (rt_lab_probe_ppt > 0) ppt = rt_lab_probe_ppt;
-#endif
-    dim3 pgrid(((e->n + pbins - 1) / pbins) * ((e->n_probes + ppt - 1) / ppt), e->n_units);
-#ifdef RT_LAB
-    if (rt_lab_extract_mode & 16) sc.stream_stride = 0;    // timing only: the probe (and the walks) read unit 0's S, which stays in L2
-#endif
-#define RT_PROBE(L)                                                                        \
-    do {                                                                                   \
-        if (lean) probe_lean_kernel<L><<<e->lean_ctas, 128, 0, sc_st>>>(sc);               \
-        else if (ppt == 8) probe_kernel<L, 8><<<pgrid, pbins, 0, sc_st>>>(sc);             \
-        else if (ppt == 16) probe_kernel<L, 16><<<pgrid, pbins, 0, sc_st>>>(sc);           \
-        else probe_kernel<L, 32><<<pgrid, pbins, 0, sc_st>>>(sc);                          \
-    } while (0)
-    const int layout = use_reg ? (e->tc256 ? LAYOUT_TILE : LAYOUT_PERM) : (e->s256 && aligned) ? LAYOUT_PERMR : LAYOUT_LINEAR;
-    e->last_layout = layout;
-    if (RT_LAB_SKIP(2)) {}
-    else if (layout == LAYOUT_TILE) RT_PROBE(LAYOUT_TILE);
-    else if (layout == LAYOUT_PERM) RT_PROBE(LAYOUT_PERM);
-#ifdef RT_LAB
-    else if (layout == LAYOUT_PERMR) RT_PROBE(LAYOUT_PERMR);
-#endif
-    else RT_PROBE(LAYOUT_LINEAR);
-#undef RT_PROBE
-    CU(cudaGetLastError());
-    if (evs) CU(cudaEventRecord(evs->ev[4], sc_st));
-    // full size: one wave of 128-thread CTAs, four 32-cell windows per round trip; lean: one 32-cell window, no speculative
-    // forward fetch (fewest sectors: the kernel runs beside the spectrogram of the next launch)
-    int ex_ctas = e->lean_ctas;
-#ifdef RT_LAB
-    if (rt_lab_extract_mode & 2) sc.stream_stride = 0;     // every unit's walk reads unit 0's S (19 MB: stays in L2)
-    if (rt_lab_extract_per_sm > 0) ex_ctas = 148 * rt_lab_extract_per_sm;
-#endif
-#define RT_EXTRACT(L)                                                                      \
-    do {                                                                                   \
-        if (lean) extract2_kernel<L, 16><<<ex_ctas, 128, 0, sc_st>>>(sc);                  \
-        else if (sc.widen) extract2_kernel<L, 8, 4><<<148 * 24, 128, 0, sc_st>>>(sc);      \
-        else extract2_kernel<L, 8><<<148 * 24, 128, 0, sc_st>>>(sc);                       \
-    } while (0)
-    if (RT_LAB_SKIP(4)) {}
-    else if (layout == LAYOUT_TILE) RT_EXTRACT(LAYOUT_TILE);
-    else if (layout == LAYOUT_PERM) RT_EXTRACT(LAYOUT_PERM);
-#ifdef RT_LAB
-    else if (layout == LAYOUT_PERMR) RT_EXTRACT(LAYOUT_PERMR);
-#endif
-    else RT_EXTRACT(LAYOUT_LINEAR);
-#undef RT_EXTRACT
-    CU(cudaGetLastError());
+    int rc = e->scan(e, sc, sc_st, evs ? evs->ev[4] : nullptr);
+    if (rc != RT_OK) return rc;
     if (evs) CU(cudaEventRecord(evs->ev[5], sc_st));
 
     CU(cudaEventRecord(e->done[slot], sc_st));
@@ -1349,7 +1318,7 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         if (!h) { h = 1; e->hasprev_dirty = true; }
     e->launched = true;
     e->acc.launches += 1;
-    e->acc.kernels += sep_mean ? 4 : 3;
+    e->acc.kernels += e->sep_mean ? 4 : 3;
     return RT_OK;
 }
 
@@ -1450,21 +1419,14 @@ int rt_engine_read_spectrogram(rt_engine* e, int32_t stream, float* out) {
     CU(cudaStreamSynchronize(e->stream));
     for (auto& ls : e->lstream) if (ls) CU(cudaStreamSynchronize(ls));
     if (e->scan_stream) CU(cudaStreamSynchronize(e->scan_stream));
-    if (e->reg256) {
+    if (e->layout != LAYOUT_LINEAR) {
         if (!e->d_tmp) CU(cudaMalloc(&e->d_tmp, cells * sizeof(float)));
-        if (e->tc256) untile_kernel<LAYOUT_TILE><<<(unsigned)((cells + 255) / 256), 256, 0, e->stream>>>(src, e->d_tmp, (int)cells, 256, 1.f / e->pscale);
-        else untile_kernel<LAYOUT_PERM><<<(unsigned)((cells + 255) / 256), 256, 0, e->stream>>>(src, e->d_tmp, (int)cells, 256, 1.f);
+        const unsigned blocks = (unsigned)((cells + 255) / 256);
+        if (e->layout == LAYOUT_TILE) untile_kernel<LAYOUT_TILE><<<blocks, 256, 0, e->stream>>>(src, e->d_tmp, (int)cells, 256, 1.f / e->pscale);
+        else untile_kernel<LAYOUT_PERM><<<blocks, 256, 0, e->stream>>>(src, e->d_tmp, (int)cells, 256, 1.f);
         CU(cudaGetLastError());
         src = e->d_tmp;
     }
-#ifdef RT_LAB
-    else if (e->last_layout == LAYOUT_PERMR) {
-        if (!e->d_tmp) CU(cudaMalloc(&e->d_tmp, cells * sizeof(float)));
-        untile_kernel<LAYOUT_PERMR><<<(unsigned)((cells + 255) / 256), 256, 0, e->stream>>>(src, e->d_tmp, (int)cells, e->n, 1.f);
-        CU(cudaGetLastError());
-        src = e->d_tmp;
-    }
-#endif
     CU(cudaMemcpyAsync(out, src, cells * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     return RT_OK;

@@ -7,7 +7,7 @@
 // value is one packed register pair (fft_cpk.cuh).  A warp works on 2*NSEG consecutive segments per
 // round, fed by a per-warp ring of TMA bulk copies.  The engine instantiates spectro_reg256_v8 (end of this file: v7n with a
 // cheaper byte -> float front end); spectro_reg256_v7n and its template switches stay for tools/spectro_lab.cu (variant timing on
-// the GPU box; the other losing variants live in tools/spectro256_lab.cuh) and for lab builds of the engine with other S layouts.
+// the GPU box; the other losing variants live in tools/spectro256_lab.cuh).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
