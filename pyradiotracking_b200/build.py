@@ -1,4 +1,4 @@
-"""Build the native code in-tree: the CUDA engine and down-converter `pyradiotracking_b200/csrc/librtb200.so` (sm_100a only) and the CPython
+"""Build the native code in-tree: the CUDA engine, down-converter and filter bank `pyradiotracking_b200/csrc/librtb200.so` (sm_100a only) and the CPython
 helper of the host finaliser `pyradiotracking_b200/_rtfinal.so` (csrc/rt_pyfinal.c, gcc).
 
 nvcc cross-compiles without a GPU, so this runs in the build container; the resulting
@@ -15,9 +15,10 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "librtb200.so")
 PYFINAL_SRC = os.path.join(CSRC, "rt_pyfinal.c")
 PYFINAL = os.path.join(HERE, "_rtfinal.so")
-SOURCES = ["rt_engine.cu", "rt_ddc.cu", "rt_matcher.cpp"]
-HEADERS = ["predicate.h", "sample_format.cuh", "fft_cpk.cuh", "spectro256.cuh", "spectro_tc256.cuh", "spectro_r16.cuh", os.path.join("..", "..", "include", "rt_engine.h"),
-           os.path.join("..", "..", "include", "rt_matcher.h"), os.path.join("..", "..", "include", "rt_ddc.h")]
+SOURCES = ["rt_engine.cu", "rt_ddc.cu", "rt_fbank.cu", "rt_matcher.cpp"]
+HEADERS = ["predicate.h", "sample_format.cuh", "fir_history.cuh", "fft_cpk.cuh", "spectro256.cuh", "spectro_tc256.cuh", "spectro_r16.cuh", os.path.join("..", "..", "include", "rt_engine.h"),
+           os.path.join("..", "..", "include", "rt_matcher.h"), os.path.join("..", "..", "include", "rt_ddc.h"),
+           os.path.join("..", "..", "include", "rt_fbank.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-shared",

@@ -8,8 +8,8 @@
 //                       g_c of its CW channels.  A thread owns one channel and DDC_MR consecutive outputs: for a tap phase r
 //                       the outputs read consecutive samples of one polyphase row, so eight taps of a phase need 15 samples
 //                       and 8 taps (shared loads) for 64 complex products (128 packed fp32x2 FMAs, fft_cpk.cuh)
-//   ddc_history_kernel  the last L - 1 normalised samples of every input, for the next call (double-buffered)
-//   ddc_reset_kernel    rt_ddc_reset_input, applied in stream order at the next run
+//   fir_history_kernel  the last L - 1 normalised samples of every input, for the next call (double-buffered; fir_history.cuh)
+//   fir_reset_kernel    rt_ddc_reset_input, applied in stream order at the next run (fir_history.cuh)
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -21,6 +21,7 @@
 
 #include "../../include/rt_ddc.h"
 #include "fft_cpk.cuh"
+#include "fir_history.cuh"
 #include "sample_format.cuh"
 
 int rt_internal_fail(int code, const char* msg);   // rt_engine.cu: sets the thread-local rt_last_error() text
@@ -68,13 +69,6 @@ inline size_t ddc_smem(int cw, int mt, int D, int L) {
 }
 
 template <int FMT>
-__device__ __forceinline__ float2 ddc_sample(const DdcArgs& a, const unsigned char* row, const float2* hist, long long rel) {
-    if (rel < 0) return hist[a.hist_len + rel];
-    if (rel >= a.n_samples) return make_float2(0.f, 0.f);       // only read by outputs past the end, which are not stored
-    return rt::load_normalised<FMT>(row, rel, a.scale, a.offset);
-}
-
-template <int FMT>
 __global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgs a) {
     extern __shared__ float2 sm[];
     float2* gs = sm;                                    // [cw][L]
@@ -93,7 +87,7 @@ __global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgs a) {
     const int n_fill = (a.rows - DDC_PAD) * a.D;
     for (int t = tid; t < n_fill; t += DDC_THREADS) {
         const int q = t / a.D, b = t - q * a.D;
-        xs[b * a.rows + DDC_PAD + q] = t < span ? ddc_sample<FMT>(a, row, hist, rel0 + t) : make_float2(0.f, 0.f);
+        xs[b * a.rows + DDC_PAD + q] = t < span ? rt::fir_sample<FMT>(a, row, hist, rel0 + t) : make_float2(0.f, 0.f);
     }
     for (int p = tid; p < DDC_PAD * a.D; p += DDC_THREADS) {
         const int q = p / a.D;
@@ -151,21 +145,6 @@ __global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgs a) {
     }
 }
 
-template <int FMT>
-__global__ void ddc_history_kernel(const DdcArgs a) {
-    const int input = blockIdx.y;
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= a.hist_len) return;
-    const unsigned char* row = a.iq + (size_t)input * a.in_stride;
-    const float2* hist = a.hist + (size_t)input * a.hist_len;
-    a.hist_out[(size_t)input * a.hist_len + j] = ddc_sample<FMT>(a, row, hist, a.n_samples - a.hist_len + j);
-}
-
-__global__ void ddc_reset_kernel(float2* hist, uint32_t* off, int input, int hist_len, uint32_t off_value) {
-    for (int j = threadIdx.x; j < hist_len; j += blockDim.x) hist[(size_t)input * hist_len + j] = make_float2(0.f, 0.f);
-    if (threadIdx.x == 0) off[input] = off_value;
-}
-
 typedef void (*DdcKernel)(const DdcArgs);
 DdcKernel ddc_main(int fmt) {
     switch (fmt) {
@@ -177,10 +156,10 @@ DdcKernel ddc_main(int fmt) {
 }
 DdcKernel ddc_history(int fmt) {
     switch (fmt) {
-        case RT_SAMPLE_CU8: return ddc_history_kernel<RT_SAMPLE_CU8>;
-        case RT_SAMPLE_CI8: return ddc_history_kernel<RT_SAMPLE_CI8>;
-        case RT_SAMPLE_CI16: return ddc_history_kernel<RT_SAMPLE_CI16>;
-        default: return ddc_history_kernel<RT_SAMPLE_CF32>;
+        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, DdcArgs>;
+        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, DdcArgs>;
+        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, DdcArgs>;
+        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, DdcArgs>;
     }
 }
 
@@ -339,25 +318,14 @@ int rt_ddc_run(rt_ddc* d, void* cuda_stream, const void* iq, int32_t iq_on_devic
     const unsigned char* src = static_cast<const unsigned char*>(iq);
     size_t stride = d->n_in > 1 ? in_stride_bytes : row_bytes;
     if (!iq_on_device) {
-        const size_t sstride = (row_bytes + 255) & ~(size_t)255;
-        if (sstride * d->n_in > d->stage_bytes) {
-            DCU(cudaStreamSynchronize(st));
-            DCU(cudaFree(d->d_stage));
-            d->d_stage = nullptr;
-            d->stage_bytes = 0;
-            DCU(cudaMalloc(&d->d_stage, sstride * d->n_in));
-            d->stage_bytes = sstride * d->n_in;
-        }
-        DCU(cudaMemcpy2DAsync(d->d_stage, sstride, src, stride, row_bytes, d->n_in, cudaMemcpyHostToDevice, st));
-        src = d->d_stage;
-        stride = sstride;
+        DCU(rt::fir_stage_host_input(st, &src, &stride, row_bytes, d->n_in, &d->d_stage, &d->stage_bytes));
     } else if (((uintptr_t)src | (d->n_in > 1 ? stride : 0)) % (uintptr_t)d->info.bytes != 0) {
         return fail(RT_ERR_INVALID, "IQ pointer / input stride not aligned to one complex sample");
     }
 
     const int hist_len = std::max(1, d->L - 1);
     for (const auto& r : d->resets)
-        ddc_reset_kernel<<<1, 256, 0, st>>>(d->d_hist[d->cur], d->d_off, r.first, d->L - 1, r.second - d->advance);
+        rt::fir_reset_kernel<<<1, 256, 0, st>>>(d->d_hist[d->cur], d->d_off, r.first, d->L - 1, r.second - d->advance);
 
     DdcArgs a;
     a.iq = src;

@@ -7,9 +7,13 @@ channels -- complex baseband streams at fs / D centred on `center_freq + offset`
 analyzer unit, exactly as the reference analyses one RTL-SDR (one analyzer per SDR with its own centre frequency, device name
 and calibration; the shadow filter per analyzer).
 
-    Channelizer        the ctypes binding of rt_ddc: wideband blocks -> float32 [inputs * channels, 2 * samples / D] on the GPU
-    WidebandAnalyzer   a Channelizer plus one cf32 BatchAnalyzer with an analyzer unit per (input, channel); `replay()` drives it
-                       like a BatchAnalyzer with one stream per input
+    Channelizer        the ctypes binding of rt_ddc: wideband blocks -> float32 [inputs * channels, 2 * samples / D] on the GPU,
+                       for arbitrary channel offsets
+    FilterBank         the ctypes binding of rt_fbank (include/rt_fbank.h): the same quantity for every in-band channel of the
+                       uniform grid k fs / (2 D), -(D - 1) <= k <= D - 1, from a polyphase FFT filter bank (about L / log2(2 D)
+                       times less work than the DDC on that grid)
+    WidebandAnalyzer   a Channelizer (or, from `WidebandAnalyzer.full_band`, a FilterBank) plus one cf32 BatchAnalyzer with an
+                       analyzer unit per (input, channel); `replay()` drives it like a BatchAnalyzer with one stream per input
 
 Default channel filter (`default_taps`): `scipy.signal.firwin(8 D + 1, 1 / D, window=("kaiser", 8.0))`, cutoff at the channel
 Nyquist frequency fs / (2 D), unit gain at DC.  Its response (scipy.signal.freqz, D = 4, 8, 64 alike): flat within 0.07 dB over
@@ -35,6 +39,14 @@ KAISER_BETA = 8.0
 # every symbol include/rt_ddc.h declares
 EXPORTS = ("rt_ddc_create", "rt_ddc_destroy", "rt_ddc_reset_input", "rt_ddc_run")
 
+RT_FBANK_ABI_VERSION = 1
+FBANK_MIN_DECIMATION = 4     # RT_FBANK_MIN_DECIMATION
+FBANK_MAX_DECIMATION = 512   # RT_FBANK_MAX_DECIMATION
+MAX_ENGINE_UNITS = 65535     # rt_engine: n_streams * blocks_per_launch
+
+# every symbol include/rt_fbank.h declares
+FBANK_EXPORTS = ("rt_fbank_create", "rt_fbank_destroy", "rt_fbank_reset_input", "rt_fbank_run")
+
 
 class RtDdcConfig(ctypes.Structure):
     _fields_ = [
@@ -43,6 +55,15 @@ class RtDdcConfig(ctypes.Structure):
         ("n_taps", ctypes.c_int32), ("sample_format", ctypes.c_int32), ("reserved", ctypes.c_int32),
         ("sample_rate", ctypes.c_double), ("taps", ctypes.POINTER(ctypes.c_double)),
         ("phase_inc", ctypes.POINTER(ctypes.c_uint32)),
+    ]
+
+
+class RtFbankConfig(ctypes.Structure):
+    _fields_ = [
+        ("abi_version", ctypes.c_int32), ("cuda_device", ctypes.c_int32), ("n_inputs", ctypes.c_int32),
+        ("decimation", ctypes.c_int32), ("block_samples", ctypes.c_int64), ("n_taps", ctypes.c_int32),
+        ("sample_format", ctypes.c_int32), ("reserved", ctypes.c_int32), ("sample_rate", ctypes.c_double),
+        ("taps", ctypes.POINTER(ctypes.c_double)),
     ]
 
 
@@ -55,6 +76,11 @@ def _load():
         lib.rt_ddc_reset_input.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64]
         lib.rt_ddc_run.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_size_t,
                                    ctypes.c_int32, ctypes.c_void_p, ctypes.c_size_t]
+        lib.rt_fbank_create.argtypes = [ctypes.POINTER(RtFbankConfig), ctypes.POINTER(ctypes.c_void_p)]
+        lib.rt_fbank_destroy.argtypes = [ctypes.c_void_p]
+        lib.rt_fbank_destroy.restype = None
+        lib.rt_fbank_reset_input.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64]
+        lib.rt_fbank_run.argtypes = lib.rt_ddc_run.argtypes
         lib._ddc_types = True
     return lib
 
@@ -82,50 +108,38 @@ def channel_center_freqs(center_freq, offsets_hz: Sequence[float]) -> list:
     return [center_freq + off for off in offsets_hz]
 
 
-class Channelizer:
-    """The down-converter of include/rt_ddc.h for `n_inputs` wideband streams and one channel plan (`offsets_hz`)."""
+def grid_offsets(sample_rate: float, decimation: int) -> list:
+    """Offsets of the filter bank's channels, in row order: k fs / (2 D) for k = -(D - 1) ... D - 1."""
+    D = int(decimation)
+    return [k * sample_rate / (2 * D) for k in range(-(D - 1), D)]
 
-    def __init__(self, sample_rate: int, block_samples: int, offsets_hz: Sequence[float], decimation: int,
-                 taps: Optional[Sequence[float]] = None, sample_format: str = "cu8", n_inputs: int = 1, cuda_device: int = 0,
-                 blocks_per_launch: int = 1):
-        """`taps`: real FIR taps (odd count, at most MAX_TAPS); None: `default_taps(decimation)`.  ValueError for a channel plan
-        the down-converter cannot produce; the CUDA side checks the rest (engine.EngineError)."""
-        fs, D = sample_rate, int(decimation)
-        if not 2 <= D <= MAX_DECIMATION:
-            raise ValueError(f"decimation = {decimation}: must be in [2, {MAX_DECIMATION}]")
-        if fs % D or block_samples % D:
-            raise ValueError(f"sample_rate ({fs}) and block_samples ({block_samples}) must be multiples of the decimation {D}")
-        off = [float(o) for o in np.atleast_1d(offsets_hz)]
-        if not off:
-            raise ValueError("no channels")
-        for o in off:
-            if abs(o) + fs / (2 * D) > fs / 2:
-                raise ValueError(f"channel at {o} Hz with half-width {fs / (2 * D)} Hz does not lie inside the input band +-{fs / 2} Hz")
-        h = default_taps(D) if taps is None else np.asarray(taps, dtype=np.float64)
-        if h.ndim != 1 or len(h) % 2 == 0 or len(h) > MAX_TAPS:
-            raise ValueError(f"taps: an odd number of real taps up to {MAX_TAPS} is needed, got {h.shape}")
-        if not np.all(np.isfinite(h)):
-            raise ValueError("taps must be finite")
-        if blocks_per_launch < 1:
-            raise ValueError("blocks_per_launch must be >= 1")
+
+def grid_phase_increment(decimation: int) -> np.ndarray:
+    """The rt_ddc phase increment of every filter-bank row: ((k mod 2 D) 2^32) / (2 D), exact."""
+    D = int(decimation)
+    return np.array([((k % (2 * D)) << 32) // (2 * D) for k in range(-(D - 1), D)], dtype=np.uint32)
+
+
+def _check_taps(h: np.ndarray, max_taps: int) -> None:
+    if h.ndim != 1 or len(h) % 2 == 0 or len(h) > max_taps:
+        raise ValueError(f"taps: an odd number of real taps up to {max_taps} is needed, got {h.shape}")
+    if not np.all(np.isfinite(h)):
+        raise ValueError("taps must be finite")
+
+
+class _WidebandFrontEnd:
+    """What Channelizer and FilterBank share: the sample format, the handle's life cycle and the input / output handling of
+    `run`.  A subclass sets `_lib`, `_h`, `_destroy`, `_reset`, `_run`, `n_inputs`, `n_channels`, `block_samples`,
+    `decimation`, `blocks_per_launch`, `cuda_device` and calls `_set_format`."""
+
+    _h = None
+
+    def _set_format(self, sample_format: str) -> None:
         self.sample_format = _engine.sample_format_name(sample_format)
         code, dtype, self.sample_bytes = _engine.SAMPLE_FORMATS[self.sample_format]
+        self._format_code = code
         self._dtypes = (dtype, np.dtype(np.complex64)) if self.sample_format == "cf32_le" else (dtype,)
         self._dtype_names = tuple(d.name for d in self._dtypes)
-        self.sample_rate, self.block_samples, self.decimation = fs, int(block_samples), D
-        self.offsets_hz, self.taps = off, np.ascontiguousarray(h)
-        self.phase_inc = phase_increment(off, fs)
-        self.n_inputs, self.n_channels = int(n_inputs), len(off)
-        self.blocks_per_launch = int(blocks_per_launch)
-        self.cuda_device = cuda_device
-        self._lib = _load()
-        self._h = ctypes.c_void_p()
-        cfg = RtDdcConfig(
-            abi_version=RT_DDC_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, n_channels=self.n_channels,
-            block_samples=self.block_samples, decimation=D, n_taps=len(h), sample_format=code, reserved=0,
-            sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
-            phase_inc=self.phase_inc.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)))
-        _engine._check(self._lib.rt_ddc_create(ctypes.byref(cfg), ctypes.byref(self._h)))
 
     @property
     def n_taps(self) -> int:
@@ -133,7 +147,7 @@ class Channelizer:
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
-            self._lib.rt_ddc_destroy(self._h)            # waits for the last run
+            self._destroy(self._h)            # waits for the last run
             self._h = ctypes.c_void_p()
 
     def __del__(self):
@@ -150,10 +164,10 @@ class Channelizer:
 
     def reset_input(self, i: int, first_sample: int = 0) -> None:
         """Restart input `i` at the global sample index `first_sample`, with a zero filter history (from the next `run`)."""
-        _engine._check(self._lib.rt_ddc_reset_input(self._h, int(i), int(first_sample)))
+        _engine._check(self._reset(self._h, int(i), int(first_sample)))
 
     def run(self, iq, out=None):
-        """Down-convert `blocks_per_launch` consecutive blocks of every input: `iq` is `[n_inputs, 2 * blocks_per_launch *
+        """Channelize `blocks_per_launch` consecutive blocks of every input: `iq` is `[n_inputs, 2 * blocks_per_launch *
         block_samples]` elements of the sample format (cf32_le also complex64 with half as many) on the host (pinned or not) or a
         CUDA tensor / __cuda_array_interface__ object.  -> float32 CUDA tensor `[n_inputs * n_channels, 2 * blocks_per_launch *
         block_samples / D]` (interleaved I, Q; row i * n_channels + c), written by work enqueued on the current torch stream.  A
@@ -186,14 +200,94 @@ class Channelizer:
             out = torch.empty((self.n_inputs * self.n_channels, 2 * m), dtype=torch.float32, device=f"cuda:{self.cuda_device}")
         elif out.dtype != torch.float32 or tuple(out.shape) != (self.n_inputs * self.n_channels, 2 * m) or out.stride(1) != 1:
             raise ValueError("out must be float32 [n_inputs * n_channels, 2 * samples / D] with contiguous rows")
-        _engine._check(self._lib.rt_ddc_run(self._h, ctypes.c_void_p(cur.cuda_stream), ctypes.c_void_p(ptr), on_dev, stride,
-                                            self.blocks_per_launch, ctypes.c_void_p(out.data_ptr()), out.stride(0) * 4))
+        _engine._check(self._run(self._h, ctypes.c_void_p(cur.cuda_stream), ctypes.c_void_p(ptr), on_dev, stride,
+                                 self.blocks_per_launch, ctypes.c_void_p(out.data_ptr()), out.stride(0) * 4))
         return out
 
 
+class Channelizer(_WidebandFrontEnd):
+    """The down-converter of include/rt_ddc.h for `n_inputs` wideband streams and one channel plan (`offsets_hz`)."""
+
+    def __init__(self, sample_rate: int, block_samples: int, offsets_hz: Sequence[float], decimation: int,
+                 taps: Optional[Sequence[float]] = None, sample_format: str = "cu8", n_inputs: int = 1, cuda_device: int = 0,
+                 blocks_per_launch: int = 1):
+        """`taps`: real FIR taps (odd count, at most MAX_TAPS); None: `default_taps(decimation)`.  ValueError for a channel plan
+        the down-converter cannot produce; the CUDA side checks the rest (engine.EngineError)."""
+        fs, D = sample_rate, int(decimation)
+        if not 2 <= D <= MAX_DECIMATION:
+            raise ValueError(f"decimation = {decimation}: must be in [2, {MAX_DECIMATION}]")
+        if fs % D or block_samples % D:
+            raise ValueError(f"sample_rate ({fs}) and block_samples ({block_samples}) must be multiples of the decimation {D}")
+        off = [float(o) for o in np.atleast_1d(offsets_hz)]
+        if not off:
+            raise ValueError("no channels")
+        for o in off:
+            if abs(o) + fs / (2 * D) > fs / 2:
+                raise ValueError(f"channel at {o} Hz with half-width {fs / (2 * D)} Hz does not lie inside the input band +-{fs / 2} Hz")
+        h = default_taps(D) if taps is None else np.asarray(taps, dtype=np.float64)
+        _check_taps(h, MAX_TAPS)
+        if blocks_per_launch < 1:
+            raise ValueError("blocks_per_launch must be >= 1")
+        self._set_format(sample_format)
+        self.sample_rate, self.block_samples, self.decimation = fs, int(block_samples), D
+        self.offsets_hz, self.taps = off, np.ascontiguousarray(h)
+        self.phase_inc = phase_increment(off, fs)
+        self.n_inputs, self.n_channels = int(n_inputs), len(off)
+        self.blocks_per_launch = int(blocks_per_launch)
+        self.cuda_device = cuda_device
+        self._lib = _load()
+        self._destroy, self._reset, self._run = self._lib.rt_ddc_destroy, self._lib.rt_ddc_reset_input, self._lib.rt_ddc_run
+        self._h = ctypes.c_void_p()
+        cfg = RtDdcConfig(
+            abi_version=RT_DDC_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, n_channels=self.n_channels,
+            block_samples=self.block_samples, decimation=D, n_taps=len(h), sample_format=self._format_code, reserved=0,
+            sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+            phase_inc=self.phase_inc.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)))
+        _engine._check(self._lib.rt_ddc_create(ctypes.byref(cfg), ctypes.byref(self._h)))
+
+
+class FilterBank(_WidebandFrontEnd):
+    """The polyphase FFT filter bank of include/rt_fbank.h for `n_inputs` wideband streams: every in-band channel of the grid
+    k fs / (2 D), -(D - 1) <= k <= D - 1 (`n_channels` = 2 D - 1, row k + D - 1, ascending frequency).  Its output is the
+    quantity `Channelizer` computes for `offsets_hz` = `grid_offsets(fs, D)`, at about L / log2(2 D) times less work."""
+
+    def __init__(self, sample_rate: int, block_samples: int, decimation: int, taps: Optional[Sequence[float]] = None,
+                 sample_format: str = "cu8", n_inputs: int = 1, cuda_device: int = 0, blocks_per_launch: int = 1):
+        """`decimation` D: a power of two in [FBANK_MIN_DECIMATION, FBANK_MAX_DECIMATION]; `taps`: real FIR taps (odd count,
+        at most 16 D + 1); None: `default_taps(decimation)`.  ValueError for a plan the filter bank cannot produce; the CUDA
+        side checks the rest (engine.EngineError)."""
+        fs, D = sample_rate, int(decimation)
+        if not FBANK_MIN_DECIMATION <= D <= FBANK_MAX_DECIMATION or D & (D - 1):
+            raise ValueError(f"decimation = {decimation}: must be a power of two in [{FBANK_MIN_DECIMATION}, {FBANK_MAX_DECIMATION}]")
+        if fs % D or block_samples % D or block_samples < D:
+            raise ValueError(f"sample_rate ({fs}) and block_samples ({block_samples}) must be multiples of the decimation {D}")
+        h = default_taps(D) if taps is None else np.asarray(taps, dtype=np.float64)
+        _check_taps(h, 16 * D + 1)
+        if blocks_per_launch < 1:
+            raise ValueError("blocks_per_launch must be >= 1")
+        if not 1 <= int(n_inputs) <= 65535 or int(n_inputs) * (2 * D - 1) > 1 << 30:
+            raise ValueError(f"n_inputs = {n_inputs}: must be in [1, 65535] with n_inputs * (2 D - 1) <= 2^30")
+        self._set_format(sample_format)
+        self.sample_rate, self.block_samples, self.decimation = fs, int(block_samples), D
+        self.offsets_hz, self.taps = grid_offsets(fs, D), np.ascontiguousarray(h)
+        self.phase_inc = grid_phase_increment(D)
+        self.n_inputs, self.n_channels = int(n_inputs), 2 * D - 1
+        self.blocks_per_launch = int(blocks_per_launch)
+        self.cuda_device = cuda_device
+        self._lib = _load()
+        self._destroy, self._reset, self._run = self._lib.rt_fbank_destroy, self._lib.rt_fbank_reset_input, self._lib.rt_fbank_run
+        self._h = ctypes.c_void_p()
+        cfg = RtFbankConfig(
+            abi_version=RT_FBANK_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, decimation=D,
+            block_samples=self.block_samples, n_taps=len(h), sample_format=self._format_code, reserved=0,
+            sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)))
+        _engine._check(self._lib.rt_fbank_create(ctypes.byref(cfg), ctypes.byref(self._h)))
+
+
 class WidebandAnalyzer:
-    """Wideband recordings (`n_streams` inputs) analysed as narrowband SDR channels: a `Channelizer` plus one cf32_le
-    `BatchAnalyzer` with one analyzer unit per (input, channel).
+    """Wideband recordings (`n_streams` inputs) analysed as narrowband SDR channels: a `Channelizer` (the constructor, for
+    arbitrary `offsets_hz`) or a `FilterBank` (`full_band`, the whole uniform grid) plus one cf32_le `BatchAnalyzer` with one
+    analyzer unit per (input, channel).
 
     The channel analyzer runs at `sample_rate / decimation` with blocks of `block_samples / decimation`.  Channel c of input i
     is the device `f"{devices[i]}:{c}"` with the calibration of input i and the centre frequency `center_freq + offsets_hz[c]`;
@@ -208,6 +302,37 @@ class WidebandAnalyzer:
                  sdr_callback_length: Optional[int] = None, taps: Optional[Sequence[float]] = None, sample_format: str = "cu8",
                  cuda_device: int = 0, blocks_per_launch: int = 1, **batch_options):
         """`batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, ...)."""
+        block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
+        front = Channelizer(sample_rate, block, offsets_hz, int(decimation), taps=taps, sample_format=sample_format,
+                            n_inputs=len(self.devices), cuda_device=cuda_device, blocks_per_launch=blocks_per_launch)
+        self._attach(front, center_freq, fft_nperseg, fft_window, signal_min_duration_ms, signal_max_duration_ms,
+                     signal_threshold_dbw, snr_threshold_db, cuda_device, batch_options)
+
+    @classmethod
+    def full_band(cls, devices: Sequence[str], calibration_db: Sequence[float], sample_rate: int, center_freq, decimation: int,
+                  fft_nperseg: int, fft_window, signal_min_duration_ms: float, signal_max_duration_ms: float,
+                  signal_threshold_dbw: float, snr_threshold_db: float, sdr_callback_length: Optional[int] = None,
+                  taps: Optional[Sequence[float]] = None, sample_format: str = "cu8", cuda_device: int = 0,
+                  blocks_per_launch: int = 1, **batch_options) -> "WidebandAnalyzer":
+        """The whole band of every input: a `FilterBank` in front, so channel c (0 ... 2 D - 2) of input i is the device
+        `f"{devices[i]}:{c}"` at `center_freq + (c - D + 1) fs / (2 D)`.  Adjacent channels overlap by half their width, so
+        every frequency within fs / 2 - fs / (4 D) of the centre lies in the flat central half of some channel.  ValueError
+        when the 2 D - 1 channels of every input and block exceed the engine's 65535 analyzer units per launch."""
+        self = cls.__new__(cls)
+        block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
+        D = int(decimation)
+        units = len(self.devices) * (2 * D - 1) * int(blocks_per_launch)
+        if units > MAX_ENGINE_UNITS:
+            raise ValueError(f"{len(self.devices)} inputs * {2 * D - 1} channels * {blocks_per_launch} blocks per launch = {units} "
+                             f"analyzer units: more than the engine's {MAX_ENGINE_UNITS}")
+        front = FilterBank(sample_rate, block, D, taps=taps, sample_format=sample_format, n_inputs=len(self.devices),
+                           cuda_device=cuda_device, blocks_per_launch=blocks_per_launch)
+        self._attach(front, center_freq, fft_nperseg, fft_window, signal_min_duration_ms, signal_max_duration_ms,
+                     signal_threshold_dbw, snr_threshold_db, cuda_device, batch_options)
+        return self
+
+    def _check_plan(self, devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length) -> int:
+        """Set the devices and calibrations; -> the wideband block length."""
         self.devices = [str(d) for d in devices]
         self.calibration_db = [float(c) for c in calibration_db]
         if len(self.calibration_db) != len(self.devices):
@@ -216,8 +341,13 @@ class WidebandAnalyzer:
         D = int(decimation)
         if D >= 1 and block % D == 0 and (block // D) // fft_nperseg < 2:
             raise ValueError(f"a channel block of {block // D} samples holds fewer than two FFT segments of {fft_nperseg}")
-        self.ddc = Channelizer(sample_rate, block, offsets_hz, D, taps=taps, sample_format=sample_format,
-                               n_inputs=len(self.devices), cuda_device=cuda_device, blocks_per_launch=blocks_per_launch)
+        return block
+
+    def _attach(self, front, center_freq, fft_nperseg, fft_window, signal_min_duration_ms, signal_max_duration_ms,
+                signal_threshold_dbw, snr_threshold_db, cuda_device, batch_options) -> None:
+        """The channel analyzer behind the Channelizer or FilterBank `front` (kept as `self.ddc`)."""
+        self.ddc = front
+        sample_rate, block, D = front.sample_rate, front.block_samples, front.decimation
         self.n_streams = len(self.devices)
         self.n_channels = self.ddc.n_channels
         self.sample_rate, self.block_samples = sample_rate, block
