@@ -91,6 +91,40 @@ int rt_fbank_reset_input(rt_fbank *f, int32_t input, int64_t first_sample);
 int rt_fbank_run(rt_fbank *f, void *cuda_stream, const void *iq, int32_t iq_on_device, size_t in_stride_bytes, int32_t blocks,
                  void *out, size_t out_stride_bytes);
 
+/*
+ * DC and IQ-imbalance correction (default off).  A zero-IF receiver (HackRF, bladeRF 1, uncorrected GNU Radio captures) forms
+ * I and Q in two analog paths whose gain and phase differ slightly, so every signal at offset +f has a mirror image at -f,
+ * typically 25-40 dB down, and a DC spike at 0 Hz.  With the correction on, the filter runs on y instead of x (normative;
+ * tests/iq_oracle.py restates it in float64).  For input i and each block b of block_samples samples -- the handle's own
+ * block, whatever `blocks` a call carries -- with x the normalised samples of that block:
+ *
+ *     m = mean(x)      p = mean(|x - m|^2)      c = mean((x - m)^2)
+ *     w = -c / (p + sqrt(p^2 - |c|^2))  (w = 0 when p = 0)      y = (x - m) + w conj(x - m)
+ *
+ * Each block's samples get that block's own m and w.  mean(y^2) = c + 2 w p + w^2 conj(c) = 0: the block comes out proper,
+ * which removes the image; a proper block (c = 0) only loses its DC.  A frequency-flat gain / phase imbalance is undone up to a
+ * complex gain.  A frequency-dependent imbalance (I and Q filters that differ across the band) is only partly corrected: one
+ * w per block is the best flat correction, not a per-frequency one.  The history carried into the next run holds y, so
+ * switching the correction on or off in the middle of a recording changes only how later samples enter the filter.
+ *
+ * The moments are exact int64 sums of the elements for cu8, ci8 and ci16, and float64 sums of fixed 16384-sample tiles for
+ * cf32, in an order that does not depend on the call, the batch or the grid; m and w are formed in float64 and rounded to fp32
+ * once.  So every split of the same samples into calls, block counts or batches still gives bit-identical outputs.
+ *
+ * Accuracy with the correction on: the bound of the definition above holds for the quantity computed from y, with max |x|
+ * replaced by max |y| of the corrected samples (|y| <= (1 + |w|) |x - m|); the fp32 rounding of m and w adds at most a few
+ * units of 2^-24 (|m| + |w| max |x - m|) per sample, inside the same bound.
+ *
+ * Limit: block_samples <= 2^30 while the correction is on.
+ */
+
+/* enable != 0: correct every block from the next rt_fbank_run on, in that run's stream order (like rt_fbank_reset_input); 0: stop.
+ * RT_ERR_INVALID when block_samples exceeds 2^30. */
+int rt_fbank_set_iq_correction(rt_fbank *f, int32_t enable);
+/* Test hook: m and w of (input, block) of the last run, out = {m.re, m.im, w.re, w.im} (fp32, as the kernels apply them).
+ * Waits for that run.  RT_ERR_INVALID when the last run did not correct, or for an index outside it. */
+int rt_fbank_read_iq_correction(rt_fbank *f, int32_t input, int32_t block, float out[4]);
+
 #ifdef __cplusplus
 }
 #endif

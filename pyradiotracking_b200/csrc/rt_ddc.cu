@@ -10,12 +10,15 @@
 //                       and 8 taps (shared loads) for 64 complex products (128 packed fp32x2 FMAs, fft_cpk.cuh)
 //   fir_history_kernel  the last L - 1 normalised samples of every input, for the next call (double-buffered; fir_history.cuh)
 //   fir_reset_kernel    rt_ddc_reset_input, applied in stream order at the next run (fir_history.cuh)
+//   iq_moments_kernel, iq_coef_kernel   with rt_ddc_set_iq_correction on: each block's DC and IQ-imbalance coefficients,
+//                       which the IQ = true instantiations of the two kernels above apply as they decode (iq_correction.cuh)
 #include <cuda_runtime.h>
 
 #include <algorithm>
 #include <cmath>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -61,6 +64,12 @@ struct DdcArgs {
     int D, L, n_channels, cw, lg_cw, mt, rows;
     float scale, offset;
 };
+// the arguments of the corrected kernels (rt_ddc_set_iq_correction)
+struct DdcArgsIq : DdcArgs {
+    rt::IqCorrArgs corr;
+};
+template <bool IQ>
+using DdcArgsOf = typename std::conditional<IQ, DdcArgsIq, DdcArgs>::type;
 
 // polyphase row length: a zero pad, the MT outputs' own samples and the (L - 1) / D earlier ones, odd (conflict-free fills)
 inline int ddc_rows(int mt, int D, int L) { return (DDC_PAD + mt + (L - 1) / D) | 1; }
@@ -68,8 +77,8 @@ inline size_t ddc_smem(int cw, int mt, int D, int L) {
     return (size_t)cw * L * sizeof(float2) + (size_t)D * ddc_rows(mt, D, L) * sizeof(float2);
 }
 
-template <int FMT>
-__global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgs a) {
+template <int FMT, bool IQ>
+__global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgsOf<IQ> a) {
     extern __shared__ float2 sm[];
     float2* gs = sm;                                    // [cw][L]
     float2* xs = sm + (size_t)a.cw * a.L;               // [D][rows]
@@ -85,9 +94,10 @@ __global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgs a) {
     const long long rel0 = m0 * a.D - (a.L - 1);
     const long long span = (long long)(a.mt - 1) * a.D + a.L;
     const int n_fill = (a.rows - DDC_PAD) * a.D;
+    const rt::IqSpan<IQ> sp = rt::iq_span<IQ>(a, input, rel0);
     for (int t = tid; t < n_fill; t += DDC_THREADS) {
         const int q = t / a.D, b = t - q * a.D;
-        xs[b * a.rows + DDC_PAD + q] = t < span ? rt::fir_sample<FMT>(a, row, hist, rel0 + t) : make_float2(0.f, 0.f);
+        xs[b * a.rows + DDC_PAD + q] = t < span ? rt::fir_sample<FMT, IQ>(a, row, hist, rel0 + t, sp) : make_float2(0.f, 0.f);
     }
     for (int p = tid; p < DDC_PAD * a.D; p += DDC_THREADS) {
         const int q = p / a.D;
@@ -145,22 +155,43 @@ __global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgs a) {
     }
 }
 
-typedef void (*DdcKernel)(const DdcArgs);
-DdcKernel ddc_main(int fmt) {
+template <bool IQ>
+using DdcKernel = void (*)(const DdcArgsOf<IQ>);
+template <bool IQ>
+DdcKernel<IQ> ddc_main(int fmt) {
     switch (fmt) {
-        case RT_SAMPLE_CU8: return ddc_kernel<RT_SAMPLE_CU8>;
-        case RT_SAMPLE_CI8: return ddc_kernel<RT_SAMPLE_CI8>;
-        case RT_SAMPLE_CI16: return ddc_kernel<RT_SAMPLE_CI16>;
-        default: return ddc_kernel<RT_SAMPLE_CF32>;
+        case RT_SAMPLE_CU8: return ddc_kernel<RT_SAMPLE_CU8, IQ>;
+        case RT_SAMPLE_CI8: return ddc_kernel<RT_SAMPLE_CI8, IQ>;
+        case RT_SAMPLE_CI16: return ddc_kernel<RT_SAMPLE_CI16, IQ>;
+        default: return ddc_kernel<RT_SAMPLE_CF32, IQ>;
     }
 }
-DdcKernel ddc_history(int fmt) {
+template <bool IQ>
+DdcKernel<IQ> ddc_history(int fmt) {
     switch (fmt) {
-        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, DdcArgs>;
-        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, DdcArgs>;
-        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, DdcArgs>;
-        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, DdcArgs>;
+        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, IQ, DdcArgsOf<IQ>>;
+        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, IQ, DdcArgsOf<IQ>>;
+        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, IQ, DdcArgsOf<IQ>>;
+        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, IQ, DdcArgsOf<IQ>>;
     }
+}
+
+// the filter kernel and the history kernel of one run
+template <bool IQ>
+void ddc_launch(const DdcArgsOf<IQ>& a, int fmt, dim3 grid, size_t smem, int n_in, cudaStream_t st) {
+    ddc_main<IQ>(fmt)<<<grid, DDC_THREADS, smem, st>>>(a);
+    if (a.L > 1) ddc_history<IQ>(fmt)<<<dim3((unsigned)((a.L - 1 + 127) / 128), (unsigned)n_in), 128, 0, st>>>(a);
+}
+
+// the limit belongs to the kernel: only ever raise it (handles with other geometries may exist in this process)
+template <class Kernel>
+int raise_smem_limit(Kernel k, size_t smem) {
+    cudaFuncAttributes fa;
+    cudaError_t ferr = cudaFuncGetAttributes(&fa, k);
+    if (ferr != cudaSuccess)
+        return fail(RT_ERR_CUDA, std::string("kernels not loadable on this device (built for sm_100a only): ") + cudaGetErrorString(ferr));
+    if ((size_t)fa.maxDynamicSharedSizeBytes < smem) DCU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    return RT_OK;
 }
 
 }  // namespace
@@ -182,6 +213,7 @@ struct rt_ddc {
     size_t stage_bytes = 0;
     cudaEvent_t done = nullptr;
     bool ran = false;
+    rt::IqState iq;                                     // rt_ddc_set_iq_correction
 };
 
 static void free_ddc(rt_ddc* d) {
@@ -197,6 +229,7 @@ static void free_ddc(rt_ddc* d) {
     cudaFree(d->d_hist[0]);
     cudaFree(d->d_hist[1]);
     cudaFree(d->d_stage);
+    d->iq.release();
     delete d;
 }
 
@@ -234,15 +267,11 @@ int rt_ddc_create(const rt_ddc_config* cfg, rt_ddc** out) {
     if (cfg->cuda_device < 0 || cfg->cuda_device >= ndev) return fail(RT_ERR_CUDA, "no such CUDA device (this engine has no CPU fallback)");
     DCU(cudaSetDevice(cfg->cuda_device));
     {
-        // the limit belongs to the kernel: only ever raise it (handles with other geometries may exist in this process)
         static std::mutex mu;
         std::lock_guard<std::mutex> lock(mu);
-        cudaFuncAttributes fa;
-        cudaError_t ferr = cudaFuncGetAttributes(&fa, ddc_main(cfg->sample_format));
-        if (ferr != cudaSuccess)
-            return fail(RT_ERR_CUDA, std::string("kernels not loadable on this device (built for sm_100a only): ") + cudaGetErrorString(ferr));
-        if ((size_t)fa.maxDynamicSharedSizeBytes < smem)
-            DCU(cudaFuncSetAttribute(ddc_main(cfg->sample_format), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int rc = raise_smem_limit(ddc_main<false>(cfg->sample_format), smem);
+        if (rc == RT_OK) rc = raise_smem_limit(ddc_main<true>(cfg->sample_format), smem);
+        if (rc != RT_OK) return rc;
     }
 
     rt_ddc* d = new rt_ddc();
@@ -323,7 +352,8 @@ int rt_ddc_run(rt_ddc* d, void* cuda_stream, const void* iq, int32_t iq_on_devic
         return fail(RT_ERR_INVALID, "IQ pointer / input stride not aligned to one complex sample");
     }
 
-    const int hist_len = std::max(1, d->L - 1);
+    rt::IqCorrArgs corr;
+    DCU(rt::iq_prepare(d->iq, st, d->done, d->ran, d->fmt, d->info, src, stride, d->n_in, d->block, blocks, &corr));
     for (const auto& r : d->resets)
         rt::fir_reset_kernel<<<1, 256, 0, st>>>(d->d_hist[d->cur], d->d_off, r.first, d->L - 1, r.second - d->advance);
 
@@ -351,14 +381,36 @@ int rt_ddc_run(rt_ddc* d, void* cuda_stream, const void* iq, int32_t iq_on_devic
     a.scale = (float)(1.0 / d->info.full_scale);
     a.offset = (float)d->info.offset;
     const dim3 grid((unsigned)((m_total + d->mt - 1) / d->mt), (unsigned)((d->nch + d->cw - 1) / d->cw), (unsigned)d->n_in);
-    ddc_main(d->fmt)<<<grid, DDC_THREADS, d->smem, st>>>(a);
-    if (d->L > 1) ddc_history(d->fmt)<<<dim3((unsigned)((hist_len + 127) / 128), (unsigned)d->n_in), 128, 0, st>>>(a);
+    if (d->iq.applied) {
+        DdcArgsIq ai;
+        static_cast<DdcArgs&>(ai) = a;
+        ai.corr = corr;
+        ddc_launch<true>(ai, d->fmt, grid, d->smem, d->n_in, st);
+    } else {
+        ddc_launch<false>(a, d->fmt, grid, d->smem, d->n_in, st);
+    }
     DCU(cudaGetLastError());
     DCU(cudaEventRecord(d->done, st));
     d->ran = true;
     d->resets.clear();
     d->cur ^= d->L > 1 ? 1 : 0;
     d->advance += (uint32_t)(uint64_t)n;
+    return RT_OK;
+}
+
+int rt_ddc_set_iq_correction(rt_ddc* d, int32_t enable) {
+    if (!d) return fail(RT_ERR_INVALID, "null handle");
+    if (enable && d->block > rt::IQ_MAX_BLOCK) return fail(RT_ERR_INVALID, "block_samples must be <= 2^30 for the IQ correction");
+    d->iq.on = enable != 0;
+    return RT_OK;
+}
+
+int rt_ddc_read_iq_correction(rt_ddc* d, int32_t input, int32_t block, float out[4]) {
+    if (!d || !out) return fail(RT_ERR_INVALID, "null argument");
+    if (!d->iq.applied) return fail(RT_ERR_INVALID, "the last run did not apply the IQ correction");
+    if (input < 0 || input >= d->n_in || block < 0 || block >= d->iq.blocks) return fail(RT_ERR_INVALID, "bad input / block index");
+    DCU(cudaSetDevice(d->dev));
+    DCU(rt::iq_read(d->iq, d->done, input, block, out));
     return RT_OK;
 }
 

@@ -10,12 +10,15 @@
 //                       so reading one bin across frames is free of bank conflicts)
 //   fir_history_kernel  the last L - 1 normalised samples of every input, for the next call (double-buffered; fir_history.cuh)
 //   fir_reset_kernel    rt_fbank_reset_input, applied in stream order at the next run (fir_history.cuh)
+//   iq_moments_kernel, iq_coef_kernel   with rt_fbank_set_iq_correction on: each block's DC and IQ-imbalance coefficients,
+//                       which the IQ = true instantiations of the two kernels above apply as they decode (iq_correction.cuh)
 #include <cuda_runtime.h>
 
 #include <algorithm>
 #include <cmath>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -58,14 +61,20 @@ struct FbankArgs {
     int D, L, lg_c, mt;
     float scale, offset;
 };
+// the arguments of the corrected kernels (rt_fbank_set_iq_correction)
+struct FbankArgsIq : FbankArgs {
+    rt::IqCorrArgs corr;
+};
+template <bool IQ>
+using FbankArgsOf = typename std::conditional<IQ, FbankArgsIq, FbankArgs>::type;
 
 inline size_t fbank_smem(int mt, int D, int L) {
     const int C = 2 * D;
     return ((size_t)(mt - 1) * D + L + (size_t)mt * (C + 1) + C / 2) * sizeof(float2);
 }
 
-template <int FMT>
-__global__ void __launch_bounds__(FB_THREADS) fbank_kernel(const FbankArgs a) {
+template <int FMT, bool IQ>
+__global__ void __launch_bounds__(FB_THREADS) fbank_kernel(const FbankArgsOf<IQ> a) {
     extern __shared__ float2 sm[];
     const int C = 1 << a.lg_c, CP = C + 1, D = a.D, L = a.L, tid = threadIdx.x;
     const int span = (a.mt - 1) * D + L;
@@ -77,7 +86,8 @@ __global__ void __launch_bounds__(FB_THREADS) fbank_kernel(const FbankArgs a) {
     const unsigned char* row = a.iq + (size_t)input * a.in_stride;
     const float2* hist = a.hist + (size_t)input * a.hist_len;
     const long long rel0 = m0 * D - (L - 1);
-    for (int t = tid; t < span; t += FB_THREADS) xs[t] = rt::fir_sample<FMT>(a, row, hist, rel0 + t);
+    const rt::IqSpan<IQ> sp = rt::iq_span<IQ>(a, input, rel0);
+    for (int t = tid; t < span; t += FB_THREADS) xs[t] = rt::fir_sample<FMT, IQ>(a, row, hist, rel0 + t, sp);
     for (int t = tid; t < C / 2; t += FB_THREADS) tw[t] = a.twiddle[t];
     __syncthreads();
 
@@ -132,22 +142,43 @@ __global__ void __launch_bounds__(FB_THREADS) fbank_kernel(const FbankArgs a) {
     }
 }
 
-typedef void (*FbankKernel)(const FbankArgs);
-FbankKernel fbank_main(int fmt) {
+template <bool IQ>
+using FbankKernel = void (*)(const FbankArgsOf<IQ>);
+template <bool IQ>
+FbankKernel<IQ> fbank_main(int fmt) {
     switch (fmt) {
-        case RT_SAMPLE_CU8: return fbank_kernel<RT_SAMPLE_CU8>;
-        case RT_SAMPLE_CI8: return fbank_kernel<RT_SAMPLE_CI8>;
-        case RT_SAMPLE_CI16: return fbank_kernel<RT_SAMPLE_CI16>;
-        default: return fbank_kernel<RT_SAMPLE_CF32>;
+        case RT_SAMPLE_CU8: return fbank_kernel<RT_SAMPLE_CU8, IQ>;
+        case RT_SAMPLE_CI8: return fbank_kernel<RT_SAMPLE_CI8, IQ>;
+        case RT_SAMPLE_CI16: return fbank_kernel<RT_SAMPLE_CI16, IQ>;
+        default: return fbank_kernel<RT_SAMPLE_CF32, IQ>;
     }
 }
-FbankKernel fbank_history(int fmt) {
+template <bool IQ>
+FbankKernel<IQ> fbank_history(int fmt) {
     switch (fmt) {
-        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, FbankArgs>;
-        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, FbankArgs>;
-        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, FbankArgs>;
-        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, FbankArgs>;
+        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, IQ, FbankArgsOf<IQ>>;
+        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, IQ, FbankArgsOf<IQ>>;
+        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, IQ, FbankArgsOf<IQ>>;
+        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, IQ, FbankArgsOf<IQ>>;
     }
+}
+
+// the filter kernel and the history kernel of one run
+template <bool IQ>
+void fbank_launch(const FbankArgsOf<IQ>& a, int fmt, dim3 grid, size_t smem, int n_in, cudaStream_t st) {
+    fbank_main<IQ>(fmt)<<<grid, FB_THREADS, smem, st>>>(a);
+    if (a.L > 1) fbank_history<IQ>(fmt)<<<dim3((unsigned)((a.L - 1 + 127) / 128), (unsigned)n_in), 128, 0, st>>>(a);
+}
+
+// the limit belongs to the kernel: only ever raise it (handles with other geometries may exist in this process)
+template <class Kernel>
+int raise_smem_limit(Kernel k, size_t smem) {
+    cudaFuncAttributes fa;
+    cudaError_t ferr = cudaFuncGetAttributes(&fa, k);
+    if (ferr != cudaSuccess)
+        return fail(RT_ERR_CUDA, std::string("kernels not loadable on this device (built for sm_100a only): ") + cudaGetErrorString(ferr));
+    if ((size_t)fa.maxDynamicSharedSizeBytes < smem) FCU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    return RT_OK;
 }
 
 }  // namespace
@@ -169,6 +200,7 @@ struct rt_fbank {
     size_t stage_bytes = 0;
     cudaEvent_t done = nullptr;
     bool ran = false;
+    rt::IqState iq;                                     // rt_fbank_set_iq_correction
 };
 
 static void free_fbank(rt_fbank* f) {
@@ -184,6 +216,7 @@ static void free_fbank(rt_fbank* f) {
     cudaFree(f->d_hist[0]);
     cudaFree(f->d_hist[1]);
     cudaFree(f->d_stage);
+    f->iq.release();
     delete f;
 }
 
@@ -221,15 +254,11 @@ int rt_fbank_create(const rt_fbank_config* cfg, rt_fbank** out) {
     if (cfg->cuda_device < 0 || cfg->cuda_device >= ndev) return fail(RT_ERR_CUDA, "no such CUDA device (this engine has no CPU fallback)");
     FCU(cudaSetDevice(cfg->cuda_device));
     {
-        // the limit belongs to the kernel: only ever raise it (handles with other geometries may exist in this process)
         static std::mutex mu;
         std::lock_guard<std::mutex> lock(mu);
-        cudaFuncAttributes fa;
-        cudaError_t ferr = cudaFuncGetAttributes(&fa, fbank_main(cfg->sample_format));
-        if (ferr != cudaSuccess)
-            return fail(RT_ERR_CUDA, std::string("kernels not loadable on this device (built for sm_100a only): ") + cudaGetErrorString(ferr));
-        if ((size_t)fa.maxDynamicSharedSizeBytes < smem)
-            FCU(cudaFuncSetAttribute(fbank_main(cfg->sample_format), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int rc = raise_smem_limit(fbank_main<false>(cfg->sample_format), smem);
+        if (rc == RT_OK) rc = raise_smem_limit(fbank_main<true>(cfg->sample_format), smem);
+        if (rc != RT_OK) return rc;
     }
 
     rt_fbank* f = new rt_fbank();
@@ -308,7 +337,8 @@ int rt_fbank_run(rt_fbank* f, void* cuda_stream, const void* iq, int32_t iq_on_d
         return fail(RT_ERR_INVALID, "IQ pointer / input stride not aligned to one complex sample");
     }
 
-    const int hist_len = std::max(1, f->L - 1);
+    rt::IqCorrArgs corr;
+    FCU(rt::iq_prepare(f->iq, st, f->done, f->ran, f->fmt, f->info, src, stride, f->n_in, f->block, blocks, &corr));
     for (const auto& r : f->resets)
         rt::fir_reset_kernel<<<1, 256, 0, st>>>(f->d_hist[f->cur], f->d_off, r.first, f->L - 1, r.second - f->advance);
 
@@ -333,14 +363,36 @@ int rt_fbank_run(rt_fbank* f, void* cuda_stream, const void* iq, int32_t iq_on_d
     a.scale = (float)(1.0 / f->info.full_scale);
     a.offset = (float)f->info.offset;
     const dim3 grid((unsigned)((m_total + f->mt - 1) / f->mt), (unsigned)f->n_in);
-    fbank_main(f->fmt)<<<grid, FB_THREADS, f->smem, st>>>(a);
-    if (f->L > 1) fbank_history(f->fmt)<<<dim3((unsigned)((hist_len + 127) / 128), (unsigned)f->n_in), 128, 0, st>>>(a);
+    if (f->iq.applied) {
+        FbankArgsIq ai;
+        static_cast<FbankArgs&>(ai) = a;
+        ai.corr = corr;
+        fbank_launch<true>(ai, f->fmt, grid, f->smem, f->n_in, st);
+    } else {
+        fbank_launch<false>(a, f->fmt, grid, f->smem, f->n_in, st);
+    }
     FCU(cudaGetLastError());
     FCU(cudaEventRecord(f->done, st));
     f->ran = true;
     f->resets.clear();
     f->cur ^= f->L > 1 ? 1 : 0;
     f->advance += (uint32_t)(uint64_t)n;
+    return RT_OK;
+}
+
+int rt_fbank_set_iq_correction(rt_fbank* f, int32_t enable) {
+    if (!f) return fail(RT_ERR_INVALID, "null handle");
+    if (enable && f->block > rt::IQ_MAX_BLOCK) return fail(RT_ERR_INVALID, "block_samples must be <= 2^30 for the IQ correction");
+    f->iq.on = enable != 0;
+    return RT_OK;
+}
+
+int rt_fbank_read_iq_correction(rt_fbank* f, int32_t input, int32_t block, float out[4]) {
+    if (!f || !out) return fail(RT_ERR_INVALID, "null argument");
+    if (!f->iq.applied) return fail(RT_ERR_INVALID, "the last run did not apply the IQ correction");
+    if (input < 0 || input >= f->n_in || block < 0 || block >= f->iq.blocks) return fail(RT_ERR_INVALID, "bad input / block index");
+    FCU(cudaSetDevice(f->dev));
+    FCU(rt::iq_read(f->iq, f->done, input, block, out));
     return RT_OK;
 }
 

@@ -169,3 +169,33 @@ def bytes_to_iq(u8: np.ndarray) -> np.ndarray:
     iq /= 127.5
     iq -= 1 + 1j
     return iq
+
+
+def quantise(x: np.ndarray, fmt: str) -> np.ndarray:
+    """Interleaved I,Q elements of the sample format `fmt` (cu8, ci8, ci16_le, cf32_le) whose normalised value is (close to)
+    the complex samples x: rounded and clipped to the format's range."""
+    v = np.ascontiguousarray(x, np.complex128).view(np.float64)
+    if fmt == "cu8":
+        return np.clip(np.rint(v * 127.5 + 127.5), 0, 255).astype(np.uint8)
+    if fmt == "ci8":
+        return np.clip(np.rint(v * 128.0), -128, 127).astype(np.int8)
+    if fmt == "ci16_le":
+        return np.clip(np.rint(v * 32768.0), -32768, 32767).astype("<i2")
+    if fmt == "cf32_le":
+        return v.astype("<f4")
+    raise ValueError(f"unknown sample format {fmt}")
+
+
+def zero_if_imbalance(x: np.ndarray, gain_db: float = 0.0, phase_deg: float = 0.0, dc: complex = 0j) -> np.ndarray:
+    """What a zero-IF receiver with unequal I and Q paths makes of the complex baseband x: I' = Re x, Q' = g (Im x cos phi +
+    Re x sin phi) with g = 10^(gain_db / 20), plus a DC offset.  That is mu x + nu conj(x) + dc with mu = (1 + g e^(i phi)) / 2
+    and nu = (1 - g e^(-i phi)) / 2, so a signal at +f leaves a mirror image at -f |mu|^2 / |nu|^2 below it (0.5 dB / 3 deg:
+    28 dB; 1 dB / 6 deg: 22 dB)."""
+    x = np.asarray(x, np.complex128)
+    g, phi = 10.0 ** (gain_db / 20.0), np.deg2rad(phase_deg)
+    return x.real + 1j * g * (x.imag * np.cos(phi) + x.real * np.sin(phi)) + dc
+
+
+def zero_if_capture(x: np.ndarray, fmt: str, gain_db: float = 0.0, phase_deg: float = 0.0, dc: complex = 0j) -> np.ndarray:
+    """A synthetic zero-IF recording: `zero_if_imbalance` of x, quantised to `fmt` (ci8 is what a HackRF writes)."""
+    return quantise(zero_if_imbalance(x, gain_db, phase_deg, dc), fmt)

@@ -15,6 +15,10 @@ and calibration; the shadow filter per analyzer).
     WidebandAnalyzer   a Channelizer (or, from `WidebandAnalyzer.full_band`, a FilterBank) plus one cf32 BatchAnalyzer with an
                        analyzer unit per (input, channel); `replay()` drives it like a BatchAnalyzer with one stream per input
 
+`iq_correction=True` (both front ends, default off) removes each wideband block's DC and makes the block proper before the
+channel filter (include/rt_ddc.h): the mirror images a zero-IF receiver (HackRF, bladeRF 1) puts at -f of every signal at +f
+then no longer reach the channel analyzers as tags that do not exist.
+
 Default channel filter (`default_taps`): `scipy.signal.firwin(8 D + 1, 1 / D, window=("kaiser", 8.0))`, cutoff at the channel
 Nyquist frequency fs / (2 D), unit gain at DC.  Its response (scipy.signal.freqz, D = 4, 8, 64 alike): flat within 0.07 dB over
 the central half of the channel (|f| <= fs / (4 D)), -6.0 dB at the channel edge, at most -42 dB from 1.5 times the edge on
@@ -37,7 +41,8 @@ MAX_DECIMATION = 1024     # RT_DDC_MAX_DECIMATION
 KAISER_BETA = 8.0
 
 # every symbol include/rt_ddc.h declares
-EXPORTS = ("rt_ddc_create", "rt_ddc_destroy", "rt_ddc_reset_input", "rt_ddc_run")
+EXPORTS = ("rt_ddc_create", "rt_ddc_destroy", "rt_ddc_reset_input", "rt_ddc_run", "rt_ddc_set_iq_correction",
+           "rt_ddc_read_iq_correction")
 
 RT_FBANK_ABI_VERSION = 1
 FBANK_MIN_DECIMATION = 4     # RT_FBANK_MIN_DECIMATION
@@ -45,7 +50,8 @@ FBANK_MAX_DECIMATION = 512   # RT_FBANK_MAX_DECIMATION
 MAX_ENGINE_UNITS = 65535     # rt_engine: n_streams * blocks_per_launch
 
 # every symbol include/rt_fbank.h declares
-FBANK_EXPORTS = ("rt_fbank_create", "rt_fbank_destroy", "rt_fbank_reset_input", "rt_fbank_run")
+FBANK_EXPORTS = ("rt_fbank_create", "rt_fbank_destroy", "rt_fbank_reset_input", "rt_fbank_run", "rt_fbank_set_iq_correction",
+                 "rt_fbank_read_iq_correction")
 
 
 class RtDdcConfig(ctypes.Structure):
@@ -81,6 +87,10 @@ def _load():
         lib.rt_fbank_destroy.restype = None
         lib.rt_fbank_reset_input.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64]
         lib.rt_fbank_run.argtypes = lib.rt_ddc_run.argtypes
+        for name in ("rt_ddc", "rt_fbank"):
+            getattr(lib, name + "_set_iq_correction").argtypes = [ctypes.c_void_p, ctypes.c_int32]
+            getattr(lib, name + "_read_iq_correction").argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32,
+                                                                   ctypes.POINTER(ctypes.c_float)]
         lib._ddc_types = True
     return lib
 
@@ -129,10 +139,12 @@ def _check_taps(h: np.ndarray, max_taps: int) -> None:
 
 class _WidebandFrontEnd:
     """What Channelizer and FilterBank share: the sample format, the handle's life cycle and the input / output handling of
-    `run`.  A subclass sets `_lib`, `_h`, `_destroy`, `_reset`, `_run`, `n_inputs`, `n_channels`, `block_samples`,
-    `decimation`, `blocks_per_launch`, `cuda_device` and calls `_set_format`."""
+    `run`.  A subclass sets `_lib`, `_h`, `_destroy`, `_reset`, `_run`, `_set_iq`, `_read_iq`, `n_inputs`, `n_channels`,
+    `block_samples`, `decimation`, `blocks_per_launch`, `cuda_device`, calls `_set_format` and, after creating the handle,
+    `set_iq_correction`."""
 
     _h = None
+    iq_correction = False
 
     def _set_format(self, sample_format: str) -> None:
         self.sample_format = _engine.sample_format_name(sample_format)
@@ -161,6 +173,18 @@ class _WidebandFrontEnd:
 
     def __exit__(self, *exc):
         self.close()
+
+    def set_iq_correction(self, enable: bool) -> None:
+        """Turn the per-block DC and IQ-imbalance correction (include/rt_ddc.h) on or off from the next `run` on."""
+        _engine._check(self._set_iq(self._h, 1 if enable else 0))
+        self.iq_correction = bool(enable)
+
+    def read_iq_correction(self, i: int, block: int):
+        """Test hook: `(m, w)` (complex, from the fp32 values the kernels applied) of input `i` and block `block` of the last
+        `run`, which must have corrected; waits for that run."""
+        out = (ctypes.c_float * 4)()
+        _engine._check(self._read_iq(self._h, int(i), int(block), out))
+        return complex(out[0], out[1]), complex(out[2], out[3])
 
     def reset_input(self, i: int, first_sample: int = 0) -> None:
         """Restart input `i` at the global sample index `first_sample`, with a zero filter history (from the next `run`)."""
@@ -210,9 +234,10 @@ class Channelizer(_WidebandFrontEnd):
 
     def __init__(self, sample_rate: int, block_samples: int, offsets_hz: Sequence[float], decimation: int,
                  taps: Optional[Sequence[float]] = None, sample_format: str = "cu8", n_inputs: int = 1, cuda_device: int = 0,
-                 blocks_per_launch: int = 1):
-        """`taps`: real FIR taps (odd count, at most MAX_TAPS); None: `default_taps(decimation)`.  ValueError for a channel plan
-        the down-converter cannot produce; the CUDA side checks the rest (engine.EngineError)."""
+                 blocks_per_launch: int = 1, iq_correction: bool = False):
+        """`taps`: real FIR taps (odd count, at most MAX_TAPS); None: `default_taps(decimation)`.  `iq_correction`: correct
+        every block's DC and IQ imbalance before the filter (`set_iq_correction`).  ValueError for a channel plan the
+        down-converter cannot produce; the CUDA side checks the rest (engine.EngineError)."""
         fs, D = sample_rate, int(decimation)
         if not 2 <= D <= MAX_DECIMATION:
             raise ValueError(f"decimation = {decimation}: must be in [2, {MAX_DECIMATION}]")
@@ -237,6 +262,7 @@ class Channelizer(_WidebandFrontEnd):
         self.cuda_device = cuda_device
         self._lib = _load()
         self._destroy, self._reset, self._run = self._lib.rt_ddc_destroy, self._lib.rt_ddc_reset_input, self._lib.rt_ddc_run
+        self._set_iq, self._read_iq = self._lib.rt_ddc_set_iq_correction, self._lib.rt_ddc_read_iq_correction
         self._h = ctypes.c_void_p()
         cfg = RtDdcConfig(
             abi_version=RT_DDC_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, n_channels=self.n_channels,
@@ -244,6 +270,8 @@ class Channelizer(_WidebandFrontEnd):
             sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
             phase_inc=self.phase_inc.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)))
         _engine._check(self._lib.rt_ddc_create(ctypes.byref(cfg), ctypes.byref(self._h)))
+        if iq_correction:
+            self.set_iq_correction(True)
 
 
 class FilterBank(_WidebandFrontEnd):
@@ -252,10 +280,11 @@ class FilterBank(_WidebandFrontEnd):
     quantity `Channelizer` computes for `offsets_hz` = `grid_offsets(fs, D)`, at about L / log2(2 D) times less work."""
 
     def __init__(self, sample_rate: int, block_samples: int, decimation: int, taps: Optional[Sequence[float]] = None,
-                 sample_format: str = "cu8", n_inputs: int = 1, cuda_device: int = 0, blocks_per_launch: int = 1):
+                 sample_format: str = "cu8", n_inputs: int = 1, cuda_device: int = 0, blocks_per_launch: int = 1,
+                 iq_correction: bool = False):
         """`decimation` D: a power of two in [FBANK_MIN_DECIMATION, FBANK_MAX_DECIMATION]; `taps`: real FIR taps (odd count,
-        at most 16 D + 1); None: `default_taps(decimation)`.  ValueError for a plan the filter bank cannot produce; the CUDA
-        side checks the rest (engine.EngineError)."""
+        at most 16 D + 1); None: `default_taps(decimation)`; `iq_correction` as for `Channelizer`.  ValueError for a plan the
+        filter bank cannot produce; the CUDA side checks the rest (engine.EngineError)."""
         fs, D = sample_rate, int(decimation)
         if not FBANK_MIN_DECIMATION <= D <= FBANK_MAX_DECIMATION or D & (D - 1):
             raise ValueError(f"decimation = {decimation}: must be a power of two in [{FBANK_MIN_DECIMATION}, {FBANK_MAX_DECIMATION}]")
@@ -276,12 +305,15 @@ class FilterBank(_WidebandFrontEnd):
         self.cuda_device = cuda_device
         self._lib = _load()
         self._destroy, self._reset, self._run = self._lib.rt_fbank_destroy, self._lib.rt_fbank_reset_input, self._lib.rt_fbank_run
+        self._set_iq, self._read_iq = self._lib.rt_fbank_set_iq_correction, self._lib.rt_fbank_read_iq_correction
         self._h = ctypes.c_void_p()
         cfg = RtFbankConfig(
             abi_version=RT_FBANK_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, decimation=D,
             block_samples=self.block_samples, n_taps=len(h), sample_format=self._format_code, reserved=0,
             sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)))
         _engine._check(self._lib.rt_fbank_create(ctypes.byref(cfg), ctypes.byref(self._h)))
+        if iq_correction:
+            self.set_iq_correction(True)
 
 
 class WidebandAnalyzer:
@@ -300,11 +332,13 @@ class WidebandAnalyzer:
                  offsets_hz: Sequence[float], decimation: int, fft_nperseg: int, fft_window, signal_min_duration_ms: float,
                  signal_max_duration_ms: float, signal_threshold_dbw: float, snr_threshold_db: float,
                  sdr_callback_length: Optional[int] = None, taps: Optional[Sequence[float]] = None, sample_format: str = "cu8",
-                 cuda_device: int = 0, blocks_per_launch: int = 1, **batch_options):
-        """`batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, ...)."""
+                 cuda_device: int = 0, blocks_per_launch: int = 1, iq_correction: bool = False, **batch_options):
+        """`iq_correction`: correct every wideband block's DC and IQ imbalance before the channel filter (`Channelizer`).
+        `batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, ...)."""
         block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
         front = Channelizer(sample_rate, block, offsets_hz, int(decimation), taps=taps, sample_format=sample_format,
-                            n_inputs=len(self.devices), cuda_device=cuda_device, blocks_per_launch=blocks_per_launch)
+                            n_inputs=len(self.devices), cuda_device=cuda_device, blocks_per_launch=blocks_per_launch,
+                            iq_correction=iq_correction)
         self._attach(front, center_freq, fft_nperseg, fft_window, signal_min_duration_ms, signal_max_duration_ms,
                      signal_threshold_dbw, snr_threshold_db, cuda_device, batch_options)
 
@@ -313,11 +347,12 @@ class WidebandAnalyzer:
                   fft_nperseg: int, fft_window, signal_min_duration_ms: float, signal_max_duration_ms: float,
                   signal_threshold_dbw: float, snr_threshold_db: float, sdr_callback_length: Optional[int] = None,
                   taps: Optional[Sequence[float]] = None, sample_format: str = "cu8", cuda_device: int = 0,
-                  blocks_per_launch: int = 1, **batch_options) -> "WidebandAnalyzer":
+                  blocks_per_launch: int = 1, iq_correction: bool = False, **batch_options) -> "WidebandAnalyzer":
         """The whole band of every input: a `FilterBank` in front, so channel c (0 ... 2 D - 2) of input i is the device
         `f"{devices[i]}:{c}"` at `center_freq + (c - D + 1) fs / (2 D)`.  Adjacent channels overlap by half their width, so
         every frequency within fs / 2 - fs / (4 D) of the centre lies in the flat central half of some channel.  ValueError
-        when the 2 D - 1 channels of every input and block exceed the engine's 65535 analyzer units per launch."""
+        when the 2 D - 1 channels of every input and block exceed the engine's 65535 analyzer units per launch.
+        `iq_correction` as in the constructor."""
         self = cls.__new__(cls)
         block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
         D = int(decimation)
@@ -326,7 +361,7 @@ class WidebandAnalyzer:
             raise ValueError(f"{len(self.devices)} inputs * {2 * D - 1} channels * {blocks_per_launch} blocks per launch = {units} "
                              f"analyzer units: more than the engine's {MAX_ENGINE_UNITS}")
         front = FilterBank(sample_rate, block, D, taps=taps, sample_format=sample_format, n_inputs=len(self.devices),
-                           cuda_device=cuda_device, blocks_per_launch=blocks_per_launch)
+                           cuda_device=cuda_device, blocks_per_launch=blocks_per_launch, iq_correction=iq_correction)
         self._attach(front, center_freq, fft_nperseg, fft_window, signal_min_duration_ms, signal_max_duration_ms,
                      signal_threshold_dbw, snr_threshold_db, cuda_device, batch_options)
         return self
