@@ -219,6 +219,25 @@ int rt_engine_read_spectrogram(rt_engine *e, int32_t stream, float *out_T_by_npe
 int rt_engine_read_row_means(rt_engine *e, int32_t stream, float *out_nperseg);
 
 /*
+ * Band survey: what the band looked like in each analyzed block, for choosing signal_threshold_dbw and calibration_db and for
+ * spotting interferers.  Off by default; with it off no survey work is enqueued.  For analyzer unit u of a launch with T columns,
+ * bin fi in FFT order, the launch's power cells S[fi, t] and its row means avg = mean_t S[fi, :] (the record's row_mean),
+ * thr[u] = rt_config.signal_threshold of u's stream and snr = rt_config.snr_threshold, exactly as the scan uses them:
+ *     noise[u][fi]      = avg                                                   (linear)
+ *     peak[u][fi]       = max_t S[fi, t]                                        (linear)
+ *     above_cols[u][fi] = #{ t < T : !(S[fi,t] < thr[u]) && !(S[fi,t] / avg < snr) }
+ * all over the current block's columns only (no carry).  above_cols uses the scan's fp32 predicate (predicate.h), so it agrees
+ * with what the detection saw.  On RT_FFT_TC256 the power scale the kernels carry is undone (a power of two: exact).  The values
+ * are the same bits run after run, and for a unit alone or inside a batch.  Cost: one more read of the spectrogram per launch,
+ * on the scan stream after the extraction kernel; the peek and fetch of a surveyed launch wait for it.
+ */
+/* Survey the launches from the next one on (enable != 0) or stop. */
+int rt_engine_set_survey(rt_engine *e, int32_t enable);
+/* The survey of the last fetched launch, each [units][nperseg] (units = n_streams * blocks_per_launch; bins in FFT order); a
+ * null pointer skips that array.  RT_ERR_INVALID when that launch did not survey. */
+int rt_engine_read_survey(rt_engine *e, float *noise, float *peak, int32_t *above_cols);
+
+/*
  * Parity hook (tests only, no GPU needed): the constant operands of the RT_FFT_TC256 kernel for a 256-point window
  * (as scipy returns it): the 16 stage-1 matrices as two fp16 terms in the tensor-core operand layout
  * (bmat_out: 16 * 2 * 1024 halves, element (n, k) of matrix (n2, hi|lo) at ((n2*2 + hl)*1024 + (n>>3)*256 + (k>>3)*64 + (n&7)*8 + (k&7)),

@@ -26,6 +26,7 @@ import numpy as np
 
 from . import engine as _engine
 from .messages import from_dB, message_types
+from .survey import BandSurvey, unit_surveys
 
 try:
     from . import _rtfinal                  # csrc/rt_pyfinal.c: the Signal-object builder of the finaliser
@@ -179,10 +180,11 @@ class BatchAnalyzer:
                  signal_threshold_dbw: float, snr_threshold_db: float, sdr_callback_length: Optional[int] = None,
                  cuda_device: int = 0, max_records: int = 0, fft_impl: int = _engine.FFT_AUTO,
                  scan_schedule: int = _engine.SCAN_AUTO, launch_streams: int = 0, chunk_segs: int = 0,
-                 blocks_per_launch: int = 1, sample_format: str = "cu8"):
+                 blocks_per_launch: int = 1, sample_format: str = "cu8", survey: bool = False):
         """`sample_format`: the SigMF datatype of the input blocks, one of `engine.SAMPLE_FORMATS` (cu8: RTL-SDR bytes, ci8, ci16_le,
         cf32_le); the thresholds apply to the normalised samples (INTEGRATION.md).  `center_freq`: one value for every device, or
-        one per device (the channels of a wideband recording, wideband.py); a Signal's frequency is `freqs[fi] + center_freq`."""
+        one per device (the channels of a wideband recording, wideband.py); a Signal's frequency is `freqs[fi] + center_freq`.
+        `survey`: survey the band in every launch (`last_survey`)."""
         if sample_format not in _engine.SAMPLE_FORMATS:
             raise ValueError(f"sample_format = {sample_format!r}: the B200 engine reads {', '.join(_engine.SAMPLE_FORMATS)} (see INTEGRATION.md)")
         self.sample_format = sample_format
@@ -218,6 +220,7 @@ class BatchAnalyzer:
         self.max_records = max_records
         self.fft_impl = fft_impl
         self.scan_schedule, self.launch_streams, self.chunk_segs = scan_schedule, launch_streams, chunk_segs
+        self.survey = bool(survey)
         self.timings = {"fetch_wait_s": 0.0, "finalize_s": 0.0, "build_s": 0.0, "collects": 0}   # host-side split of collect()
         self._engine: Optional[_engine.Engine] = None
         self.last_record_count = 0          # candidate records copied back by the last collect()
@@ -239,6 +242,8 @@ class BatchAnalyzer:
                 max_records=self.max_records, cuda_device=self.cuda_device, fft_impl=self.fft_impl,
                 scan_schedule=self.scan_schedule, launch_streams=self.launch_streams, chunk_segs=self.chunk_segs,
                 blocks_per_launch=self.blocks_per_launch, sample_format=self.sample_format)
+            if self.survey:
+                self._engine.set_survey(True)
         return self._engine
 
     def close(self):
@@ -378,6 +383,15 @@ class BatchAnalyzer:
         tm["build_s"] += time.perf_counter() - t2
         tm["collects"] += 1
         return out
+
+    def last_survey(self) -> List[BandSurvey]:
+        """The band survey of the last collected launch (the analyzer needs `survey=True`): one `BandSurvey` per analyzer unit,
+        stream-major and block-minor like `collect`."""
+        noise, peak, above = self.engine.read_survey()
+        s = np.arange(self.n_units) // self.blocks_per_launch
+        cf = self.center_freq if self._center_freqs is None else self._center_freqs[s]
+        return unit_surveys([self.devices[i] for i in s], self.plan.freqs, np.broadcast_to(cf, s.shape),
+                            np.asarray(self.calibration_db)[s], noise, peak, above, self.plan.T)
 
     def process_blocks(self, iq, ts_start: Sequence[datetime.datetime]):
         """`iq`: `[n_streams, 2*block_samples]` (`[n_streams, blocks_per_launch, 2*block_samples]`) interleaved I,Q elements of

@@ -625,6 +625,64 @@ __global__ void __launch_bounds__(128, MINB) extract2_kernel(ScanArgs a) {
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// band survey (rt_engine_set_survey): per unit and bin, the row mean, the peak and the columns that pass the scan's predicate
+// ---------------------------------------------------------------------------------------------
+// Its own argument struct: the scan kernels' ScanArgs stays as it is, so they compile to the same code with the survey off.
+struct SurveyArgs {
+    const float* S;        // current block, in the engine's layout
+    size_t stream_stride;  // floats per unit
+    const float* avg;      // [unit][n] row means of this launch (complete once the probe kernel has run)
+    const float* thr;      // [unit]
+    float snr;
+    int n, T;
+    float* noise;          // [unit][n] <- avg (the CTAs of column chunk 0)
+    unsigned* peak;        // [unit][n] <- max_t S as a bit pattern (zeroed before): powers are >= 0, so atomicMax on the bits
+                           //              is the float maximum, whatever order the chunks arrive in
+    int* above;            // [unit][n] <- columns that pass the predicate (zeroed before; integer sums: order-free)
+};
+
+constexpr int SURVEY_COLS = 128;     // columns per thread: 74 chunks x 64 units x 256 bins = 1.2 M threads at configs[1]
+constexpr int SURVEY_BATCH = 8;      // cells of a thread in flight together
+
+// row position -> bin for the survey: as pos_to_bin, except that on TILE consecutive threads take consecutive floats of a time
+// step (16-byte quads of 4 bins, 512 bytes apart), as the PERM positions do
+template <int L>
+__device__ __forceinline__ int survey_bin(int idx) {
+    return L == LAYOUT_TILE ? (idx >> 4) + 16 * (idx & 3) + 64 * ((idx >> 2) & 3) : pos_to_bin<L>(idx);
+}
+
+// One thread per (unit, bin, chunk of SURVEY_COLS columns); min(n, 256) row positions of one unit per CTA.
+template <int L>
+__global__ void __launch_bounds__(256) survey_kernel(SurveyArgs a) {
+    const int nbb = (a.n + blockDim.x - 1) / blockDim.x;           // bin blocks
+    const int bb = blockIdx.x % nbb, chunk = blockIdx.x / nbb;
+    const int idx = bb * blockDim.x + threadIdx.x;
+    const int s = blockIdx.y;
+    if (idx >= a.n) return;
+    const int fi = survey_bin<L>(idx);
+    const size_t cell = (size_t)s * a.n + fi;
+    const float avg = a.avg[cell];
+    if (chunk == 0) a.noise[cell] = avg;
+    const Pred pred(a.thr[s], avg, a.snr);           // bit for bit the probe's above() (predicate.h)
+    const CellRef col = CellRef::make<L>(a.S, a.stream_stride, s, fi, a.n);
+    const int t0 = chunk * SURVEY_COLS, t1 = min(a.T, t0 + SURVEY_COLS);
+    float mx = 0.f;
+    int cnt = 0;
+    for (int tb = t0; tb < t1; tb += SURVEY_BATCH) {
+        float c[SURVEY_BATCH];
+#pragma unroll
+        for (int i = 0; i < SURVEY_BATCH; ++i) c[i] = (tb + i < t1) ? col.at<L>(tb + i) : -1.f;      // -1: no such column
+#pragma unroll
+        for (int i = 0; i < SURVEY_BATCH; ++i) {
+            mx = fmaxf(mx, c[i]);
+            cnt += (c[i] >= 0.f && pred(c[i])) ? 1 : 0;
+        }
+    }
+    atomicMax(&a.peak[cell], __float_as_uint(mx));
+    if (cnt) atomicAdd(&a.above[cell], cnt);
+}
+
 // PERM / TILE -> [T][n] for the parity hook, with the power scale of the tensor-core path undone (a power of two: exact)
 template <int L>
 __global__ void untile_kernel(const float* S, float* out, int total, int n, float inv_scale) {
@@ -720,6 +778,12 @@ struct rt_engine {
     float* d_tmp = nullptr;         // parity hook scratch
     bool launched = false;
     int last_work_items = 0, last_records = 0;   // counters of the last fetched launch
+    // band survey (rt_engine_set_survey): [noise | peak bits | above columns], each [unit][n], per result slot
+    bool survey = false;                         // survey the launches from the next one on
+    bool surveyed[RT_SLOTS] = {false, false};    // the launch in this slot surveyed
+    bool last_surveyed = false;                  // the last fetched launch surveyed: h_survey holds it
+    uint32_t* d_survey[RT_SLOTS] = {nullptr, nullptr};
+    uint32_t* h_survey = nullptr;                // pinned, allocated by the first fetch of a survey
     // timing
     struct EvSet { cudaEvent_t ev[6]; };   // launch stream: before / after spectrogram; scan stream: start, row mean, probe, extract
     std::vector<EvSet> ev_pool;
@@ -764,7 +828,8 @@ void free_engine(rt_engine* e) {
         for (auto& ev : s.ev) cudaEventDestroy(ev);
     cudaFree(e->d_win); cudaFree(e->d_tw); cudaFree(e->d_tw1);
     for (auto& p : e->d_S) cudaFree(p);
-    for (int k = 0; k < RT_SLOTS; ++k) { cudaFree(e->d_part[k]); cudaFree(e->d_avg[k]); cudaFree(e->d_ctr[k]); cudaFree(e->d_rec[k]); }
+    for (int k = 0; k < RT_SLOTS; ++k) { cudaFree(e->d_part[k]); cudaFree(e->d_avg[k]); cudaFree(e->d_ctr[k]); cudaFree(e->d_rec[k]); cudaFree(e->d_survey[k]); }
+    if (e->h_survey) cudaFreeHost(e->h_survey);
     cudaFree(e->d_bmat); cudaFree(e->d_thr); cudaFree(e->d_hasprev);
     cudaFree(e->d_stage[0]); cudaFree(e->d_stage[1]); cudaFree(e->d_work); cudaFree(e->d_counters); cudaFree(e->d_tmp);
     for (int k = 0; k < 2; ++k) { if (e->h2d_done[k]) cudaEventDestroy(e->h2d_done[k]); if (e->stage_free[k]) cudaEventDestroy(e->stage_free[k]); }
@@ -973,6 +1038,31 @@ int select_scan(rt_engine* e) {
         case LAYOUT_TILE: return use_scan_layout<LAYOUT_TILE>(e);
         default: return use_scan_layout<LAYOUT_LINEAR>(e);
     }
+}
+
+size_t survey_words(const rt_engine* e) { return (size_t)3 * e->n_units * e->n; }
+
+// The band survey of one launch into d_survey[slot], on the scan stream behind the probe and extraction kernels (the row means are
+// complete there under every schedule) and in front of done[slot], which orders the next writer of this S buffer and of
+// d_survey[slot] after it.  So the fetch of a surveyed launch, which waits for done[slot], also waits for its survey, and the next
+// launch's scan kernels queue behind it on the scan stream.
+int launch_survey(const rt_engine* e, const float* S, int slot, cudaStream_t st) {
+    const size_t cells = (size_t)e->n_units * e->n;
+    uint32_t* buf = e->d_survey[slot];
+    CU(cudaMemsetAsync(buf + cells, 0, 2 * cells * sizeof(uint32_t), st));
+    SurveyArgs a;
+    a.S = S; a.stream_stride = e->s_stride; a.avg = e->d_avg[slot]; a.thr = e->d_thr; a.snr = (float)e->cfg.snr_threshold;
+    a.n = e->n; a.T = e->T;
+    a.noise = reinterpret_cast<float*>(buf); a.peak = buf + cells; a.above = reinterpret_cast<int*>(buf + 2 * cells);
+    const int bins = std::min(e->n, 256);
+    const dim3 grid(((e->n + bins - 1) / bins) * ((e->T + SURVEY_COLS - 1) / SURVEY_COLS), e->n_units);
+    switch (e->layout) {
+        case LAYOUT_PERM: survey_kernel<LAYOUT_PERM><<<grid, bins, 0, st>>>(a); break;
+        case LAYOUT_TILE: survey_kernel<LAYOUT_TILE><<<grid, bins, 0, st>>>(a); break;
+        default: survey_kernel<LAYOUT_LINEAR><<<grid, bins, 0, st>>>(a);
+    }
+    CU(cudaGetLastError());
+    return RT_OK;
 }
 
 }  // namespace
@@ -1310,6 +1400,12 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
     int rc = e->scan(e, sc, sc_st, evs ? evs->ev[4] : nullptr);
     if (rc != RT_OK) return rc;
     if (evs) CU(cudaEventRecord(evs->ev[5], sc_st));
+    e->surveyed[slot] = false;
+    if (e->survey) {
+        rc = launch_survey(e, e->d_S[next], slot, sc_st);
+        if (rc != RT_OK) return rc;
+        e->surveyed[slot] = true;
+    }
 
     CU(cudaEventRecord(e->done[slot], sc_st));
     e->launch_seq++;
@@ -1318,7 +1414,7 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         if (!h) { h = 1; e->hasprev_dirty = true; }
     e->launched = true;
     e->acc.launches += 1;
-    e->acc.kernels += e->sep_mean ? 4 : 3;
+    e->acc.kernels += (e->sep_mean ? 4 : 3) + (e->survey ? 1 : 0);
     return RT_OK;
 }
 
@@ -1345,6 +1441,13 @@ int rt_engine_fetch(rt_engine* e, rt_record* out, int32_t max_out, int32_t* n_ou
     e->last_work_items = e->h_counters[0];
     e->last_records = nrec;
     *n_out = nrec;
+    // the survey and the records come back on the copy stream, which waited for done[slot] in peek_oldest; one synchronize for both
+    const bool surveyed = e->surveyed[slot];
+    e->last_surveyed = false;
+    if (surveyed) {
+        if (!e->h_survey) CU(cudaMallocHost(&e->h_survey, survey_words(e) * sizeof(uint32_t)));
+        CU(cudaMemcpyAsync(e->h_survey, e->d_survey[slot], survey_words(e) * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->copy_stream));
+    }
     const int have = std::max(0, std::min(nrec, std::min(e->max_records, out ? max_out : 0)));
     if (have > 0) {
         if ((size_t)have > e->h_rec_cap) {
@@ -1354,7 +1457,10 @@ int rt_engine_fetch(rt_engine* e, rt_record* out, int32_t max_out, int32_t* n_ou
             CU(cudaMallocHost(&e->h_rec, e->h_rec_cap * sizeof(rt_record)));
         }
         CU(cudaMemcpyAsync(e->h_rec, e->d_rec[slot], (size_t)have * sizeof(rt_record), cudaMemcpyDeviceToHost, e->copy_stream));
-        CU(cudaStreamSynchronize(e->copy_stream));
+    }
+    if (surveyed || have > 0) CU(cudaStreamSynchronize(e->copy_stream));
+    e->last_surveyed = surveyed;
+    if (have > 0) {
         std::sort(e->h_rec, e->h_rec + have, [](const rt_record& x, const rt_record& y) {
             if (x.stream != y.stream) return x.stream < y.stream;
             if (x.fi != y.fi) return x.fi < y.fi;
@@ -1442,6 +1548,31 @@ int rt_engine_read_row_means(rt_engine* e, int32_t stream, float* out) {
     CU(cudaStreamSynchronize(e->stream));
     if (e->pscale != 1.f)
         for (int i = 0; i < e->n; ++i) out[i] *= 1.f / e->pscale;
+    return RT_OK;
+}
+
+int rt_engine_set_survey(rt_engine* e, int32_t enable) {
+    if (!e) return fail(RT_ERR_INVALID, "null engine");
+    if (enable) {
+        CU(cudaSetDevice(e->dev));
+        for (auto& p : e->d_survey)              // every slot: a failed allocation leaves the rest to the next call
+            if (!p) CU(cudaMalloc(&p, survey_words(e) * sizeof(uint32_t)));
+    }
+    e->survey = enable != 0;
+    return RT_OK;
+}
+
+int rt_engine_read_survey(rt_engine* e, float* noise, float* peak, int32_t* above_cols) {
+    if (!e) return fail(RT_ERR_INVALID, "null engine");
+    if (!e->last_surveyed) return fail(RT_ERR_INVALID, "the last fetched launch did not survey (rt_engine_set_survey)");
+    const size_t cells = (size_t)e->n_units * e->n;
+    const float inv = 1.f / e->pscale;                  // power of two: exact
+    const float* h_noise = reinterpret_cast<const float*>(e->h_survey);
+    for (size_t i = 0; i < cells; ++i) {
+        if (noise) noise[i] = h_noise[i] * inv;
+        if (peak) { float p; std::memcpy(&p, &e->h_survey[cells + i], sizeof(float)); peak[i] = p * inv; }
+    }
+    if (above_cols) std::memcpy(above_cols, e->h_survey + 2 * cells, cells * sizeof(int32_t));
     return RT_OK;
 }
 

@@ -50,6 +50,7 @@ EXPORTS = (
     "rt_engine_set_stream", "rt_engine_reset_stream", "rt_engine_process", "rt_engine_launch", "rt_engine_fetch", "rt_engine_peek",
     "rt_engine_shape", "rt_engine_read_spectrogram", "rt_engine_read_row_means", "rt_engine_enable_timing",
     "rt_engine_get_timing", "rt_engine_join", "rt_engine_wait_stream", "rt_engine_last_counts", "rt_tc256_tables",
+    "rt_engine_set_survey", "rt_engine_read_survey",
     # include/rt_matcher.h
     "rt_matcher_create", "rt_matcher_destroy", "rt_matcher_add", "rt_matcher_pending", "rt_matcher_drain",
     "rt_matcher_open", "rt_matcher_read_open",
@@ -124,6 +125,8 @@ def load_library() -> ctypes.CDLL:
     lib.rt_engine_read_row_means.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p]
     lib.rt_engine_enable_timing.argtypes = [ctypes.c_void_p, ctypes.c_int32]
     lib.rt_engine_get_timing.argtypes = [ctypes.c_void_p, ctypes.POINTER(RtTiming), ctypes.c_int32]
+    lib.rt_engine_set_survey.argtypes = [ctypes.c_void_p, ctypes.c_int32]
+    lib.rt_engine_read_survey.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
     if lib.rt_abi_version() != RT_ABI_VERSION:
         raise ImportError(f"{path}: ABI {lib.rt_abi_version()} != {RT_ABI_VERSION}; rebuild (python -m pyradiotracking_b200.build --force)")
     _lib = lib
@@ -338,6 +341,21 @@ class Engine:
         w, r = ctypes.c_int32(0), ctypes.c_int32(0)
         _check(self._lib.rt_engine_last_counts(self._h, ctypes.byref(w), ctypes.byref(r)))
         return w.value, r.value
+
+    def set_survey(self, enable: bool) -> None:
+        """Survey every launch from the next one on (include/rt_engine.h): per unit and bin the row mean, the peak cell and the
+        columns above the detection threshold."""
+        _check(self._lib.rt_engine_set_survey(self._h, 1 if enable else 0))
+
+    def read_survey(self) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """The survey of the last fetched launch: `(noise, peak, above_cols)`, each `[n_units, nperseg]` in FFT order (noise and
+        peak float32, linear; above_cols int32).  EngineError (RT_ERR_INVALID) when that launch did not survey."""
+        noise = np.empty((self.n_units, self.nperseg), dtype=np.float32)
+        peak = np.empty_like(noise)
+        above = np.empty((self.n_units, self.nperseg), dtype=np.int32)
+        _check(self._lib.rt_engine_read_survey(self._h, noise.ctypes.data_as(ctypes.c_void_p), peak.ctypes.data_as(ctypes.c_void_p),
+                                               above.ctypes.data_as(ctypes.c_void_p)))
+        return noise, peak, above
 
     def join(self) -> None:
         """Make the launch stream wait for the scan kernels of every launch so far (they run on an

@@ -34,6 +34,7 @@ import numpy as np
 
 from . import engine as _engine
 from .analyze import BatchAnalyzer
+from .survey import stitch
 
 RT_DDC_ABI_VERSION = 1
 MAX_TAPS = 2049           # RT_DDC_MAX_TAPS
@@ -334,7 +335,8 @@ class WidebandAnalyzer:
                  sdr_callback_length: Optional[int] = None, taps: Optional[Sequence[float]] = None, sample_format: str = "cu8",
                  cuda_device: int = 0, blocks_per_launch: int = 1, iq_correction: bool = False, **batch_options):
         """`iq_correction`: correct every wideband block's DC and IQ imbalance before the channel filter (`Channelizer`).
-        `batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, ...)."""
+        `batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, survey, ...); with
+        `survey=True` every channel is surveyed (`last_survey`)."""
         block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
         front = Channelizer(sample_rate, block, offsets_hz, int(decimation), taps=taps, sample_format=sample_format,
                             n_inputs=len(self.devices), cuda_device=cuda_device, blocks_per_launch=blocks_per_launch,
@@ -352,7 +354,7 @@ class WidebandAnalyzer:
         `f"{devices[i]}:{c}"` at `center_freq + (c - D + 1) fs / (2 D)`.  Adjacent channels overlap by half their width, so
         every frequency within fs / 2 - fs / (4 D) of the centre lies in the flat central half of some channel.  ValueError
         when the 2 D - 1 channels of every input and block exceed the engine's 65535 analyzer units per launch.
-        `iq_correction` as in the constructor."""
+        `iq_correction` and `batch_options` as in the constructor; with `survey=True`, `band_survey` stitches the channels."""
         self = cls.__new__(cls)
         block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
         D = int(decimation)
@@ -437,6 +439,23 @@ class WidebandAnalyzer:
                 per = [res[(i * C + c) * B + b] for c in range(C)]
                 out.append(per if with_all else ([s for p in per for s in p[0]], sum(p[1] for p in per)))
         return out
+
+    def last_survey(self) -> list:
+        """The band survey of the last collected launch (built with `survey=True`): per input unit (input-major, block-minor,
+        like `collect`) the list of its channels' `BandSurvey`s in channel order."""
+        C, B = self.n_channels, self.blocks_per_launch
+        res = self.channels.last_survey()
+        return [[res[(i * C + c) * B + b] for c in range(C)] for i in range(self.n_streams) for b in range(B)]
+
+    def band_survey(self) -> list:
+        """`full_band` only: per input unit (input-major, block-minor) one `BandSurvey` of the whole band, stitched from the flat
+        central halves of its channels (`survey.stitch`): a uniform grid of spacing fs / (D nperseg) from
+        center_freq - (fs / 2 - fs / (4 D)) up to, not including, center_freq + fs / 2 - fs / (4 D), with the frequencies of the
+        channels' Signals.  ValueError for an analyzer on arbitrary channel offsets, whose channels may overlap or leave gaps."""
+        if not isinstance(self.ddc, FilterBank):
+            raise ValueError("band_survey needs the uniform channel grid of full_band; last_survey gives the channels of this plan")
+        B = self.blocks_per_launch
+        return [stitch(self.devices[u // B], chans) for u, chans in enumerate(self.last_survey())]
 
     def process_blocks(self, iq, ts_start: Sequence[datetime.datetime]):
         self.submit(iq)
