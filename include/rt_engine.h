@@ -238,6 +238,32 @@ int rt_engine_set_survey(rt_engine *e, int32_t enable);
 int rt_engine_read_survey(rt_engine *e, float *noise, float *peak, int32_t *above_cols);
 
 /*
+ * Neighbour bins: what a carrier estimate finer than one FFT bin needs (pyradiotracking_b200/finefreq.py).  Off by default; with
+ * it off nothing is enqueued.  For a record (stream = unit u, fi, start, end) of a launch with T columns and n = nperseg, its
+ * cells in bin b are exactly those the record's mean_lin averages in bin fi:
+ *     start >= 0:  S_u[b][start .. end-1]
+ *     start <  0:  prev_u[b][T+start .. T-1]  and  S_u[b][0 .. end-1]
+ * where prev_u is unit u - 1 of the same launch, or for u % blocks_per_launch == 0 the last block of u's stream in the previous
+ * launch (the extraction's carry).  With lo = (fi - 1) mod n and hi = (fi + 1) mod n:
+ *     mean_lo / mean_hi         = the mean of those end - start cells in bin lo / hi (float64 sum of the fp32 cells)
+ *     row_mean_lo / row_mean_hi = the current block's row means avg[u][lo] / avg[u][hi] (as rt_record.row_mean)
+ * On RT_FFT_TC256 the power scale is undone (a power of two: exact).  The values are the same bits run after run, and for a unit
+ * alone or inside a batch.  Cost: 2 (end - start) scattered cells per record, one kernel on the scan stream after the
+ * extraction kernel (and the survey); the peek and fetch of such a launch wait for it.
+ */
+typedef struct rt_neighbours {
+    double mean_lo, mean_hi;
+    float row_mean_lo, row_mean_hi;
+} rt_neighbours;    /* 24 bytes */
+/* Compute them for the launches from the next one on (enable != 0) or stop; allocates max_records entries for every result slot
+ * that lacks them. */
+int rt_engine_set_neighbours(rt_engine *e, int32_t enable);
+/* Entry i belongs to record i of the last rt_engine_fetch, in its order; *n_out = the records that fetch returned (also after an
+ * RT_ERR_OVERFLOW fetch).  RT_ERR_INVALID when that launch did not compute them; RT_ERR_OVERFLOW when max_out < *n_out (the first
+ * max_out are written). */
+int rt_engine_read_neighbours(rt_engine *e, rt_neighbours *out, int32_t max_out, int32_t *n_out);
+
+/*
  * Parity hook (tests only, no GPU needed): the constant operands of the RT_FFT_TC256 kernel for a 256-point window
  * (as scipy returns it): the 16 stage-1 matrices as two fp16 terms in the tensor-core operand layout
  * (bmat_out: 16 * 2 * 1024 halves, element (n, k) of matrix (n2, hi|lo) at ((n2*2 + hl)*1024 + (n>>3)*256 + (k>>3)*64 + (n&7)*8 + (k&7)),

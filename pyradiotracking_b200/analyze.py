@@ -26,6 +26,7 @@ import numpy as np
 
 from . import engine as _engine
 from .messages import from_dB, message_types
+from .finefreq import FineFrequency, fine_frequencies
 from .survey import BandSurvey, unit_surveys
 
 try:
@@ -116,6 +117,7 @@ class Finalized(NamedTuple):
     noise: np.ndarray
     snr: np.ndarray
     shadow: np.ndarray          # True: dropped by filter_shadow_signals
+    fine_frequency: Optional[np.ndarray] = None     # with neighbour bins: the carrier estimate of each row (finefreq.py)
 
 
 def shadow_mask(ts_us: np.ndarray, dur_us: np.ndarray, max_dbw: np.ndarray) -> np.ndarray:
@@ -180,11 +182,12 @@ class BatchAnalyzer:
                  signal_threshold_dbw: float, snr_threshold_db: float, sdr_callback_length: Optional[int] = None,
                  cuda_device: int = 0, max_records: int = 0, fft_impl: int = _engine.FFT_AUTO,
                  scan_schedule: int = _engine.SCAN_AUTO, launch_streams: int = 0, chunk_segs: int = 0,
-                 blocks_per_launch: int = 1, sample_format: str = "cu8", survey: bool = False):
+                 blocks_per_launch: int = 1, sample_format: str = "cu8", survey: bool = False, fine_frequency: bool = False):
         """`sample_format`: the SigMF datatype of the input blocks, one of `engine.SAMPLE_FORMATS` (cu8: RTL-SDR bytes, ci8, ci16_le,
         cf32_le); the thresholds apply to the normalised samples (INTEGRATION.md).  `center_freq`: one value for every device, or
         one per device (the channels of a wideband recording, wideband.py); a Signal's frequency is `freqs[fi] + center_freq`.
-        `survey`: survey the band in every launch (`last_survey`)."""
+        `survey`: survey the band in every launch (`last_survey`).  `fine_frequency`: estimate every Signal's carrier to a
+        fraction of a bin (`last_fine_frequencies`); ValueError for a window whose response does not allow it (finefreq.py)."""
         if sample_format not in _engine.SAMPLE_FORMATS:
             raise ValueError(f"sample_format = {sample_format!r}: the B200 engine reads {', '.join(_engine.SAMPLE_FORMATS)} (see INTEGRATION.md)")
         self.sample_format = sample_format
@@ -221,6 +224,8 @@ class BatchAnalyzer:
         self.fft_impl = fft_impl
         self.scan_schedule, self.launch_streams, self.chunk_segs = scan_schedule, launch_streams, chunk_segs
         self.survey = bool(survey)
+        self.fine = FineFrequency(self.window) if fine_frequency else None
+        self._last_fine = None              # (stream, fi, shadow, fine_frequency) of the rows the last collect finalised
         self.timings = {"fetch_wait_s": 0.0, "finalize_s": 0.0, "build_s": 0.0, "collects": 0}   # host-side split of collect()
         self._engine: Optional[_engine.Engine] = None
         self.last_record_count = 0          # candidate records copied back by the last collect()
@@ -244,6 +249,8 @@ class BatchAnalyzer:
                 blocks_per_launch=self.blocks_per_launch, sample_format=self.sample_format)
             if self.survey:
                 self._engine.set_survey(True)
+            if self.fine is not None:
+                self._engine.set_neighbours(True)
         return self._engine
 
     def close(self):
@@ -256,10 +263,12 @@ class BatchAnalyzer:
         self.engine.reset_stream(stream)
 
     # -- finaliser: records -> Signal objects ----------------------------------------------------
-    def finalize_arrays(self, records: np.ndarray) -> "Finalized":
+    def finalize_arrays(self, records: np.ndarray, neighbours: Optional[np.ndarray] = None) -> "Finalized":
         """Vectorised analyze.py:419-450 for the candidate records of one engine call (sorted by stream, bin,
         start): exact float64 duration test, timestamps / durations rounded to microseconds exactly like
-        `datetime.timedelta(seconds=float)`, dB statistics, and the per-stream shadow mask (analyze.py:283-328)."""
+        `datetime.timedelta(seconds=float)`, dB statistics, and the per-stream shadow mask (analyze.py:283-328).
+        `neighbours` (`Engine.read_neighbours`, aligned with `records`; the analyzer needs `fine_frequency=True`): the rows
+        also get their carrier estimates."""
         plan = self.plan
         times = plan.times
         start = records["start"].astype(np.int64)
@@ -282,6 +291,8 @@ class BatchAnalyzer:
                 max=10 * np.log10(r["max_lin"].astype(np.float64)) - cal, avg=10 * np.log10(mean) - cal,
                 std=r["std_db"].astype(np.float64), noise=10 * np.log10(row), snr=10 * np.log10(mean / row),
                 shadow=np.zeros(len(r), dtype=bool))
+        if neighbours is not None:
+            fin = fin._replace(fine_frequency=fine_frequencies(self.fine, fin.frequency, fin.fi, neighbours[ok], self.sample_rate))
         # shadow filter per analyzer unit (signals of one callback share ts_start, so offsets are enough): one pass over the
         # whole batch, the units shifted so far apart in time that they cannot overlap
         if len(r) > 1:
@@ -358,9 +369,12 @@ class BatchAnalyzer:
         `process_blocks`.  `ts_start`: one per stream, the start of the first block of the launch."""
         t0 = time.perf_counter()
         records = self.engine.fetch()
+        neighbours = self.engine.read_neighbours() if self.fine is not None else None
         t1 = time.perf_counter()
         self.last_record_count = len(records)
-        fin = self.finalize_arrays(records)
+        fin = self.finalize_arrays(records, neighbours)
+        if self.fine is not None:
+            self._last_fine = (fin.stream, fin.fi, fin.shadow, fin.fine_frequency)
         t2 = time.perf_counter()
         if not with_all:
             kept = self.build_signals(fin, ts_start, ~fin.shadow)
@@ -392,6 +406,22 @@ class BatchAnalyzer:
         cf = self.center_freq if self._center_freqs is None else self._center_freqs[s]
         return unit_surveys([self.devices[i] for i in s], self.plan.freqs, np.broadcast_to(cf, s.shape),
                             np.asarray(self.calibration_db)[s], noise, peak, above, self.plan.T)
+
+    def last_fine_frequencies(self, all_signals: bool = False) -> List[np.ndarray]:
+        """The carrier estimates of the last collected launch (the analyzer needs `fine_frequency=True`): one float64 array
+        per analyzer unit, stream-major and block-minor like `collect`, element for element aligned with the unit's
+        shadow-filtered Signals, or with `all_signals` with the `all_signals` / `keys` of `collect(with_all=True)`.  Hz like
+        `Signal.frequency`; NaN where there is no estimate (finefreq.py).  `Signal.frequency` itself stays the bin centre."""
+        return [f for f, _ in self._fine_units(all_signals)]
+
+    def _fine_units(self, all_signals: bool) -> List[Tuple[np.ndarray, np.ndarray]]:
+        """Per analyzer unit `(fine frequencies, bins fi)` of the rows `last_fine_frequencies` returns."""
+        if self._last_fine is None:
+            raise ValueError("no fine frequencies: build the analyzer with fine_frequency=True and collect a launch")
+        stream, fi, shadow, fine = self._last_fine
+        keep = np.ones(len(stream), dtype=bool) if all_signals else ~shadow
+        cuts = np.cumsum(np.bincount(stream[keep], minlength=self.n_units))[:-1]
+        return list(zip(np.split(fine[keep], cuts), np.split(fi[keep], cuts)))
 
     def process_blocks(self, iq, ts_start: Sequence[datetime.datetime]):
         """`iq`: `[n_streams, 2*block_samples]` (`[n_streams, blocks_per_launch, 2*block_samples]`) interleaved I,Q elements of

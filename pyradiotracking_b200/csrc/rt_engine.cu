@@ -683,6 +683,66 @@ __global__ void __launch_bounds__(256) survey_kernel(SurveyArgs a) {
     if (cnt) atomicAdd(&a.above[cell], cnt);
 }
 
+// ---------------------------------------------------------------------------------------------
+// neighbour bins (rt_engine_set_neighbours): per record, the mean of bins fi - 1 and fi + 1 over the record's own cells
+// ---------------------------------------------------------------------------------------------
+// Its own argument struct, like SurveyArgs: ScanArgs stays as it is.
+struct NeighbourArgs {
+    const float* S;          // current block, in the engine's layout
+    const float* Sprev;      // previous block (the carry of the first unit of every stream)
+    size_t stream_stride;    // floats per unit
+    const float* avg;        // [unit][n] row means of this launch
+    const rt_record* rec;    // this launch's records, in the order the extraction kernel wrote them
+    const int* counters;     // [1]: records emitted (may exceed max_records)
+    int max_records;
+    int bpl, n, T;
+    rt_neighbours* out;      // [max_records], entry i for rec[i]
+};
+
+constexpr int NEIGHBOUR_CTAS = 296;       // 2 per SM of a B200; the warps grid-stride over the device-side record count
+
+// One warp per record.  Lane l accumulates in double the carried columns T + start + l, + 32, ... and then the current columns
+// max(start, 0) + l, + 32, ...; warp_sum's xor-butterfly adds the lanes.  That order depends only on the record, so every launch,
+// batch and schedule returns the same bits.  The cells are exactly those extract2_kernel averaged into mean_lin, with its carry
+// rule (the previous unit of the same launch, or the last unit of the stream in the previous launch's buffer).
+template <int L>
+__global__ void __launch_bounds__(256) neighbour_kernel(NeighbourArgs a) {
+    const int lane = threadIdx.x & 31;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int n_warps = (gridDim.x * blockDim.x) >> 5;
+    const int n_rec = min(a.counters[1], a.max_records);
+    const int n = a.n, T = a.T;
+    for (int i = warp; i < n_rec; i += n_warps) {
+        const rt_record r = a.rec[i];
+        const int s = r.stream, lo = (r.fi + n - 1) % n, hi = (r.fi + 1) % n;
+        double slo = 0.0, shi = 0.0;
+        if (r.start < 0) {
+            const bool own = a.bpl == 1 || (s % a.bpl) == 0;
+            const float* P = own ? a.Sprev : a.S;
+            const int ps = own ? s + a.bpl - 1 : s - 1;
+            const CellRef plo = CellRef::make<L>(P, a.stream_stride, ps, lo, n), phi = CellRef::make<L>(P, a.stream_stride, ps, hi, n);
+            for (int t = T + r.start + lane; t < T; t += 32) {
+                slo += (double)plo.at<L>(t);
+                shi += (double)phi.at<L>(t);
+            }
+        }
+        const CellRef clo = CellRef::make<L>(a.S, a.stream_stride, s, lo, n), chi = CellRef::make<L>(a.S, a.stream_stride, s, hi, n);
+        for (int t = max(r.start, 0) + lane; t < r.end; t += 32) {
+            slo += (double)clo.at<L>(t);
+            shi += (double)chi.at<L>(t);
+        }
+        slo = warp_sum(slo);
+        shi = warp_sum(shi);
+        if (lane == 0) {
+            const int cnt = r.end - r.start;
+            rt_neighbours o;
+            o.mean_lo = slo / cnt; o.mean_hi = shi / cnt;
+            o.row_mean_lo = a.avg[(size_t)s * n + lo]; o.row_mean_hi = a.avg[(size_t)s * n + hi];
+            a.out[i] = o;
+        }
+    }
+}
+
 // PERM / TILE -> [T][n] for the parity hook, with the power scale of the tensor-core path undone (a power of two: exact)
 template <int L>
 __global__ void untile_kernel(const float* S, float* out, int total, int n, float inv_scale) {
@@ -784,6 +844,14 @@ struct rt_engine {
     bool last_surveyed = false;                  // the last fetched launch surveyed: h_survey holds it
     uint32_t* d_survey[RT_SLOTS] = {nullptr, nullptr};
     uint32_t* h_survey = nullptr;                // pinned, allocated by the first fetch of a survey
+    // neighbour bins (rt_engine_set_neighbours): one rt_neighbours per record, per result slot
+    bool neighbours = false;                     // compute them for the launches from the next one on
+    bool refined[RT_SLOTS] = {false, false};     // the launch in this slot computed them
+    bool last_refined = false;                   // the last fetched launch computed them: h_nb_sorted holds them
+    rt_neighbours* d_nb[RT_SLOTS] = {nullptr, nullptr};
+    rt_neighbours* h_nb = nullptr;               // pinned, grown on demand like h_rec
+    size_t h_nb_cap = 0;
+    std::vector<rt_neighbours> h_nb_sorted;      // entry i for record i of the last fetch, power scale undone
     // timing
     struct EvSet { cudaEvent_t ev[6]; };   // launch stream: before / after spectrogram; scan stream: start, row mean, probe, extract
     std::vector<EvSet> ev_pool;
@@ -828,8 +896,9 @@ void free_engine(rt_engine* e) {
         for (auto& ev : s.ev) cudaEventDestroy(ev);
     cudaFree(e->d_win); cudaFree(e->d_tw); cudaFree(e->d_tw1);
     for (auto& p : e->d_S) cudaFree(p);
-    for (int k = 0; k < RT_SLOTS; ++k) { cudaFree(e->d_part[k]); cudaFree(e->d_avg[k]); cudaFree(e->d_ctr[k]); cudaFree(e->d_rec[k]); cudaFree(e->d_survey[k]); }
+    for (int k = 0; k < RT_SLOTS; ++k) { cudaFree(e->d_part[k]); cudaFree(e->d_avg[k]); cudaFree(e->d_ctr[k]); cudaFree(e->d_rec[k]); cudaFree(e->d_survey[k]); cudaFree(e->d_nb[k]); }
     if (e->h_survey) cudaFreeHost(e->h_survey);
+    if (e->h_nb) cudaFreeHost(e->h_nb);
     cudaFree(e->d_bmat); cudaFree(e->d_thr); cudaFree(e->d_hasprev);
     cudaFree(e->d_stage[0]); cudaFree(e->d_stage[1]); cudaFree(e->d_work); cudaFree(e->d_counters); cudaFree(e->d_tmp);
     for (int k = 0; k < 2; ++k) { if (e->h2d_done[k]) cudaEventDestroy(e->h2d_done[k]); if (e->stage_free[k]) cudaEventDestroy(e->stage_free[k]); }
@@ -1060,6 +1129,24 @@ int launch_survey(const rt_engine* e, const float* S, int slot, cudaStream_t st)
         case LAYOUT_PERM: survey_kernel<LAYOUT_PERM><<<grid, bins, 0, st>>>(a); break;
         case LAYOUT_TILE: survey_kernel<LAYOUT_TILE><<<grid, bins, 0, st>>>(a); break;
         default: survey_kernel<LAYOUT_LINEAR><<<grid, bins, 0, st>>>(a);
+    }
+    CU(cudaGetLastError());
+    return RT_OK;
+}
+
+// The neighbour bins of one launch's records into d_nb[slot], on the scan stream behind the extraction kernel (and the survey) and in
+// front of done[slot], which orders the next writer of S[next], of the carry buffer, of d_rec[slot] and of d_nb[slot] after it.
+// The record count stays on the device: the grid is fixed and the warps stride over it.
+int launch_neighbours(const rt_engine* e, const float* S, const float* Sprev, int slot, const int* d_cnt, cudaStream_t st) {
+    NeighbourArgs a;
+    a.S = S; a.Sprev = Sprev; a.stream_stride = e->s_stride; a.avg = e->d_avg[slot];
+    a.rec = e->d_rec[slot]; a.counters = d_cnt; a.max_records = e->max_records;
+    a.bpl = e->bpl; a.n = e->n; a.T = e->T;
+    a.out = e->d_nb[slot];
+    switch (e->layout) {
+        case LAYOUT_PERM: neighbour_kernel<LAYOUT_PERM><<<NEIGHBOUR_CTAS, 256, 0, st>>>(a); break;
+        case LAYOUT_TILE: neighbour_kernel<LAYOUT_TILE><<<NEIGHBOUR_CTAS, 256, 0, st>>>(a); break;
+        default: neighbour_kernel<LAYOUT_LINEAR><<<NEIGHBOUR_CTAS, 256, 0, st>>>(a);
     }
     CU(cudaGetLastError());
     return RT_OK;
@@ -1406,6 +1493,12 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         if (rc != RT_OK) return rc;
         e->surveyed[slot] = true;
     }
+    e->refined[slot] = false;
+    if (e->neighbours) {
+        rc = launch_neighbours(e, e->d_S[next], e->d_S[e->cur], slot, d_cnt, sc_st);
+        if (rc != RT_OK) return rc;
+        e->refined[slot] = true;
+    }
 
     CU(cudaEventRecord(e->done[slot], sc_st));
     e->launch_seq++;
@@ -1414,7 +1507,7 @@ int rt_engine_launch(rt_engine* e, const uint8_t* iq, int32_t iq_on_device, size
         if (!h) { h = 1; e->hasprev_dirty = true; }
     e->launched = true;
     e->acc.launches += 1;
-    e->acc.kernels += (e->sep_mean ? 4 : 3) + (e->survey ? 1 : 0);
+    e->acc.kernels += (e->sep_mean ? 4 : 3) + (e->survey ? 1 : 0) + (e->neighbours ? 1 : 0);
     return RT_OK;
 }
 
@@ -1458,14 +1551,45 @@ int rt_engine_fetch(rt_engine* e, rt_record* out, int32_t max_out, int32_t* n_ou
         }
         CU(cudaMemcpyAsync(e->h_rec, e->d_rec[slot], (size_t)have * sizeof(rt_record), cudaMemcpyDeviceToHost, e->copy_stream));
     }
+    // the neighbour bins of the returned records, next to them
+    const bool refined = e->refined[slot];
+    e->last_refined = false;
+    if (refined && have > 0) {
+        if ((size_t)have > e->h_nb_cap) {
+            if (e->h_nb) CU(cudaFreeHost(e->h_nb));
+            e->h_nb = nullptr;
+            e->h_nb_cap = std::max<size_t>((size_t)have + have / 2, 4096);
+            CU(cudaMallocHost(&e->h_nb, e->h_nb_cap * sizeof(rt_neighbours)));
+        }
+        CU(cudaMemcpyAsync(e->h_nb, e->d_nb[slot], (size_t)have * sizeof(rt_neighbours), cudaMemcpyDeviceToHost, e->copy_stream));
+    }
     if (surveyed || have > 0) CU(cudaStreamSynchronize(e->copy_stream));
     e->last_surveyed = surveyed;
+    const auto rec_less = [](const rt_record& x, const rt_record& y) {
+        if (x.stream != y.stream) return x.stream < y.stream;
+        if (x.fi != y.fi) return x.fi < y.fi;
+        return x.start < y.start;
+    };
+    if (refined) {
+        // records and neighbours through one permutation; the records end up in the order the plain sort gives them ((stream,
+        // fi, start) is unique: two records of one bin and unit are two runs)
+        std::vector<int> perm(have);
+        for (int i = 0; i < have; ++i) perm[i] = i;
+        std::sort(perm.begin(), perm.end(), [&](int i, int j) { return rec_less(e->h_rec[i], e->h_rec[j]); });
+        std::vector<rt_record> rec(e->h_rec, e->h_rec + have);
+        e->h_nb_sorted.resize(have);
+        const double inv = 1.0 / e->pscale;              // power of two: exact
+        for (int i = 0; i < have; ++i) {
+            e->h_rec[i] = rec[perm[i]];
+            rt_neighbours nb = e->h_nb[perm[i]];
+            nb.mean_lo *= inv; nb.mean_hi *= inv;
+            nb.row_mean_lo *= (float)inv; nb.row_mean_hi *= (float)inv;
+            e->h_nb_sorted[i] = nb;
+        }
+        e->last_refined = true;
+    }
     if (have > 0) {
-        std::sort(e->h_rec, e->h_rec + have, [](const rt_record& x, const rt_record& y) {
-            if (x.stream != y.stream) return x.stream < y.stream;
-            if (x.fi != y.fi) return x.fi < y.fi;
-            return x.start < y.start;
-        });
+        if (!refined) std::sort(e->h_rec, e->h_rec + have, rec_less);
         if (e->pscale != 1.f) {
             const float inv = 1.f / e->pscale;           // power of two: exact
             for (int i = 0; i < have; ++i) {
@@ -1573,6 +1697,28 @@ int rt_engine_read_survey(rt_engine* e, float* noise, float* peak, int32_t* abov
         if (peak) { float p; std::memcpy(&p, &e->h_survey[cells + i], sizeof(float)); peak[i] = p * inv; }
     }
     if (above_cols) std::memcpy(above_cols, e->h_survey + 2 * cells, cells * sizeof(int32_t));
+    return RT_OK;
+}
+
+int rt_engine_set_neighbours(rt_engine* e, int32_t enable) {
+    if (!e) return fail(RT_ERR_INVALID, "null engine");
+    if (enable) {
+        CU(cudaSetDevice(e->dev));
+        for (auto& p : e->d_nb)                  // every slot: a failed allocation leaves the rest to the next call
+            if (!p) CU(cudaMalloc(&p, (size_t)e->max_records * sizeof(rt_neighbours)));
+    }
+    e->neighbours = enable != 0;
+    return RT_OK;
+}
+
+int rt_engine_read_neighbours(rt_engine* e, rt_neighbours* out, int32_t max_out, int32_t* n_out) {
+    if (!e || !n_out || (max_out > 0 && !out)) return fail(RT_ERR_INVALID, "null argument");
+    if (!e->last_refined) return fail(RT_ERR_INVALID, "the last fetched launch did not compute neighbour bins (rt_engine_set_neighbours)");
+    const int have = (int)e->h_nb_sorted.size();
+    *n_out = have;
+    const int k = std::max(0, std::min(have, max_out));
+    if (k > 0) std::memcpy(out, e->h_nb_sorted.data(), (size_t)k * sizeof(rt_neighbours));
+    if (have > k) return fail(RT_ERR_OVERFLOW, "output buffer smaller than the number of entries (the first max_out were returned)");
     return RT_OK;
 }
 

@@ -50,7 +50,7 @@ EXPORTS = (
     "rt_engine_set_stream", "rt_engine_reset_stream", "rt_engine_process", "rt_engine_launch", "rt_engine_fetch", "rt_engine_peek",
     "rt_engine_shape", "rt_engine_read_spectrogram", "rt_engine_read_row_means", "rt_engine_enable_timing",
     "rt_engine_get_timing", "rt_engine_join", "rt_engine_wait_stream", "rt_engine_last_counts", "rt_tc256_tables",
-    "rt_engine_set_survey", "rt_engine_read_survey",
+    "rt_engine_set_survey", "rt_engine_read_survey", "rt_engine_set_neighbours", "rt_engine_read_neighbours",
     # include/rt_matcher.h
     "rt_matcher_create", "rt_matcher_destroy", "rt_matcher_add", "rt_matcher_pending", "rt_matcher_drain",
     "rt_matcher_open", "rt_matcher_read_open",
@@ -82,6 +82,10 @@ RECORD_DTYPE = np.dtype([
     ("max_lin", "<f4"), ("row_mean", "<f4"), ("mean_lin", "<f8"), ("std_db", "<f8"),
 ])
 assert RECORD_DTYPE.itemsize == 40
+
+# rt_neighbours, 24 bytes
+NEIGHBOURS_DTYPE = np.dtype([("mean_lo", "<f8"), ("mean_hi", "<f8"), ("row_mean_lo", "<f4"), ("row_mean_hi", "<f4")])
+assert NEIGHBOURS_DTYPE.itemsize == 24
 
 _lib = None
 
@@ -127,6 +131,8 @@ def load_library() -> ctypes.CDLL:
     lib.rt_engine_get_timing.argtypes = [ctypes.c_void_p, ctypes.POINTER(RtTiming), ctypes.c_int32]
     lib.rt_engine_set_survey.argtypes = [ctypes.c_void_p, ctypes.c_int32]
     lib.rt_engine_read_survey.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    lib.rt_engine_set_neighbours.argtypes = [ctypes.c_void_p, ctypes.c_int32]
+    lib.rt_engine_read_neighbours.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]
     if lib.rt_abi_version() != RT_ABI_VERSION:
         raise ImportError(f"{path}: ABI {lib.rt_abi_version()} != {RT_ABI_VERSION}; rebuild (python -m pyradiotracking_b200.build --force)")
     _lib = lib
@@ -248,6 +254,7 @@ class Engine:
         self._held = []
         self._launches = self._fetches = 0    # mirror of the engine's ring: launches made, results fetched or dropped
         self._stream = None                   # the cudaStream_t handle last given to set_stream
+        self._last_fetched = 0                # records the last fetch returned (read_neighbours)
 
     # -- lifetime ---------------------------------------------------------------------------
     def close(self):
@@ -316,6 +323,7 @@ class Engine:
         self.truncated = 0
         if rc in (RT_OK, RT_ERR_OVERFLOW):              # the launch was consumed: release its input and every older one
             self._fetches += 1
+            self._last_fetched = len(out)
             del self._held[:len(self._held) - (self._launches - self._fetches)]
         if rc == RT_ERR_OVERFLOW:
             self.truncated = need.value - n.value
@@ -356,6 +364,19 @@ class Engine:
         _check(self._lib.rt_engine_read_survey(self._h, noise.ctypes.data_as(ctypes.c_void_p), peak.ctypes.data_as(ctypes.c_void_p),
                                                above.ctypes.data_as(ctypes.c_void_p)))
         return noise, peak, above
+
+    def set_neighbours(self, enable: bool) -> None:
+        """Compute the neighbour bins of every record from the next launch on (include/rt_engine.h): the mean of bins fi - 1 and
+        fi + 1 over the record's own cells, and their row means."""
+        _check(self._lib.rt_engine_set_neighbours(self._h, 1 if enable else 0))
+
+    def read_neighbours(self) -> np.ndarray:
+        """`NEIGHBOURS_DTYPE` entries aligned with the records of the last `fetch` (linear powers).  EngineError
+        (RT_ERR_INVALID) when that launch did not compute them."""
+        out = np.empty(self._last_fetched, dtype=NEIGHBOURS_DTYPE)
+        n = ctypes.c_int32(0)
+        _check(self._lib.rt_engine_read_neighbours(self._h, out.ctypes.data_as(ctypes.c_void_p), len(out), ctypes.byref(n)))
+        return out[:n.value]
 
     def join(self) -> None:
         """Make the launch stream wait for the scan kernels of every launch so far (they run on an

@@ -166,14 +166,17 @@ class CaptureReader:
 
 
 def replay(paths: Sequence[str], analyzer, t0: datetime.datetime, on_block: Optional[Callable] = None,
-           max_blocks: Optional[int] = None, pinned: bool = True, on_survey: Optional[Callable] = None) -> int:
+           max_blocks: Optional[int] = None, pinned: bool = True, on_survey: Optional[Callable] = None,
+           on_fine_frequencies: Optional[Callable] = None) -> int:
     """Run every full block of the recordings through `analyzer` (a `BatchAnalyzer` with one stream per file), read in the
     analyzer's `sample_format` (a SigMF metadata file beside a recording must agree with it).
 
     `on_block(block_index, per_stream)` receives what `BatchAnalyzer.collect` returns for that block
     (`per_stream[s] = (shadow-filtered Signals, candidates before the filter)`), in block order -- also when the
     analyzer takes several blocks per launch.  `on_survey(block_index, surveys)` (an analyzer built with `survey=True`) receives
-    what `analyzer.last_survey()` gives for that block, regrouped per block the same way.  Returns the number of blocks processed."""
+    what `analyzer.last_survey()` gives for that block, regrouped per block the same way; `on_fine_frequencies(block_index,
+    per_stream)` (an analyzer built with `fine_frequency=True`) what `analyzer.last_fine_frequencies()` gives, aligned with the
+    filtered Signals `on_block` received.  Returns the number of blocks processed."""
     if analyzer.n_streams != len(paths):
         raise ValueError("one capture file per analyzer stream")
     B = getattr(analyzer, "blocks_per_launch", 1)
@@ -188,11 +191,14 @@ def replay(paths: Sequence[str], analyzer, t0: datetime.datetime, on_block: Opti
         b0 = pending.pop(0)
         res = analyzer.collect([t0 + b0 * dt] * analyzer.n_streams)      # per analyzer unit: stream-major, block-minor
         surveys = analyzer.last_survey() if on_survey is not None else None
+        fine = analyzer.last_fine_frequencies() if on_fine_frequencies is not None else None
         for k in range(min(B, reader.n_blocks - b0)):                     # (the padding blocks of a last group are ignored)
             if on_block is not None:
                 on_block(b0 + k, [res[s * B + k] for s in range(analyzer.n_streams)])
             if on_survey is not None:
                 on_survey(b0 + k, [surveys[s * B + k] for s in range(analyzer.n_streams)])
+            if on_fine_frequencies is not None:
+                on_fine_frequencies(b0 + k, [fine[s * B + k] for s in range(analyzer.n_streams)])
             done += 1
 
     try:

@@ -52,7 +52,7 @@ class MultiStreamAnalyzer:
             fft_nperseg=fft_nperseg, fft_window=fft_window, signal_min_duration_ms=signal_min_duration_ms,
             signal_max_duration_ms=signal_max_duration_ms, signal_threshold_dbw=signal_threshold_dbw,
             snr_threshold_db=snr_threshold_db, sdr_callback_length=self.sdr_callback_length, cuda_device=cuda_device,
-            **{k: v for k, v in kwargs.items() if k in ("fft_impl", "max_records", "survey")})
+            **{k: v for k, v in kwargs.items() if k in ("fft_impl", "max_records", "survey", "fine_frequency")})
         self.Signal, self.StateMessage = message_types()
         self._ts: List[Optional[datetime.datetime]] = [None] * self.n_streams
         self.last_state: List[object] = [None] * self.n_streams

@@ -34,6 +34,7 @@ import numpy as np
 
 from . import engine as _engine
 from .analyze import BatchAnalyzer
+from .finefreq import central_half
 from .survey import stitch
 
 RT_DDC_ABI_VERSION = 1
@@ -335,8 +336,9 @@ class WidebandAnalyzer:
                  sdr_callback_length: Optional[int] = None, taps: Optional[Sequence[float]] = None, sample_format: str = "cu8",
                  cuda_device: int = 0, blocks_per_launch: int = 1, iq_correction: bool = False, **batch_options):
         """`iq_correction`: correct every wideband block's DC and IQ imbalance before the channel filter (`Channelizer`).
-        `batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, survey, ...); with
-        `survey=True` every channel is surveyed (`last_survey`)."""
+        `batch_options`: further `BatchAnalyzer` keys of the channel analyzer (max_records, fft_impl, survey, fine_frequency,
+        ...); with `survey=True` every channel is surveyed (`last_survey`), with `fine_frequency=True` every Signal gets a
+        carrier estimate (`last_fine_frequencies`)."""
         block = self._check_plan(devices, calibration_db, sample_rate, decimation, fft_nperseg, sdr_callback_length)
         front = Channelizer(sample_rate, block, offsets_hz, int(decimation), taps=taps, sample_format=sample_format,
                             n_inputs=len(self.devices), cuda_device=cuda_device, blocks_per_launch=blocks_per_launch,
@@ -446,6 +448,18 @@ class WidebandAnalyzer:
         C, B = self.n_channels, self.blocks_per_launch
         res = self.channels.last_survey()
         return [[res[(i * C + c) * B + b] for c in range(C)] for i in range(self.n_streams) for b in range(B)]
+
+    def last_fine_frequencies(self, all_signals: bool = False) -> list:
+        """The carrier estimates of the last collected launch (built with `fine_frequency=True`): per input unit (input-major,
+        block-minor, like `collect`) one float64 array aligned with the Signals `collect` returned for it, its channels'
+        concatenated in channel order (with `all_signals`: their `all_signals`), computed at the channel rate fs / D.
+        An estimate is kept only where the Signal's bin lies in its channel's flat central half, signed bin k in
+        [-n/4, n/4); elsewhere it is NaN.  On the `full_band` grid those halves tile the band without overlap, so a pulse
+        found in two overlapping channels gets its estimate from exactly one of them -- except within about two bins of a
+        channel centre, where the estimator has none (finefreq.py: the bins next to DC), so such a pulse gets none."""
+        C, B, n = self.n_channels, self.blocks_per_launch, self.channels.fft_nperseg
+        res = [np.where(central_half(fi, n), f, np.nan) for f, fi in self.channels._fine_units(all_signals)]
+        return [np.concatenate([res[(i * C + c) * B + b] for c in range(C)]) for i in range(self.n_streams) for b in range(B)]
 
     def band_survey(self) -> list:
         """`full_band` only: per input unit (input-major, block-minor) one `BandSurvey` of the whole band, stitched from the flat
