@@ -15,8 +15,8 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "librtb200.so")
 PYFINAL_SRC = os.path.join(CSRC, "rt_pyfinal.c")
 PYFINAL = os.path.join(HERE, "_rtfinal.so")
-SOURCES = ["rt_engine.cu", "rt_ddc.cu", "rt_fbank.cu", "rt_matcher.cpp"]
-HEADERS = ["predicate.h", "sample_format.cuh", "fir_history.cuh", "iq_correction.cuh", "fft_cpk.cuh", "spectro256.cuh", "spectro_tc256.cuh", "spectro_r16.cuh", os.path.join("..", "..", "include", "rt_engine.h"),
+SOURCES = ["rt_engine.cu", "rt_ddc.cu", "rt_fbank.cu", "fir_frontend.cu", "rt_matcher.cpp"]
+HEADERS = ["predicate.h", "sample_format.cuh", "fir_frontend.cuh", "fir_history.cuh", "iq_correction.cuh", "fft_cpk.cuh", "spectro256.cuh", "spectro_tc256.cuh", "spectro_r16.cuh", os.path.join("..", "..", "include", "rt_engine.h"),
            os.path.join("..", "..", "include", "rt_matcher.h"), os.path.join("..", "..", "include", "rt_ddc.h"),
            os.path.join("..", "..", "include", "rt_fbank.h")]
 NVCC_FLAGS = [

@@ -1,5 +1,6 @@
-// fir_history.cuh -- what the FIR front ends of librtb200.so (rt_ddc.cu, rt_fbank.cu) share: the per-input history of the last
-// L - 1 normalised samples, its reset in stream order, and the staging copy of a host input.
+// fir_history.cuh -- the device side that the FIR front ends of librtb200.so (rt_ddc.cu, rt_fbank.cu) share: the loader of one
+// normalised sample of a call, which reads the per-input history of the last L - 1 samples for indices before the call, and the
+// kernel that saves that history for the next call.  The history's reset and the rest of the host side are in fir_frontend.cu.
 //
 // The kernels take the front end's own argument struct A, which has these fields:
 //   const unsigned char* iq; size_t in_stride;   input i at iq + i * in_stride
@@ -52,32 +53,6 @@ __global__ void fir_history_kernel(const A a) {
     a.hist_out[(size_t)input * a.hist_len + j] = fir_sample<FMT, IQ>(a, row, hist, rel, iq_span<IQ>(a, input, rel));
 }
 
-// reset_input, applied in stream order at the next run: zero history, and the phase offset of the input
-__global__ void fir_reset_kernel(float2* hist, uint32_t* off, int input, int hist_len, uint32_t off_value) {
-    for (int j = threadIdx.x; j < hist_len; j += blockDim.x) hist[(size_t)input * hist_len + j] = make_float2(0.f, 0.f);
-    if (threadIdx.x == 0) off[input] = off_value;
-}
-
 }  // namespace
-
-// Copy n_in host rows of row_bytes (stride `stride`) into the device staging buffer (*stage, grown when too small, rows 256-byte
-// aligned) on `st`; *src and *stride then describe the staged copy.
-inline cudaError_t fir_stage_host_input(cudaStream_t st, const unsigned char** src, size_t* stride, size_t row_bytes, int n_in,
-                                        unsigned char** stage, size_t* stage_bytes) {
-    const size_t sstride = (row_bytes + 255) & ~(size_t)255;
-    cudaError_t e;
-    if (sstride * n_in > *stage_bytes) {
-        if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
-        if ((e = cudaFree(*stage)) != cudaSuccess) return e;
-        *stage = nullptr;
-        *stage_bytes = 0;
-        if ((e = cudaMalloc(stage, sstride * n_in)) != cudaSuccess) return e;
-        *stage_bytes = sstride * n_in;
-    }
-    if ((e = cudaMemcpy2DAsync(*stage, sstride, *src, *stride, row_bytes, n_in, cudaMemcpyHostToDevice, st)) != cudaSuccess) return e;
-    *src = *stage;
-    *stride = sstride;
-    return cudaSuccess;
-}
 
 }  // namespace rt

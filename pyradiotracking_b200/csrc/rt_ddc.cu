@@ -9,25 +9,19 @@
 //                       the outputs read consecutive samples of one polyphase row, so eight taps of a phase need 15 samples
 //                       and 8 taps (shared loads) for 64 complex products (128 packed fp32x2 FMAs, fft_cpk.cuh)
 //   fir_history_kernel  the last L - 1 normalised samples of every input, for the next call (double-buffered; fir_history.cuh)
-//   fir_reset_kernel    rt_ddc_reset_input, applied in stream order at the next run (fir_history.cuh)
-//   iq_moments_kernel, iq_coef_kernel   with rt_ddc_set_iq_correction on: each block's DC and IQ-imbalance coefficients,
-//                       which the IQ = true instantiations of the two kernels above apply as they decode (iq_correction.cuh)
+// With rt_ddc_set_iq_correction on, the IQ = true instantiations of both apply each block's DC and IQ-imbalance coefficients as
+// they decode (iq_correction.cuh).  The handle, the checks and steps a run shares with the filter bank, the reset kernel and
+// the kernels that form the coefficients are in fir_frontend.cu.
 #include <cuda_runtime.h>
 
-#include <algorithm>
 #include <cmath>
-#include <mutex>
-#include <string>
+#include <memory>
 #include <type_traits>
-#include <utility>
 #include <vector>
 
 #include "../../include/rt_ddc.h"
 #include "fft_cpk.cuh"
-#include "fir_history.cuh"
-#include "sample_format.cuh"
-
-int rt_internal_fail(int code, const char* msg);   // rt_engine.cu: sets the thread-local rt_last_error() text
+#include "fir_frontend.cuh"
 
 namespace {
 
@@ -36,16 +30,8 @@ constexpr int DDC_MR = 8;                           // consecutive outputs per t
 constexpr int DDC_PAD = 8;                          // zero samples in front of every polyphase row (masked tap tails read them)
 constexpr size_t DDC_TAP_BUDGET = 66 * 1024;        // shared memory for the taps of one channel group
 constexpr size_t DDC_SMEM_TARGET = 112 * 1024;      // two CTAs per SM
-constexpr size_t DDC_SMEM_MAX = 227 * 1024;
 
-int fail(int code, const std::string& msg) { return rt_internal_fail(code, msg.c_str()); }
-
-#define DCU(call)                                                                                  \
-    do {                                                                                           \
-        cudaError_t _e = (call);                                                                   \
-        if (_e != cudaSuccess)                                                                     \
-            return fail(RT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_e));          \
-    } while (0)
+using rt::fail;
 
 struct DdcArgs {
     const unsigned char* iq;        // input i at iq + i * in_stride
@@ -155,83 +141,14 @@ __global__ void __launch_bounds__(DDC_THREADS) ddc_kernel(const DdcArgsOf<IQ> a)
     }
 }
 
-template <bool IQ>
-using DdcKernel = void (*)(const DdcArgsOf<IQ>);
-template <bool IQ>
-DdcKernel<IQ> ddc_main(int fmt) {
-    switch (fmt) {
-        case RT_SAMPLE_CU8: return ddc_kernel<RT_SAMPLE_CU8, IQ>;
-        case RT_SAMPLE_CI8: return ddc_kernel<RT_SAMPLE_CI8, IQ>;
-        case RT_SAMPLE_CI16: return ddc_kernel<RT_SAMPLE_CI16, IQ>;
-        default: return ddc_kernel<RT_SAMPLE_CF32, IQ>;
-    }
-}
-template <bool IQ>
-DdcKernel<IQ> ddc_history(int fmt) {
-    switch (fmt) {
-        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, IQ, DdcArgsOf<IQ>>;
-        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, IQ, DdcArgsOf<IQ>>;
-        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, IQ, DdcArgsOf<IQ>>;
-        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, IQ, DdcArgsOf<IQ>>;
-    }
-}
-
-// the filter kernel and the history kernel of one run
-template <bool IQ>
-void ddc_launch(const DdcArgsOf<IQ>& a, int fmt, dim3 grid, size_t smem, int n_in, cudaStream_t st) {
-    ddc_main<IQ>(fmt)<<<grid, DDC_THREADS, smem, st>>>(a);
-    if (a.L > 1) ddc_history<IQ>(fmt)<<<dim3((unsigned)((a.L - 1 + 127) / 128), (unsigned)n_in), 128, 0, st>>>(a);
-}
-
-// the limit belongs to the kernel: only ever raise it (handles with other geometries may exist in this process)
-template <class Kernel>
-int raise_smem_limit(Kernel k, size_t smem) {
-    cudaFuncAttributes fa;
-    cudaError_t ferr = cudaFuncGetAttributes(&fa, k);
-    if (ferr != cudaSuccess)
-        return fail(RT_ERR_CUDA, std::string("kernels not loadable on this device (built for sm_100a only): ") + cudaGetErrorString(ferr));
-    if ((size_t)fa.maxDynamicSharedSizeBytes < smem) DCU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    return RT_OK;
-}
+// ddc_kernel of a format and IQ, given as std::integral_constant values (rt::fir_kernels, rt::fir_launch)
+constexpr auto ddc_main = [](auto fmt, auto iq) { return ddc_kernel<decltype(fmt)::value, decltype(iq)::value>; };
 
 }  // namespace
 
-struct rt_ddc {
-    int dev = 0, fmt = 0, n_in = 0, nch = 0, D = 0, L = 0;
-    long long block = 0;
-    rt::SampleFormatInfo info{};
-    int cw = 1, lg_cw = 0, mt = DDC_MR;
-    size_t smem = 0;
-    float2* d_taps = nullptr;
-    uint32_t* d_inc = nullptr;
-    uint32_t* d_off = nullptr;
-    float2* d_hist[2] = {nullptr, nullptr};
-    int cur = 0;                                        // d_hist[cur] holds the history before the next run
-    uint32_t advance = 0;                               // input samples per input since create, mod 2^32
-    std::vector<std::pair<int, uint32_t>> resets;       // (input, first sample mod 2^32), applied at the next run
-    unsigned char* d_stage = nullptr;
-    size_t stage_bytes = 0;
-    cudaEvent_t done = nullptr;
-    bool ran = false;
-    rt::IqState iq;                                     // rt_ddc_set_iq_correction
+struct rt_ddc : rt::FirFrontEnd {
+    int cw = 1, lg_cw = 0;                              // channels per CTA, its log2
 };
-
-static void free_ddc(rt_ddc* d) {
-    if (!d) return;
-    cudaSetDevice(d->dev);
-    if (d->done) {
-        cudaEventSynchronize(d->done);
-        cudaEventDestroy(d->done);
-    }
-    cudaFree(d->d_taps);
-    cudaFree(d->d_inc);
-    cudaFree(d->d_off);
-    cudaFree(d->d_hist[0]);
-    cudaFree(d->d_hist[1]);
-    cudaFree(d->d_stage);
-    d->iq.release();
-    delete d;
-}
 
 extern "C" {
 
@@ -239,179 +156,66 @@ int rt_ddc_create(const rt_ddc_config* cfg, rt_ddc** out) {
     if (!cfg || !out) return fail(RT_ERR_INVALID, "null argument");
     *out = nullptr;
     if (cfg->abi_version != RT_DDC_ABI_VERSION) return fail(RT_ERR_INVALID, "rt_ddc_config.abi_version mismatch");
-    if (cfg->n_inputs < 1 || cfg->n_inputs > 65535) return fail(RT_ERR_INVALID, "n_inputs must be in [1, 65535]");
+    if (cfg->reserved != 0) return fail(RT_ERR_INVALID, "rt_ddc_config.reserved must be zero");
     if (cfg->n_channels < 1 || (long long)cfg->n_inputs * cfg->n_channels > (1 << 30)) return fail(RT_ERR_INVALID, "n_channels must be >= 1");
     if (cfg->decimation < 2 || cfg->decimation > RT_DDC_MAX_DECIMATION) return fail(RT_ERR_INVALID, "decimation must be in [2, RT_DDC_MAX_DECIMATION]");
-    if (cfg->n_taps < 1 || cfg->n_taps > RT_DDC_MAX_TAPS || cfg->n_taps % 2 == 0) return fail(RT_ERR_INVALID, "n_taps must be odd and in [1, RT_DDC_MAX_TAPS]");
-    if (cfg->block_samples < cfg->decimation || cfg->block_samples % cfg->decimation != 0)
-        return fail(RT_ERR_INVALID, "block_samples must be a positive multiple of decimation");
-    rt::SampleFormatInfo info;
-    if (!rt::sample_format_info(cfg->sample_format, &info)) return fail(RT_ERR_INVALID, "unknown sample_format");
     if (!cfg->taps || !cfg->phase_inc) return fail(RT_ERR_INVALID, "taps / phase_inc missing");
-    if (cfg->reserved != 0) return fail(RT_ERR_INVALID, "rt_ddc_config.reserved must be zero");
-    for (int k = 0; k < cfg->n_taps; ++k)
-        if (!std::isfinite(cfg->taps[k])) return fail(RT_ERR_INVALID, "taps must be finite");
+    const rt::FirPlan p{cfg->cuda_device, cfg->sample_format, cfg->n_inputs, cfg->n_channels, cfg->decimation, cfg->n_taps,
+                        cfg->block_samples, cfg->taps};
+    int rc = rt::fir_check(p, RT_DDC_MAX_TAPS, "RT_DDC_MAX_TAPS");
+    if (rc != RT_OK) return rc;
 
     // geometry: CW channels per CTA (a power of two <= 16 whose taps fit DDC_TAP_BUDGET), MT outputs per CTA (every thread group
     // busy unless the span would not fit two CTAs per SM)
-    const int D = cfg->decimation, L = cfg->n_taps;
+    const int D = p.D, L = p.L;
     int cw = 1, lg = 0;
-    while (cw < 16 && cw < cfg->n_channels && (size_t)(2 * cw) * L * sizeof(float2) <= DDC_TAP_BUDGET) { cw <<= 1; ++lg; }
+    while (cw < 16 && cw < p.nch && (size_t)(2 * cw) * L * sizeof(float2) <= DDC_TAP_BUDGET) { cw <<= 1; ++lg; }
     int mt = (DDC_THREADS / cw) * DDC_MR;
     while (mt > DDC_MR && ddc_smem(cw, mt, D, L) > DDC_SMEM_TARGET) mt -= DDC_MR;
-    const size_t smem = ddc_smem(cw, mt, D, L);
-    if (smem > DDC_SMEM_MAX) return fail(RT_ERR_INVALID, "decimation and n_taps need more shared memory than a CTA has");
-
-    int ndev = 0;
-    DCU(cudaGetDeviceCount(&ndev));
-    if (cfg->cuda_device < 0 || cfg->cuda_device >= ndev) return fail(RT_ERR_CUDA, "no such CUDA device (this engine has no CPU fallback)");
-    DCU(cudaSetDevice(cfg->cuda_device));
-    {
-        static std::mutex mu;
-        std::lock_guard<std::mutex> lock(mu);
-        int rc = raise_smem_limit(ddc_main<false>(cfg->sample_format), smem);
-        if (rc == RT_OK) rc = raise_smem_limit(ddc_main<true>(cfg->sample_format), smem);
-        if (rc != RT_OK) return rc;
-    }
-
-    rt_ddc* d = new rt_ddc();
-    d->dev = cfg->cuda_device;
-    d->fmt = cfg->sample_format;
-    d->n_in = cfg->n_inputs;
-    d->nch = cfg->n_channels;
-    d->D = D;
-    d->L = L;
-    d->block = cfg->block_samples;
-    d->info = info;
-    d->cw = cw;
-    d->lg_cw = lg;
-    d->mt = mt;
-    d->smem = smem;
 
     // g_c[k] = h[k] exp(+2 pi i ((inc_c k) mod 2^32) / 2^32), in float64, rounded once
-    std::vector<float2> g((size_t)d->nch * L);
-    for (int c = 0; c < d->nch; ++c)
+    std::vector<float2> g((size_t)p.nch * L);
+    for (int c = 0; c < p.nch; ++c)
         for (int k = 0; k < L; ++k) {
             const uint32_t ph = cfg->phase_inc[c] * (uint32_t)k;
             const double ang = 2.0 * M_PI * (double)ph / 4294967296.0;
             g[(size_t)c * L + k] = make_float2((float)(cfg->taps[k] * std::cos(ang)), (float)(cfg->taps[k] * std::sin(ang)));
         }
-    const size_t hist_bytes = (size_t)d->n_in * std::max(1, L - 1) * sizeof(float2);
-#define DCUE(call)                                                                                 \
-    do {                                                                                           \
-        cudaError_t _e = (call);                                                                   \
-        if (_e != cudaSuccess) {                                                                   \
-            free_ddc(d);                                                                           \
-            return fail(RT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_e));          \
-        }                                                                                          \
-    } while (0)
-    DCUE(cudaMalloc(&d->d_taps, g.size() * sizeof(float2)));
-    DCUE(cudaMalloc(&d->d_inc, d->nch * sizeof(uint32_t)));
-    DCUE(cudaMalloc(&d->d_off, d->n_in * sizeof(uint32_t)));
-    DCUE(cudaMalloc(&d->d_hist[0], hist_bytes));
-    DCUE(cudaMalloc(&d->d_hist[1], hist_bytes));
-    DCUE(cudaMemcpy(d->d_taps, g.data(), g.size() * sizeof(float2), cudaMemcpyHostToDevice));
-    DCUE(cudaMemcpy(d->d_inc, cfg->phase_inc, d->nch * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    DCUE(cudaMemset(d->d_off, 0, d->n_in * sizeof(uint32_t)));
-    DCUE(cudaMemset(d->d_hist[0], 0, hist_bytes));
-    DCUE(cudaEventCreateWithFlags(&d->done, cudaEventDisableTiming));
-#undef DCUE
-    *out = d;
-    return RT_OK;
+    std::unique_ptr<rt_ddc> d(new rt_ddc());
+    d->cw = cw;
+    d->lg_cw = lg;
+    rc = rt::fir_open(d.get(), p, mt, ddc_smem(cw, mt, D, L), rt::fir_kernels(ddc_main, p.fmt),
+                      {{g.data(), g.size() * sizeof(float2)}, {cfg->phase_inc, (size_t)p.nch * sizeof(uint32_t)}});
+    if (rc == RT_OK) *out = d.release();
+    return rc;
 }
 
-void rt_ddc_destroy(rt_ddc* d) { free_ddc(d); }
+void rt_ddc_destroy(rt_ddc* d) { delete d; }
 
-int rt_ddc_reset_input(rt_ddc* d, int32_t input, int64_t first_sample) {
-    if (!d || input < 0 || input >= d->n_in) return fail(RT_ERR_INVALID, "bad input index");
-    d->resets.emplace_back(input, (uint32_t)(uint64_t)first_sample);
-    return RT_OK;
-}
+int rt_ddc_reset_input(rt_ddc* d, int32_t input, int64_t first_sample) { return rt::fir_reset_input(d, input, first_sample); }
 
 int rt_ddc_run(rt_ddc* d, void* cuda_stream, const void* iq, int32_t iq_on_device, size_t in_stride_bytes, int32_t blocks,
                void* out, size_t out_stride_bytes) {
-    if (!d || !iq || !out) return fail(RT_ERR_INVALID, "null argument");
-    if (blocks < 1) return fail(RT_ERR_INVALID, "blocks must be >= 1");
-    const long long n = d->block * blocks;
-    const long long m_total = n / d->D;
-    const size_t row_bytes = (size_t)d->info.bytes * (size_t)n;
-    if (d->n_in > 1 && in_stride_bytes < row_bytes) return fail(RT_ERR_INVALID, "in_stride_bytes smaller than one input's blocks");
-    if (out_stride_bytes < (size_t)m_total * sizeof(float2) && (long long)d->n_in * d->nch > 1)
-        return fail(RT_ERR_INVALID, "out_stride_bytes smaller than one channel's outputs");
-    if (((uintptr_t)out | out_stride_bytes) % sizeof(float2) != 0) return fail(RT_ERR_INVALID, "output pointer / stride not aligned to 8 bytes");
-    if ((m_total + d->mt - 1) / d->mt > 0x7fffffffLL) return fail(RT_ERR_INVALID, "call too long");
-    DCU(cudaSetDevice(d->dev));
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    if (d->ran) DCU(cudaStreamWaitEvent(st, d->done, 0));      // history, offsets and the staging buffer of the previous run
-
-    const unsigned char* src = static_cast<const unsigned char*>(iq);
-    size_t stride = d->n_in > 1 ? in_stride_bytes : row_bytes;
-    if (!iq_on_device) {
-        DCU(rt::fir_stage_host_input(st, &src, &stride, row_bytes, d->n_in, &d->d_stage, &d->stage_bytes));
-    } else if (((uintptr_t)src | (d->n_in > 1 ? stride : 0)) % (uintptr_t)d->info.bytes != 0) {
-        return fail(RT_ERR_INVALID, "IQ pointer / input stride not aligned to one complex sample");
-    }
-
-    rt::IqCorrArgs corr;
-    DCU(rt::iq_prepare(d->iq, st, d->done, d->ran, d->fmt, d->info, src, stride, d->n_in, d->block, blocks, &corr));
-    for (const auto& r : d->resets)
-        rt::fir_reset_kernel<<<1, 256, 0, st>>>(d->d_hist[d->cur], d->d_off, r.first, d->L - 1, r.second - d->advance);
-
+    rt::FirRun r;
+    const int rc = rt::fir_run_begin(d, cuda_stream, iq, iq_on_device, in_stride_bytes, blocks, out, out_stride_bytes, &r);
+    if (rc != RT_OK) return rc;
     DdcArgs a;
-    a.iq = src;
-    a.in_stride = stride;
-    a.hist = d->d_hist[d->cur];
-    a.hist_out = d->d_hist[d->cur ^ 1];
-    a.hist_len = d->L - 1;
-    a.taps = d->d_taps;
-    a.inc = d->d_inc;
-    a.off = d->d_off;
-    a.advance = d->advance;
-    a.out = static_cast<float2*>(out);
-    a.out_stride = out_stride_bytes;
-    a.n_samples = n;
-    a.m_total = m_total;
-    a.D = d->D;
-    a.L = d->L;
+    rt::fir_args(a, *d, r);
+    a.taps = static_cast<const float2*>(d->tables[0]);
+    a.inc = static_cast<const uint32_t*>(d->tables[1]);
     a.n_channels = d->nch;
     a.cw = d->cw;
     a.lg_cw = d->lg_cw;
-    a.mt = d->mt;
     a.rows = ddc_rows(d->mt, d->D, d->L);
-    a.scale = (float)(1.0 / d->info.full_scale);
-    a.offset = (float)d->info.offset;
-    const dim3 grid((unsigned)((m_total + d->mt - 1) / d->mt), (unsigned)((d->nch + d->cw - 1) / d->cw), (unsigned)d->n_in);
-    if (d->iq.applied) {
-        DdcArgsIq ai;
-        static_cast<DdcArgs&>(ai) = a;
-        ai.corr = corr;
-        ddc_launch<true>(ai, d->fmt, grid, d->smem, d->n_in, st);
-    } else {
-        ddc_launch<false>(a, d->fmt, grid, d->smem, d->n_in, st);
-    }
-    DCU(cudaGetLastError());
-    DCU(cudaEventRecord(d->done, st));
-    d->ran = true;
-    d->resets.clear();
-    d->cur ^= d->L > 1 ? 1 : 0;
-    d->advance += (uint32_t)(uint64_t)n;
-    return RT_OK;
+    const dim3 grid((unsigned)((r.m_total + d->mt - 1) / d->mt), (unsigned)((d->nch + d->cw - 1) / d->cw), (unsigned)d->n_in);
+    rt::fir_launch<DdcArgsIq>(*d, r, a, ddc_main, grid, DDC_THREADS);
+    return rt::fir_run_end(d, r);
 }
 
-int rt_ddc_set_iq_correction(rt_ddc* d, int32_t enable) {
-    if (!d) return fail(RT_ERR_INVALID, "null handle");
-    if (enable && d->block > rt::IQ_MAX_BLOCK) return fail(RT_ERR_INVALID, "block_samples must be <= 2^30 for the IQ correction");
-    d->iq.on = enable != 0;
-    return RT_OK;
-}
+int rt_ddc_set_iq_correction(rt_ddc* d, int32_t enable) { return rt::fir_set_iq_correction(d, enable); }
 
 int rt_ddc_read_iq_correction(rt_ddc* d, int32_t input, int32_t block, float out[4]) {
-    if (!d || !out) return fail(RT_ERR_INVALID, "null argument");
-    if (!d->iq.applied) return fail(RT_ERR_INVALID, "the last run did not apply the IQ correction");
-    if (input < 0 || input >= d->n_in || block < 0 || block >= d->iq.blocks) return fail(RT_ERR_INVALID, "bad input / block index");
-    DCU(cudaSetDevice(d->dev));
-    DCU(rt::iq_read(d->iq, d->done, input, block, out));
-    return RT_OK;
+    return rt::fir_read_iq_correction(d, input, block, out);
 }
 
 }  // extern "C"

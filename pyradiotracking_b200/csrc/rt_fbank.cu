@@ -9,40 +9,26 @@
 //                       memory and stores each channel row's MT outputs contiguously (the frames are padded to C + 1 points,
 //                       so reading one bin across frames is free of bank conflicts)
 //   fir_history_kernel  the last L - 1 normalised samples of every input, for the next call (double-buffered; fir_history.cuh)
-//   fir_reset_kernel    rt_fbank_reset_input, applied in stream order at the next run (fir_history.cuh)
-//   iq_moments_kernel, iq_coef_kernel   with rt_fbank_set_iq_correction on: each block's DC and IQ-imbalance coefficients,
-//                       which the IQ = true instantiations of the two kernels above apply as they decode (iq_correction.cuh)
+// With rt_fbank_set_iq_correction on, the IQ = true instantiations of both apply each block's DC and IQ-imbalance coefficients
+// as they decode (iq_correction.cuh).  The handle, the checks and steps a run shares with the down-converter, the reset kernel
+// and the kernels that form the coefficients are in fir_frontend.cu.
 #include <cuda_runtime.h>
 
-#include <algorithm>
 #include <cmath>
-#include <mutex>
-#include <string>
+#include <memory>
 #include <type_traits>
-#include <utility>
 #include <vector>
 
 #include "../../include/rt_fbank.h"
-#include "fir_history.cuh"
-#include "sample_format.cuh"
-
-int rt_internal_fail(int code, const char* msg);   // rt_engine.cu: sets the thread-local rt_last_error() text
+#include "fir_frontend.cuh"
 
 namespace {
 
 constexpr int FB_THREADS = 256;
 constexpr int FB_MAX_MT = 64;                       // output frames per CTA: 512-byte row segments at most
 constexpr size_t FB_SMEM_TARGET = 112 * 1024;       // two CTAs per SM
-constexpr size_t FB_SMEM_MAX = 227 * 1024;
 
-int fail(int code, const std::string& msg) { return rt_internal_fail(code, msg.c_str()); }
-
-#define FCU(call)                                                                                  \
-    do {                                                                                           \
-        cudaError_t _e = (call);                                                                   \
-        if (_e != cudaSuccess)                                                                     \
-            return fail(RT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_e));          \
-    } while (0)
+using rt::fail;
 
 struct FbankArgs {
     const unsigned char* iq;        // input i at iq + i * in_stride
@@ -142,83 +128,14 @@ __global__ void __launch_bounds__(FB_THREADS) fbank_kernel(const FbankArgsOf<IQ>
     }
 }
 
-template <bool IQ>
-using FbankKernel = void (*)(const FbankArgsOf<IQ>);
-template <bool IQ>
-FbankKernel<IQ> fbank_main(int fmt) {
-    switch (fmt) {
-        case RT_SAMPLE_CU8: return fbank_kernel<RT_SAMPLE_CU8, IQ>;
-        case RT_SAMPLE_CI8: return fbank_kernel<RT_SAMPLE_CI8, IQ>;
-        case RT_SAMPLE_CI16: return fbank_kernel<RT_SAMPLE_CI16, IQ>;
-        default: return fbank_kernel<RT_SAMPLE_CF32, IQ>;
-    }
-}
-template <bool IQ>
-FbankKernel<IQ> fbank_history(int fmt) {
-    switch (fmt) {
-        case RT_SAMPLE_CU8: return rt::fir_history_kernel<RT_SAMPLE_CU8, IQ, FbankArgsOf<IQ>>;
-        case RT_SAMPLE_CI8: return rt::fir_history_kernel<RT_SAMPLE_CI8, IQ, FbankArgsOf<IQ>>;
-        case RT_SAMPLE_CI16: return rt::fir_history_kernel<RT_SAMPLE_CI16, IQ, FbankArgsOf<IQ>>;
-        default: return rt::fir_history_kernel<RT_SAMPLE_CF32, IQ, FbankArgsOf<IQ>>;
-    }
-}
-
-// the filter kernel and the history kernel of one run
-template <bool IQ>
-void fbank_launch(const FbankArgsOf<IQ>& a, int fmt, dim3 grid, size_t smem, int n_in, cudaStream_t st) {
-    fbank_main<IQ>(fmt)<<<grid, FB_THREADS, smem, st>>>(a);
-    if (a.L > 1) fbank_history<IQ>(fmt)<<<dim3((unsigned)((a.L - 1 + 127) / 128), (unsigned)n_in), 128, 0, st>>>(a);
-}
-
-// the limit belongs to the kernel: only ever raise it (handles with other geometries may exist in this process)
-template <class Kernel>
-int raise_smem_limit(Kernel k, size_t smem) {
-    cudaFuncAttributes fa;
-    cudaError_t ferr = cudaFuncGetAttributes(&fa, k);
-    if (ferr != cudaSuccess)
-        return fail(RT_ERR_CUDA, std::string("kernels not loadable on this device (built for sm_100a only): ") + cudaGetErrorString(ferr));
-    if ((size_t)fa.maxDynamicSharedSizeBytes < smem) FCU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    return RT_OK;
-}
+// fbank_kernel of a format and IQ, given as std::integral_constant values (rt::fir_kernels, rt::fir_launch)
+constexpr auto fbank_main = [](auto fmt, auto iq) { return fbank_kernel<decltype(fmt)::value, decltype(iq)::value>; };
 
 }  // namespace
 
-struct rt_fbank {
-    int dev = 0, fmt = 0, n_in = 0, D = 0, L = 0, lg_c = 0;
-    long long block = 0;
-    rt::SampleFormatInfo info{};
-    int mt = 1;
-    size_t smem = 0;
-    float* d_taps = nullptr;
-    float2* d_twiddle = nullptr;
-    uint32_t* d_off = nullptr;
-    float2* d_hist[2] = {nullptr, nullptr};
-    int cur = 0;                                        // d_hist[cur] holds the history before the next run
-    uint32_t advance = 0;                               // input samples per input since create, mod 2^32
-    std::vector<std::pair<int, uint32_t>> resets;       // (input, first sample mod 2^32), applied at the next run
-    unsigned char* d_stage = nullptr;
-    size_t stage_bytes = 0;
-    cudaEvent_t done = nullptr;
-    bool ran = false;
-    rt::IqState iq;                                     // rt_fbank_set_iq_correction
+struct rt_fbank : rt::FirFrontEnd {
+    int lg_c = 0;                                       // log2 of the FFT length C = 2 D
 };
-
-static void free_fbank(rt_fbank* f) {
-    if (!f) return;
-    cudaSetDevice(f->dev);
-    if (f->done) {
-        cudaEventSynchronize(f->done);
-        cudaEventDestroy(f->done);
-    }
-    cudaFree(f->d_taps);
-    cudaFree(f->d_twiddle);
-    cudaFree(f->d_off);
-    cudaFree(f->d_hist[0]);
-    cudaFree(f->d_hist[1]);
-    cudaFree(f->d_stage);
-    f->iq.release();
-    delete f;
-}
 
 extern "C" {
 
@@ -227,51 +144,18 @@ int rt_fbank_create(const rt_fbank_config* cfg, rt_fbank** out) {
     *out = nullptr;
     if (cfg->abi_version != RT_FBANK_ABI_VERSION) return fail(RT_ERR_INVALID, "rt_fbank_config.abi_version mismatch");
     if (cfg->reserved != 0) return fail(RT_ERR_INVALID, "rt_fbank_config.reserved must be zero");
-    if (cfg->n_inputs < 1 || cfg->n_inputs > 65535) return fail(RT_ERR_INVALID, "n_inputs must be in [1, 65535]");
     const int D = cfg->decimation;
     if (D < RT_FBANK_MIN_DECIMATION || D > RT_FBANK_MAX_DECIMATION || (D & (D - 1)) != 0)
         return fail(RT_ERR_INVALID, "decimation must be a power of two in [RT_FBANK_MIN_DECIMATION, RT_FBANK_MAX_DECIMATION]");
     if ((long long)cfg->n_inputs * (2 * D - 1) > (1 << 30)) return fail(RT_ERR_INVALID, "n_inputs * (2 decimation - 1) must be <= 2^30");
-    if (cfg->n_taps < 1 || cfg->n_taps > RT_FBANK_MAX_TAPS(D) || cfg->n_taps % 2 == 0)
-        return fail(RT_ERR_INVALID, "n_taps must be odd and in [1, 16 decimation + 1]");
-    if (cfg->block_samples < D || cfg->block_samples % D != 0)
-        return fail(RT_ERR_INVALID, "block_samples must be a positive multiple of decimation");
-    rt::SampleFormatInfo info;
-    if (!rt::sample_format_info(cfg->sample_format, &info)) return fail(RT_ERR_INVALID, "unknown sample_format");
-    if (!cfg->taps) return fail(RT_ERR_INVALID, "taps missing");
-    for (int k = 0; k < cfg->n_taps; ++k)
-        if (!std::isfinite(cfg->taps[k])) return fail(RT_ERR_INVALID, "taps must be finite");
+    const rt::FirPlan p{cfg->cuda_device, cfg->sample_format, cfg->n_inputs, 2 * D - 1, D, cfg->n_taps, cfg->block_samples, cfg->taps};
+    int rc = rt::fir_check(p, RT_FBANK_MAX_TAPS(D), "16 decimation + 1");
+    if (rc != RT_OK) return rc;
 
     // geometry: the largest power-of-two tile of frames whose span and frames fit two CTAs per SM (one frame always fits)
-    const int L = cfg->n_taps;
+    const int L = p.L;
     int mt = FB_MAX_MT;
     while (mt > 1 && fbank_smem(mt, D, L) > FB_SMEM_TARGET) mt >>= 1;
-    const size_t smem = fbank_smem(mt, D, L);
-    if (smem > FB_SMEM_MAX) return fail(RT_ERR_INVALID, "decimation and n_taps need more shared memory than a CTA has");
-
-    int ndev = 0;
-    FCU(cudaGetDeviceCount(&ndev));
-    if (cfg->cuda_device < 0 || cfg->cuda_device >= ndev) return fail(RT_ERR_CUDA, "no such CUDA device (this engine has no CPU fallback)");
-    FCU(cudaSetDevice(cfg->cuda_device));
-    {
-        static std::mutex mu;
-        std::lock_guard<std::mutex> lock(mu);
-        int rc = raise_smem_limit(fbank_main<false>(cfg->sample_format), smem);
-        if (rc == RT_OK) rc = raise_smem_limit(fbank_main<true>(cfg->sample_format), smem);
-        if (rc != RT_OK) return rc;
-    }
-
-    rt_fbank* f = new rt_fbank();
-    f->dev = cfg->cuda_device;
-    f->fmt = cfg->sample_format;
-    f->n_in = cfg->n_inputs;
-    f->D = D;
-    f->L = L;
-    while ((1 << f->lg_c) < 2 * D) ++f->lg_c;
-    f->block = cfg->block_samples;
-    f->info = info;
-    f->mt = mt;
-    f->smem = smem;
 
     // taps rounded to fp32 once; twiddles exp(-2 pi i t / C) in float64, rounded once
     const int C = 2 * D;
@@ -282,118 +166,37 @@ int rt_fbank_create(const rt_fbank_config* cfg, rt_fbank** out) {
         const double ang = -2.0 * M_PI * (double)t / (double)C;
         w[t] = make_float2((float)std::cos(ang), (float)std::sin(ang));
     }
-    const size_t hist_bytes = (size_t)f->n_in * std::max(1, L - 1) * sizeof(float2);
-#define FCUE(call)                                                                                 \
-    do {                                                                                           \
-        cudaError_t _e = (call);                                                                   \
-        if (_e != cudaSuccess) {                                                                   \
-            free_fbank(f);                                                                         \
-            return fail(RT_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_e));          \
-        }                                                                                          \
-    } while (0)
-    FCUE(cudaMalloc(&f->d_taps, h.size() * sizeof(float)));
-    FCUE(cudaMalloc(&f->d_twiddle, w.size() * sizeof(float2)));
-    FCUE(cudaMalloc(&f->d_off, f->n_in * sizeof(uint32_t)));
-    FCUE(cudaMalloc(&f->d_hist[0], hist_bytes));
-    FCUE(cudaMalloc(&f->d_hist[1], hist_bytes));
-    FCUE(cudaMemcpy(f->d_taps, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
-    FCUE(cudaMemcpy(f->d_twiddle, w.data(), w.size() * sizeof(float2), cudaMemcpyHostToDevice));
-    FCUE(cudaMemset(f->d_off, 0, f->n_in * sizeof(uint32_t)));
-    FCUE(cudaMemset(f->d_hist[0], 0, hist_bytes));
-    FCUE(cudaEventCreateWithFlags(&f->done, cudaEventDisableTiming));
-#undef FCUE
-    *out = f;
-    return RT_OK;
+    std::unique_ptr<rt_fbank> f(new rt_fbank());
+    while ((1 << f->lg_c) < C) ++f->lg_c;
+    rc = rt::fir_open(f.get(), p, mt, fbank_smem(mt, D, L), rt::fir_kernels(fbank_main, p.fmt),
+                      {{h.data(), h.size() * sizeof(float)}, {w.data(), w.size() * sizeof(float2)}});
+    if (rc == RT_OK) *out = f.release();
+    return rc;
 }
 
-void rt_fbank_destroy(rt_fbank* f) { free_fbank(f); }
+void rt_fbank_destroy(rt_fbank* f) { delete f; }
 
-int rt_fbank_reset_input(rt_fbank* f, int32_t input, int64_t first_sample) {
-    if (!f || input < 0 || input >= f->n_in) return fail(RT_ERR_INVALID, "bad input index");
-    f->resets.emplace_back(input, (uint32_t)(uint64_t)first_sample);
-    return RT_OK;
-}
+int rt_fbank_reset_input(rt_fbank* f, int32_t input, int64_t first_sample) { return rt::fir_reset_input(f, input, first_sample); }
 
 int rt_fbank_run(rt_fbank* f, void* cuda_stream, const void* iq, int32_t iq_on_device, size_t in_stride_bytes, int32_t blocks,
                  void* out, size_t out_stride_bytes) {
-    if (!f || !iq || !out) return fail(RT_ERR_INVALID, "null argument");
-    if (blocks < 1) return fail(RT_ERR_INVALID, "blocks must be >= 1");
-    const long long n = f->block * blocks;
-    const long long m_total = n / f->D;
-    const size_t row_bytes = (size_t)f->info.bytes * (size_t)n;
-    if (f->n_in > 1 && in_stride_bytes < row_bytes) return fail(RT_ERR_INVALID, "in_stride_bytes smaller than one input's blocks");
-    if (out_stride_bytes < (size_t)m_total * sizeof(float2)) return fail(RT_ERR_INVALID, "out_stride_bytes smaller than one channel's outputs");
-    if (((uintptr_t)out | out_stride_bytes) % sizeof(float2) != 0) return fail(RT_ERR_INVALID, "output pointer / stride not aligned to 8 bytes");
-    if ((m_total + f->mt - 1) / f->mt > 0x7fffffffLL) return fail(RT_ERR_INVALID, "call too long");
-    FCU(cudaSetDevice(f->dev));
-    cudaStream_t st = (cudaStream_t)cuda_stream;
-    if (f->ran) FCU(cudaStreamWaitEvent(st, f->done, 0));      // history, offsets and the staging buffer of the previous run
-
-    const unsigned char* src = static_cast<const unsigned char*>(iq);
-    size_t stride = f->n_in > 1 ? in_stride_bytes : row_bytes;
-    if (!iq_on_device) {
-        FCU(rt::fir_stage_host_input(st, &src, &stride, row_bytes, f->n_in, &f->d_stage, &f->stage_bytes));
-    } else if (((uintptr_t)src | (f->n_in > 1 ? stride : 0)) % (uintptr_t)f->info.bytes != 0) {
-        return fail(RT_ERR_INVALID, "IQ pointer / input stride not aligned to one complex sample");
-    }
-
-    rt::IqCorrArgs corr;
-    FCU(rt::iq_prepare(f->iq, st, f->done, f->ran, f->fmt, f->info, src, stride, f->n_in, f->block, blocks, &corr));
-    for (const auto& r : f->resets)
-        rt::fir_reset_kernel<<<1, 256, 0, st>>>(f->d_hist[f->cur], f->d_off, r.first, f->L - 1, r.second - f->advance);
-
+    rt::FirRun r;
+    const int rc = rt::fir_run_begin(f, cuda_stream, iq, iq_on_device, in_stride_bytes, blocks, out, out_stride_bytes, &r);
+    if (rc != RT_OK) return rc;
     FbankArgs a;
-    a.iq = src;
-    a.in_stride = stride;
-    a.hist = f->d_hist[f->cur];
-    a.hist_out = f->d_hist[f->cur ^ 1];
-    a.hist_len = f->L - 1;
-    a.taps = f->d_taps;
-    a.twiddle = f->d_twiddle;
-    a.off = f->d_off;
-    a.advance = f->advance;
-    a.out = static_cast<float2*>(out);
-    a.out_stride = out_stride_bytes;
-    a.n_samples = n;
-    a.m_total = m_total;
-    a.D = f->D;
-    a.L = f->L;
+    rt::fir_args(a, *f, r);
+    a.taps = static_cast<const float*>(f->tables[0]);
+    a.twiddle = static_cast<const float2*>(f->tables[1]);
     a.lg_c = f->lg_c;
-    a.mt = f->mt;
-    a.scale = (float)(1.0 / f->info.full_scale);
-    a.offset = (float)f->info.offset;
-    const dim3 grid((unsigned)((m_total + f->mt - 1) / f->mt), (unsigned)f->n_in);
-    if (f->iq.applied) {
-        FbankArgsIq ai;
-        static_cast<FbankArgs&>(ai) = a;
-        ai.corr = corr;
-        fbank_launch<true>(ai, f->fmt, grid, f->smem, f->n_in, st);
-    } else {
-        fbank_launch<false>(a, f->fmt, grid, f->smem, f->n_in, st);
-    }
-    FCU(cudaGetLastError());
-    FCU(cudaEventRecord(f->done, st));
-    f->ran = true;
-    f->resets.clear();
-    f->cur ^= f->L > 1 ? 1 : 0;
-    f->advance += (uint32_t)(uint64_t)n;
-    return RT_OK;
+    const dim3 grid((unsigned)((r.m_total + f->mt - 1) / f->mt), (unsigned)f->n_in);
+    rt::fir_launch<FbankArgsIq>(*f, r, a, fbank_main, grid, FB_THREADS);
+    return rt::fir_run_end(f, r);
 }
 
-int rt_fbank_set_iq_correction(rt_fbank* f, int32_t enable) {
-    if (!f) return fail(RT_ERR_INVALID, "null handle");
-    if (enable && f->block > rt::IQ_MAX_BLOCK) return fail(RT_ERR_INVALID, "block_samples must be <= 2^30 for the IQ correction");
-    f->iq.on = enable != 0;
-    return RT_OK;
-}
+int rt_fbank_set_iq_correction(rt_fbank* f, int32_t enable) { return rt::fir_set_iq_correction(f, enable); }
 
 int rt_fbank_read_iq_correction(rt_fbank* f, int32_t input, int32_t block, float out[4]) {
-    if (!f || !out) return fail(RT_ERR_INVALID, "null argument");
-    if (!f->iq.applied) return fail(RT_ERR_INVALID, "the last run did not apply the IQ correction");
-    if (input < 0 || input >= f->n_in || block < 0 || block >= f->iq.blocks) return fail(RT_ERR_INVALID, "bad input / block index");
-    FCU(cudaSetDevice(f->dev));
-    FCU(rt::iq_read(f->iq, f->done, input, block, out));
-    return RT_OK;
+    return rt::fir_read_iq_correction(f, input, block, out);
 }
 
 }  // extern "C"

@@ -56,6 +56,10 @@ FBANK_EXPORTS = ("rt_fbank_create", "rt_fbank_destroy", "rt_fbank_reset_input", 
                  "rt_fbank_read_iq_correction")
 
 
+# the functions of either front end, after its prefix (rt_ddc_, rt_fbank_)
+_FRONT_END_FUNCTIONS = ("create", "destroy", "reset_input", "run", "set_iq_correction", "read_iq_correction")
+
+
 class RtDdcConfig(ctypes.Structure):
     _fields_ = [
         ("abi_version", ctypes.c_int32), ("cuda_device", ctypes.c_int32), ("n_inputs", ctypes.c_int32),
@@ -78,21 +82,16 @@ class RtFbankConfig(ctypes.Structure):
 def _load():
     lib = _engine.load_library()
     if not getattr(lib, "_ddc_types", False):
-        lib.rt_ddc_create.argtypes = [ctypes.POINTER(RtDdcConfig), ctypes.POINTER(ctypes.c_void_p)]
-        lib.rt_ddc_destroy.argtypes = [ctypes.c_void_p]
-        lib.rt_ddc_destroy.restype = None
-        lib.rt_ddc_reset_input.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64]
-        lib.rt_ddc_run.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_size_t,
-                                   ctypes.c_int32, ctypes.c_void_p, ctypes.c_size_t]
-        lib.rt_fbank_create.argtypes = [ctypes.POINTER(RtFbankConfig), ctypes.POINTER(ctypes.c_void_p)]
-        lib.rt_fbank_destroy.argtypes = [ctypes.c_void_p]
-        lib.rt_fbank_destroy.restype = None
-        lib.rt_fbank_reset_input.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64]
-        lib.rt_fbank_run.argtypes = lib.rt_ddc_run.argtypes
-        for name in ("rt_ddc", "rt_fbank"):
-            getattr(lib, name + "_set_iq_correction").argtypes = [ctypes.c_void_p, ctypes.c_int32]
-            getattr(lib, name + "_read_iq_correction").argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32,
-                                                                   ctypes.POINTER(ctypes.c_float)]
+        for prefix, config in (("rt_ddc", RtDdcConfig), ("rt_fbank", RtFbankConfig)):
+            create, destroy, reset, run, set_iq, read_iq = (getattr(lib, f"{prefix}_{name}") for name in _FRONT_END_FUNCTIONS)
+            create.argtypes = [ctypes.POINTER(config), ctypes.POINTER(ctypes.c_void_p)]
+            destroy.argtypes = [ctypes.c_void_p]
+            destroy.restype = None
+            reset.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64]
+            run.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_size_t, ctypes.c_int32,
+                            ctypes.c_void_p, ctypes.c_size_t]
+            set_iq.argtypes = [ctypes.c_void_p, ctypes.c_int32]
+            read_iq.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(ctypes.c_float)]
         lib._ddc_types = True
     return lib
 
@@ -140,13 +139,32 @@ def _check_taps(h: np.ndarray, max_taps: int) -> None:
 
 
 class _WidebandFrontEnd:
-    """What Channelizer and FilterBank share: the sample format, the handle's life cycle and the input / output handling of
-    `run`.  A subclass sets `_lib`, `_h`, `_destroy`, `_reset`, `_run`, `_set_iq`, `_read_iq`, `n_inputs`, `n_channels`,
-    `block_samples`, `decimation`, `blocks_per_launch`, `cuda_device`, calls `_set_format` and, after creating the handle,
-    `set_iq_correction`."""
+    """What Channelizer and FilterBank share: the constructor's common steps, the handle's life cycle and the input / output
+    handling of `run`.  A subclass checks its plan, sets `offsets_hz`, `phase_inc` and `n_channels`, calls `__init__` with its
+    C prefix and tap limit, and builds its config struct in `_config`."""
 
     _h = None
     iq_correction = False
+
+    def __init__(self, prefix: str, sample_rate: int, block_samples: int, decimation: int, taps, max_taps: int,
+                 sample_format: str, n_inputs: int, cuda_device: int, blocks_per_launch: int, iq_correction: bool):
+        h = default_taps(decimation) if taps is None else np.asarray(taps, dtype=np.float64)
+        _check_taps(h, max_taps)
+        if blocks_per_launch < 1:
+            raise ValueError("blocks_per_launch must be >= 1")
+        self._set_format(sample_format)
+        self.sample_rate, self.block_samples, self.decimation = sample_rate, int(block_samples), decimation
+        self.taps = np.ascontiguousarray(h)
+        self.n_inputs = int(n_inputs)
+        self.blocks_per_launch = int(blocks_per_launch)
+        self.cuda_device = cuda_device
+        self._lib = _load()
+        create, self._destroy, self._reset, self._run, self._set_iq, self._read_iq = (
+            getattr(self._lib, f"{prefix}_{name}") for name in _FRONT_END_FUNCTIONS)
+        self._h = ctypes.c_void_p()
+        _engine._check(create(ctypes.byref(self._config()), ctypes.byref(self._h)))
+        if iq_correction:
+            self.set_iq_correction(True)
 
     def _set_format(self, sample_format: str) -> None:
         self.sample_format = _engine.sample_format_name(sample_format)
@@ -251,29 +269,16 @@ class Channelizer(_WidebandFrontEnd):
         for o in off:
             if abs(o) + fs / (2 * D) > fs / 2:
                 raise ValueError(f"channel at {o} Hz with half-width {fs / (2 * D)} Hz does not lie inside the input band +-{fs / 2} Hz")
-        h = default_taps(D) if taps is None else np.asarray(taps, dtype=np.float64)
-        _check_taps(h, MAX_TAPS)
-        if blocks_per_launch < 1:
-            raise ValueError("blocks_per_launch must be >= 1")
-        self._set_format(sample_format)
-        self.sample_rate, self.block_samples, self.decimation = fs, int(block_samples), D
-        self.offsets_hz, self.taps = off, np.ascontiguousarray(h)
-        self.phase_inc = phase_increment(off, fs)
-        self.n_inputs, self.n_channels = int(n_inputs), len(off)
-        self.blocks_per_launch = int(blocks_per_launch)
-        self.cuda_device = cuda_device
-        self._lib = _load()
-        self._destroy, self._reset, self._run = self._lib.rt_ddc_destroy, self._lib.rt_ddc_reset_input, self._lib.rt_ddc_run
-        self._set_iq, self._read_iq = self._lib.rt_ddc_set_iq_correction, self._lib.rt_ddc_read_iq_correction
-        self._h = ctypes.c_void_p()
-        cfg = RtDdcConfig(
-            abi_version=RT_DDC_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, n_channels=self.n_channels,
-            block_samples=self.block_samples, decimation=D, n_taps=len(h), sample_format=self._format_code, reserved=0,
-            sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+        self.offsets_hz, self.phase_inc, self.n_channels = off, phase_increment(off, fs), len(off)
+        super().__init__("rt_ddc", fs, block_samples, D, taps, MAX_TAPS, sample_format, n_inputs, cuda_device, blocks_per_launch,
+                         iq_correction)
+
+    def _config(self) -> RtDdcConfig:
+        return RtDdcConfig(
+            abi_version=RT_DDC_ABI_VERSION, cuda_device=self.cuda_device, n_inputs=self.n_inputs, n_channels=self.n_channels,
+            block_samples=self.block_samples, decimation=self.decimation, n_taps=self.n_taps, sample_format=self._format_code,
+            reserved=0, sample_rate=float(self.sample_rate), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
             phase_inc=self.phase_inc.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)))
-        _engine._check(self._lib.rt_ddc_create(ctypes.byref(cfg), ctypes.byref(self._h)))
-        if iq_correction:
-            self.set_iq_correction(True)
 
 
 class FilterBank(_WidebandFrontEnd):
@@ -292,30 +297,17 @@ class FilterBank(_WidebandFrontEnd):
             raise ValueError(f"decimation = {decimation}: must be a power of two in [{FBANK_MIN_DECIMATION}, {FBANK_MAX_DECIMATION}]")
         if fs % D or block_samples % D or block_samples < D:
             raise ValueError(f"sample_rate ({fs}) and block_samples ({block_samples}) must be multiples of the decimation {D}")
-        h = default_taps(D) if taps is None else np.asarray(taps, dtype=np.float64)
-        _check_taps(h, 16 * D + 1)
-        if blocks_per_launch < 1:
-            raise ValueError("blocks_per_launch must be >= 1")
         if not 1 <= int(n_inputs) <= 65535 or int(n_inputs) * (2 * D - 1) > 1 << 30:
             raise ValueError(f"n_inputs = {n_inputs}: must be in [1, 65535] with n_inputs * (2 D - 1) <= 2^30")
-        self._set_format(sample_format)
-        self.sample_rate, self.block_samples, self.decimation = fs, int(block_samples), D
-        self.offsets_hz, self.taps = grid_offsets(fs, D), np.ascontiguousarray(h)
-        self.phase_inc = grid_phase_increment(D)
-        self.n_inputs, self.n_channels = int(n_inputs), 2 * D - 1
-        self.blocks_per_launch = int(blocks_per_launch)
-        self.cuda_device = cuda_device
-        self._lib = _load()
-        self._destroy, self._reset, self._run = self._lib.rt_fbank_destroy, self._lib.rt_fbank_reset_input, self._lib.rt_fbank_run
-        self._set_iq, self._read_iq = self._lib.rt_fbank_set_iq_correction, self._lib.rt_fbank_read_iq_correction
-        self._h = ctypes.c_void_p()
-        cfg = RtFbankConfig(
-            abi_version=RT_FBANK_ABI_VERSION, cuda_device=cuda_device, n_inputs=self.n_inputs, decimation=D,
-            block_samples=self.block_samples, n_taps=len(h), sample_format=self._format_code, reserved=0,
-            sample_rate=float(fs), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)))
-        _engine._check(self._lib.rt_fbank_create(ctypes.byref(cfg), ctypes.byref(self._h)))
-        if iq_correction:
-            self.set_iq_correction(True)
+        self.offsets_hz, self.phase_inc, self.n_channels = grid_offsets(fs, D), grid_phase_increment(D), 2 * D - 1
+        super().__init__("rt_fbank", fs, block_samples, D, taps, 16 * D + 1, sample_format, n_inputs, cuda_device, blocks_per_launch,
+                         iq_correction)
+
+    def _config(self) -> RtFbankConfig:
+        return RtFbankConfig(
+            abi_version=RT_FBANK_ABI_VERSION, cuda_device=self.cuda_device, n_inputs=self.n_inputs, decimation=self.decimation,
+            block_samples=self.block_samples, n_taps=self.n_taps, sample_format=self._format_code, reserved=0,
+            sample_rate=float(self.sample_rate), taps=self.taps.ctypes.data_as(ctypes.POINTER(ctypes.c_double)))
 
 
 class WidebandAnalyzer:
